@@ -26,6 +26,12 @@ legs        dense_path (same corpus, the product's default dense-state path), c3
 cpu_baseline / --impl reference
             the CPU oracle (restatement of the reference algorithm; the reference binary needs Boost and cannot be built
             here) timed on this box's host cores on a bounded sample of the main workload.
+--dump-outputs DIR
+            after the main line's timed steps, rank 0 writes what the last timed EM iteration gave its caller as
+            DIR/<name>.npy (float64): step_result (sum ln P, sum weighted ln P, examples without a derivation, max weight
+            change), params (ln weights after the M-step), counts (the all-reduced expected counts), example_ln_p (ln P of
+            rank 0's examples).  Inputs are seeded, so two builds can be compared output for output.  Above 64 MB in all,
+            every array is cut to the same share by a fixed seeded choice of indices.
 """
 from __future__ import annotations
 
@@ -47,6 +53,7 @@ FALLBACK_HBM_GBS = 6650.0  # /opt/skills/guides/B200_PROFILING.md fallback
 METRIC, UNIT = "em_iteration_trellis_arcs_per_sec", "trellis arcs/s"
 CIPHER_LINES, CIPHER_SAMPLE = 2000, 160
 C3_SENTENCES, C3_SAMPLE = 1000000, 16000
+DUMP_BYTES = (64 << 20) - (16 << 10)  # --dump-outputs: 64 MB in all, less room for the .npy headers
 
 
 def measured_traffic(kernel, units=None):
@@ -198,6 +205,22 @@ def oracle_example_lnp(w, n_pairs):
         shutil.rmtree(d, ignore_errors=True)
 
 
+def dump_outputs(outdir, arrays, limit=DUMP_BYTES):
+    """write every array as outdir/<name>.npy in float64; when together they exceed `limit` bytes, arrays above 1 MB
+    share what the smaller ones leave, each the same share of its elements, chosen by a fixed seed so that two runs
+    keep the same indices"""
+    import numpy as np
+    os.makedirs(outdir, exist_ok=True)
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float64).ravel() for k, v in arrays.items()}
+    small = sum(v.nbytes for v in arrays.values() if v.nbytes <= 1 << 20)
+    large = sum(v.nbytes for v in arrays.values()) - small
+    for name, v in arrays.items():
+        if small + large > limit and v.nbytes > 1 << 20:
+            keep = v.size * (limit - small) // large
+            v = v[np.sort(np.random.default_rng(0).choice(v.size, keep, replace=False))]
+        np.save(os.path.join(outdir, f"{name}.npy"), v)
+
+
 def measure_tf32_peak(torch):
     """dense TF32 GEMM rate of this GPU (torch.matmul, 8192^3, best of 5): the denominator of the dense-state roofline"""
     old = torch.backends.cuda.matmul.allow_tf32
@@ -240,7 +263,13 @@ def main():
     ap.add_argument("--c3-sentences", type=int, default=C3_SENTENCES)
     ap.add_argument("--unlock-lm", action="store_true",
                     help="cipher: make the bigram LM trainable too (transition counts are then part of the E-step)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the main line's last timed EM iteration computed as DIR/<name>.npy (see the module doc)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl == "reference" or a.workload in ("forest", "gibbs")):
+        ap.error("--dump-outputs writes the outputs of the B200 EM path (--workload cipher or hmm)")
     a.warmup = max(3, a.warmup)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -350,8 +379,9 @@ def main():
     tf32 = {"value": None}
 
     def measure(w, no_dense: bool, precision: int, steps: int, sample_pairs: int, shard: bool, traffic_key=None,
-                check_n: bool = False) -> dict:
-        """one job on workload w: warm-up + timed steps + e2e loop + kernel-alone pass + parity; returns what rank 0 prints"""
+                check_n: bool = False, dump_dir=None) -> dict:
+        """one job on workload w: warm-up + timed steps + e2e loop + kernel-alone pass + parity; returns what rank 0 prints.
+        dump_dir: rank 0 writes the outputs of the last timed step there (dump_outputs)"""
         extra = ["-q", f"--gpu={local}"]
         if precision == 32:
             extra.append("--float")
@@ -430,8 +460,10 @@ def main():
                 dist.all_reduce(ms, op=dist.ReduceOp.MAX)
             return float(ms.item())
 
+        last = [first]
+
         def step():
-            ctx.em_step(1.0)
+            last[0] = ctx.em_step(1.0)
 
         for _ in range(a.warmup):
             step()
@@ -445,6 +477,11 @@ def main():
         launches, collectives = ctx.launch_count() - l0, ctx.collective_count() - c0
         clocks = sampler.stop() if rank == 0 else None
         value = arcs_total * steps / (ms / 1e3)
+        if dump_dir and rank == 0:  # before the e2e loop below runs further EM iterations
+            r_last, change = last[0]
+            dump_outputs(dump_dir, {"step_result": [r_last.sum_ln_p, r_last.sum_w_ln_p, r_last.n_zero, change],
+                                    "params": ctx.get_params(), "counts": ctx.counts(),
+                                    "example_ln_p": ctx.example_logprob(int(info["examples"]))})
 
         # ---- e2e: host buffers through the C ABI every step
         n_params, n_arcs = info["n_params"], info["n_arcs"]
@@ -585,13 +622,14 @@ def main():
     if single:
         w = shared_workload(a.workload, (CIPHER_LINES if a.workload == "cipher" else 125000) * a.scale * world, "main")
         main_res = measure(w, a.no_dense, a.precision, a.steps, CIPHER_SAMPLE if a.workload == "cipher" else C3_SAMPLE, True,
-                           traffic_key=None)
+                           traffic_key=None, dump_dir=a.dump_outputs)
         other = None
         if main_res["is_dense"] and not a.no_sparse_leg:
             other = measure(w, True, a.precision, a.steps, 0, True)
     else:
         w = shared_workload("cipher", CIPHER_LINES * world, "main")
-        main_res = measure(w, True, 64, a.steps, CIPHER_SAMPLE, True, traffic_key="k_fb_wide_cipher", check_n=True)
+        main_res = measure(w, True, 64, a.steps, CIPHER_SAMPLE, True, traffic_key="k_fb_wide_cipher", check_n=True,
+                           dump_dir=a.dump_outputs)
     line = None
     if rank == 0:
         failures = []

@@ -1,4 +1,5 @@
 // micro-benchmark: throughput of fp64 count accumulation patterns on one B200 (round 2 design input)
+// build: nvcc -gencode arch=compute_100a,code=sm_100a -O3 -o profiles/micro/red_bench profiles/micro/red_bench.cu
 #include <cstdio>
 #include <cstdint>
 #include <cuda_runtime.h>
