@@ -20,6 +20,7 @@ NO_GROUP = 0xFFFFFFFF
 LOCKED_GROUP = 0
 
 OPT_ARC_COUNTS, OPT_NO_ELL, OPT_LANE_MIN, OPT_NO_COUNTS, OPT_NO_FACTOR, OPT_NO_WIDE = 1, 2, 3, 4, 5, 6
+OPT_KBEST_SCRATCH_MB = 9
 OK, ERR_ARG, ERR_CUDA, ERR_STATE, ERR_CYCLE, ERR_NODERIV, ERR_NOT_DENSE = 0, -1, -2, -3, -4, -5, -6
 
 _u32p = C.POINTER(C.c_uint32)
@@ -113,6 +114,9 @@ def load_library(path: str | None = None) -> C.CDLL:
     lib.cml_dense_kernel.argtypes = [vp, C.POINTER(C.c_int), _u32p, _u32p]
     lib.cml_gibbs_attach_dense.argtypes = [vp, C.POINTER(CmlDenseView), C.POINTER(CmlSequenceBatch)]
     lib.cml_trellis_totals.argtypes = [vp] + [C.POINTER(C.c_uint64)] * 4
+    lib.cml_viterbi.argtypes = [vp, _u32p, C.POINTER(C.c_uint64), _u32p, C.c_uint64, _f64p]
+    lib.cml_kbest.argtypes = [vp, C.c_uint32, _u32p, C.POINTER(C.c_uint64), _u32p, C.c_uint64, _f64p]
+    lib.cml_kbest_stats.argtypes = [vp, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.POINTER(C.c_float)]
     lib.cml_get_example_layout.argtypes = [vp, C.c_uint64, _u32p, _u32p, _u32p]
     lib.cml_estimate.argtypes = [vp, C.POINTER(CmlEstimateResult)]
     lib.cml_estimate_launch.argtypes = [vp]
@@ -315,6 +319,40 @@ class Context:
         v = [C.c_uint64() for _ in range(4)]
         self._check(self.lib.cml_trellis_totals(self.h, *[C.byref(x) for x in v]))
         return dict(zip(("examples", "states", "arcs", "levels"), (int(x.value) for x in v)))
+
+    # ---- decode (cml_viterbi / cml_kbest) ----
+    def _decode(self, k: int | None, cap: int | None):
+        t = self.trellis_totals()
+        n_ex, kk = t["examples"], 1 if k is None else k
+        n = n_ex * kk
+        ln_w, lens = np.zeros(max(n, 1)), np.zeros(max(n, 1), np.uint32)
+        base = np.zeros(n + 1, np.uint64)
+        if cap is None:
+            cap = kk * t["levels"]
+        arcs = np.zeros(max(cap, 1), np.uint32)
+        bp = base.ctypes.data_as(C.POINTER(C.c_uint64))
+        if k is None:
+            rc = self.lib.cml_viterbi(self.h, _ptr(lens, _u32p), bp, _ptr(arcs, _u32p), cap, _ptr(ln_w, _f64p))
+        else:
+            rc = self.lib.cml_kbest(self.h, k, _ptr(lens, _u32p), bp, _ptr(arcs, _u32p), cap, _ptr(ln_w, _f64p))
+        self._check(rc)
+        return ln_w[:n].reshape(n_ex, kk), lens[:n].reshape(n_ex, kk), base, arcs
+
+    def kbest(self, k: int, cap: int | None = None):
+        """the k best derivations of every resident lattice (cml_kbest): (ln_weight [n_ex, k], path_len [n_ex, k],
+        path_base [n_ex * k + 1], path_arcs); derivation (e, r) is path_arcs[path_base[e*k+r]:][:path_len[e, r]].
+        cap (default: k * total lattice levels) is the size of the arc buffer handed to the library."""
+        return self._decode(int(k), cap)
+
+    def viterbi(self):
+        """the best derivation of every resident lattice (cml_viterbi), in kbest()'s shapes with k = 1"""
+        return self._decode(None, None)
+
+    def kbest_stats(self) -> dict:
+        """the last decode call: scratch bytes of its largest chunk, chunks, kernel time (CUDA events, ms)"""
+        b, c, ms = C.c_uint64(), C.c_uint64(), C.c_float()
+        self._check(self.lib.cml_kbest_stats(self.h, C.byref(b), C.byref(c), C.byref(ms)))
+        return {"scratch_bytes": b.value, "chunks": c.value, "kernel_ms": ms.value}
 
     def example_layout(self, e: int, n_states: int):
         nl = C.c_uint32()

@@ -1073,8 +1073,13 @@ extern "C" int cml_viterbi(cml_ctx* ctx, uint32_t* path_len, uint64_t* path_base
   CML_CUDA(d_len.alloc(std::max<uint64_t>(1, n_ex)));
   CML_CUDA(d_lnw.alloc(std::max<uint64_t>(1, n_ex)));
   CML_CUDA(d_path.alloc(std::max<uint64_t>(1, pbase[n_ex])));
+  cudaEvent_t ev0 = nullptr, ev1 = nullptr;  // kernel time for cml_kbest_stats
+  CML_CUDA(cudaEventCreate(&ev0));
+  CML_CUDA(cudaEventCreate(&ev1));
+  CML_CUDA(cudaEventRecord(ev0, s));
   k_viterbi<<<cdiv(n_ex, 64), 64, 0, s>>>(bt.desc.p, (uint32_t)n_ex, bt.out_off.p, bt.out_arc.p, (const double*)ctx->arc_w_real.p,
                                          d_orig.p, d_sbase.p, d_pbase.p, d_best.p, d_src.p, d_arc.p, d_len.p, d_path.p, d_lnw.p);
+  cudaEventRecord(ev1, s);
   ++ctx->launches;
   CML_CUDA(cudaGetLastError());
   CML_CUDA(cudaMemcpyAsync(path_len, d_len.p, n_ex * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
@@ -1082,5 +1087,10 @@ extern "C" int cml_viterbi(cml_ctx* ctx, uint32_t* path_len, uint64_t* path_base
   if (path_arcs && pbase[n_ex])
     CML_CUDA(cudaMemcpyAsync(path_arcs, d_path.p, pbase[n_ex] * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
   CML_CUDA(cudaStreamSynchronize(s));
+  ctx->kbest_chunks = 1;
+  ctx->kbest_scratch = bt.n_states * (sizeof(double) + 2 * sizeof(uint32_t));
+  cudaEventElapsedTime(&ctx->kbest_ms, ev0, ev1);
+  cudaEventDestroy(ev0);
+  cudaEventDestroy(ev1);
   return CML_OK;
 }

@@ -158,6 +158,8 @@ struct TrainOpts {
   uint32_t final_restart = 0;       // --final-restart=N : restart index at which the tolerance reaches its final value
   double ln_restart_tolerance = kNegInf, ln_final_restart_tolerance = kNegInf;  // --restart-tolerance= --final-restart-tolerance= (none: accept all)
   uint64_t seed = 1;                // -R seed : the restarts' generator (the reference seeds boost's lagged Fibonacci; draws differ)
+  std::string kbest_arg;            // -k n : derivations per example written by --viterbi (unused when training)
+  uint32_t kbest = 1;
   TrainOpts();
 };
 // WFST::random_restart_acceptor (fst.h:999-1044): a further start must be, after its first iteration, within a

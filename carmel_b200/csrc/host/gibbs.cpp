@@ -317,8 +317,9 @@ TrainResult const& TrainJob::run_gibbs(std::ostream& log) {
   return res;
 }
 
-// Decode: best derivation per training pair (cml_viterbi).  The weights are the model's as read, after the same
-// normalisation a training run starts from (train.cc:509); no training happens.
+// Decode: the -k n best derivations per training pair (cml_viterbi for n = 1, cml_kbest otherwise), n lines per example
+// in corpus order, best first; ranks past the number of derivations read "-inf 0 |".  The weights are the model's as
+// read, after the same normalisation a training run starts from (train.cc:509); no training happens.
 void TrainJob::run_viterbi(std::ostream& log, std::string const& path) {
   opt.precision = 64;
   opt.space = CML_SPACE_LOG;  // layered-CSR lattices keep the reference's per-state arc order
@@ -326,12 +327,14 @@ void TrainJob::run_viterbi(std::ostream& log, std::string const& path) {
   opt.dense = -1;
   if (opt.shard_count > 1) throw std::runtime_error("--viterbi decodes on one GPU");
   prepare();
+  const uint64_t K = opt.kbest;
   uint64_t n_ex = 0, n_states = 0, n_arcs = 0, n_levels = 0;
   ok(cml_trellis_totals(ctx, &n_ex, &n_states, &n_arcs, &n_levels));
-  std::vector<uint32_t> len(n_ex), arcs(std::max<uint64_t>(1, n_levels));
-  std::vector<uint64_t> base(n_ex + 1);
-  std::vector<double> lnw(n_ex);
-  if (n_ex) ok(cml_viterbi(ctx, len.data(), base.data(), arcs.data(), arcs.size(), lnw.data()));
+  std::vector<uint32_t> len(n_ex * K), arcs(std::max<uint64_t>(1, n_levels * K));
+  std::vector<uint64_t> base(n_ex * K + 1);
+  std::vector<double> lnw(n_ex * K);
+  if (n_ex && K == 1) ok(cml_viterbi(ctx, len.data(), base.data(), arcs.data(), arcs.size(), lnw.data()));
+  if (n_ex && K > 1) ok(cml_kbest(ctx, (uint32_t)K, len.data(), base.data(), arcs.data(), arcs.size(), lnw.data()));
   // labels of every parameter's member arc (parameters are numbered member by member, state by state, arc by arc)
   std::vector<std::string> plabel;
   for (Wfst* m : members)
@@ -341,22 +344,26 @@ void TrainJob::run_viterbi(std::ostream& log, std::string const& path) {
   if (!o) throw std::runtime_error("cannot write " + path);
   o.precision(17);
   double total = 0;
-  for (uint64_t e = 0; e < n_ex; ++e) {
-    o << lnw[e] << " " << len[e];
-    for (uint32_t k = 0; k < len[e]; ++k) o << " " << arcs[base[e] + k];
+  uint64_t found = 0;
+  for (uint64_t i = 0; i < n_ex * K; ++i) {
+    o << lnw[i] << " " << len[i];
+    for (uint32_t k = 0; k < len[i]; ++k) o << " " << arcs[base[i] + k];
     o << " |";
-    for (uint32_t k = 0; k < len[e]; ++k) {
-      const uint32_t a = arcs[base[e] + k];
+    for (uint32_t k = 0; k < len[i]; ++k) {
+      const uint32_t a = arcs[base[i] + k];
       const uint32_t k0 = using_cascade ? M.chain_off[a] : a, k1 = using_cascade ? M.chain_off[a + 1] : a + 1;
       o << " (";
       for (uint32_t c = k0; c < k1; ++c) o << (c > k0 ? " " : "") << plabel[using_cascade ? M.chain_param[c] : c];
       o << ")";
     }
     o << "\n";
-    total += lnw[e];
+    if (i % K == 0) total += lnw[i];
+    if (lnw[i] > kNegInf) ++found;
   }
-  if (!opt.quiet)
+  if (!opt.quiet) {
     log << "Viterbi: best derivations of " << n_ex << " examples, product of their weights=" << format_base2(total) << "\n";
+    if (K > 1) log << "Viterbi: " << K << "-best lists, " << found << " derivations found\n";
+  }
 }
 
 }  // namespace cb

@@ -58,6 +58,7 @@ int open_job(int argc, const char* const* argv, TrainJob& job, std::ostream& err
         case 'F': job.outfile = arg; break;
         case '!': topt.ran_restarts = (uint32_t)std::atol(arg.c_str()); break;
         case 'R': topt.seed = std::strtoull(arg.c_str(), nullptr, 10); break;
+        case 'k': topt.kbest_arg = arg; break;
         default: break;  // accepted, unused on this path
       }
       continue;
@@ -163,6 +164,15 @@ int open_job(int argc, const char* const* argv, TrainJob& job, std::ostream& err
 
   job.corpus_file = files[0];
   job.fst_files.assign(files.begin() + 1, files.end());
+  if (lopt.count("viterbi") && flags[(unsigned)'k']) {  // -k n with --viterbi: n derivations per example
+    char* end = nullptr;
+    const unsigned long long n = std::strtoull(topt.kbest_arg.c_str(), &end, 10);
+    if (topt.kbest_arg.empty() || *end || topt.kbest_arg[0] == '-' || n < 1 || n > 0xFFFFFFFFull) {
+      err << "carmel-b200: -k needs a whole number of derivations >= 1 (got \"" << topt.kbest_arg << "\")\n";
+      return -9;
+    }
+    topt.kbest = (uint32_t)n;
+  }
   const uint32_t n_chain = (uint32_t)job.fst_files.size();
   for (auto const& f : job.fst_files) {
     std::ifstream in(f);

@@ -37,13 +37,20 @@ static void usage() {
                "  --trellis-only  build (and dump) the derivation lattices on the host, then stop\n"
                "  --fem-forest=f --fem-norm=f --fem-param=f   export the cascade for forest-em(-b200): one derivation forest\n"
                "           per example, normalisation groups, parameters after training (-M -1: the normalised input weights)\n"
-               "  --load-fem-param=f  read cascade weights written by --fem-param\n";
+               "  --load-fem-param=f  read cascade weights written by --fem-param\n"
+               "  --viterbi=file [-k n]  decode only: the n best derivations (default 1) of every training pair, n lines per\n"
+               "           example, best first (\"-inf 0 |\" past the last derivation)\n";
 }
 
 // carmel-b200 --gpus=N ...: N jobs in one process, job r keeps block r of the corpus on GPU r (--shard=r/N --gpu=r); the
 // contexts share one NCCL communicator and every iteration all-reduces the count table on the GPUs' own streams.  All
 // ranks take the same decisions (the reduced table and likelihood are identical everywhere); rank 0 logs and writes.
 static int run_multi_gpu(int argc, char** argv, int n_gpus) {
+  for (int i = 1; i < argc; ++i)
+    if (std::strncmp(argv[i], "--viterbi", 9) == 0) {
+      std::cerr << "ERROR: --viterbi decodes on one GPU (no --gpus)\n";
+      return -11;
+    }
   unsigned char id[CML_COMM_ID_BYTES];
   if (cml_comm_unique_id(id) != CML_OK) {
     std::cerr << "ERROR: --gpus needs NCCL (libnccl.so.2 could not be loaded)\n";

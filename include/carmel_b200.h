@@ -74,7 +74,8 @@ enum cml_option {
                              warp-per-lattice kernel (tests).  Set before cml_add_trellises. */
   CML_OPT_ALLOW_EMPTY = 7, /* a rank of a sharded job whose block holds no usable example still takes part in every
                              collective: its E-step contributes zeros instead of failing with CML_ERR_NODERIV */
-  CML_OPT_NO_GRAPH = 8    /* cml_em_step enqueues its launches one by one instead of replaying a CUDA graph */
+  CML_OPT_NO_GRAPH = 8,   /* cml_em_step enqueues its launches one by one instead of replaying a CUDA graph */
+  CML_OPT_KBEST_SCRATCH_MB = 9 /* device scratch budget (MiB) of one cml_kbest chunk; default 4096 */
 };
 int cml_set_option(cml_ctx* ctx, int option, int value);
 
@@ -205,6 +206,31 @@ int cml_cyclic_stats(cml_ctx* ctx, uint64_t* n_examples, uint64_t* n_back_edges)
  *   path_arcs[cap]       arc-table ids in path order; cap >= the total number of lattice levels (cml_trellis_totals)
  *   ln_weight[n_ex]      ln of the derivation's weight (-inf: none) */
 int cml_viterbi(cml_ctx* ctx, uint32_t* path_len, uint64_t* path_base, uint32_t* path_arcs, uint64_t cap, double* ln_weight);
+/* The k best derivations of every resident lattice, best first -- carmel's `-k n` on the composed
+ * string x transducer x string machine (graehl/shared/kbest.h).  Same preconditions and errors as cml_viterbi, and
+ * CML_ERR_ARG for k == 0 or a path_arcs buffer that is too small.
+ *   path_len[n_ex * k]       arcs of derivation (e, r) at [e * k + r]; 0 = no such derivation
+ *   path_base[n_ex * k + 1]  derivation (e, r) is path_arcs[path_base[e * k + r] .. + path_len[e * k + r])
+ *   path_arcs[cap]           arc-table ids in path order, or NULL for weights only; cap >= k * the total number of
+ *                            lattice levels (cml_trellis_totals)
+ *   ln_weight[n_ex * k]      ln weight of derivation (e, r); -inf where example e has fewer than r + 1 derivations
+ * Contract:
+ *   order       example e's derivations come in non-increasing ln weight
+ *   distinct    they are distinct lattice paths (in a string x transducer x string lattice: distinct arc-id sequences)
+ *   zero weight derivations of weight zero (ln -inf) are never listed; a -inf entry has path_len 0
+ *   ties        a state's list is the top k of (source list entry + arc weight) over its in-arcs; among candidates of
+ *               exactly equal score the one earlier in the state's in-list (sorted by source layered index, then the
+ *               source's stored out-arc order) comes first, then the lower source rank
+ *   rank 0      is bit-identical to cml_viterbi: same double, same arc ids
+ *   determinism the same inputs give the same bytes on every run
+ *   memory      device scratch of about 16 B * k per lattice state plus 4 B per state and per lattice arc; the
+ *               lattices are processed in chunks of consecutive lattices whose scratch fits CML_OPT_KBEST_SCRATCH_MB
+ *               (a lattice larger than that gets a chunk of its own).  Results do not depend on the chunking. */
+int cml_kbest(cml_ctx* ctx, uint32_t k, uint32_t* path_len, uint64_t* path_base, uint32_t* path_arcs, uint64_t cap,
+              double* ln_weight);
+/* the last cml_kbest / cml_viterbi call: device scratch bytes of its largest chunk, number of chunks, and the time of
+ * its derivation kernels from CUDA events (ms) */
+int cml_kbest_stats(cml_ctx* ctx, uint64_t* scratch_bytes, uint64_t* chunks, float* kernel_ms);
 /* how the resident lattices are stored: examples / arcs / padded records in the level-sliced ELL layout
  * (throughput kernel) and examples in the layered-CSR layout (general kernels) */
 int cml_layout_stats(cml_ctx* ctx, uint64_t* ell_examples, uint64_t* ell_arcs, uint64_t* ell_records,
