@@ -977,6 +977,9 @@ struct cml_forests {
   void* comm = nullptr;  // ncclComm_t of this rank (cml_forests_comm_init_rank), null on a single GPU
   int comm_size = 1;
   uint64_t collectives = 0;
+  // cml_forests_kbest: scratch budget of one chunk, and the last call's scratch / chunks / kernel time
+  uint64_t kbest_scratch_mb = 4096, kbest_scratch = 0, kbest_chunks = 0;
+  float kbest_ms = 0;
 };
 // cml_comm.cu
 int cml_nccl_init_rank(void** comm, int n_ranks, int rank, const unsigned char* id, std::string& err);
@@ -2612,4 +2615,488 @@ extern "C" int cml_forests_normalize_params(cml_forests* f) {
   if (!f) return CML_ERR_ARG;
   F_REQUIRE(f->have_params, CML_ERR_STATE, "cml_forests_normalize_params before cml_forests_set_params");
   return forest_norm(f, nullptr, 0., 0., CML_FOREST_UNIFORM, nullptr, nullptr);
+}
+
+// ---------------------------------------------------------------------------------------------------
+// k best derivations of every forest (forest-em -v --kbest=n): an eager k-best merge over the hypergraph, bottom-up by
+// height.  A derivation is a choice of one child at every OR node it reaches; a shared node (back reference) is
+// expanded independently at every use.  Lists are best first, with a fixed tie key:
+//   OR node     top k over its children's entries: score desc, then child pre-order position, then child rank;
+//   AND node    rule weight w, slots s1..sm: a left fold  L0 = [w],  Lj = top k { L(j-1)[a] + sj[b] }, ties by a then b
+//               (the sums in k_forest_viterbi's order, so rank 0 is its derivation, bit for bit);
+//   back ref.   its shared node's list.
+// Every list entry carries its score, a back pointer -- OR: (resolved child node, its rank); fold: (a, b) -- and the
+// size of its subtree in AND nodes (1 + the slots' sizes for AND, the chosen child's size for OR), so the output offsets
+// of a derivation's nodes are known without walking it: extraction needs no stack and no depth limit.
+//
+// k_forest_kbest: one warp per forest.  Real nodes come levelised by height (forest_pass1's heights, which already see
+// through back references); the nodes of one height never feed each other and are merged in parallel by lane groups of
+// G lanes, heights are separated by __syncwarp.  A merge is k rounds of a shuffle arg-max over the group; lane g owns
+// candidate rows g, g + G, ... (OR: one head per child; fold: one cursor per entry of L(j-1), rows opened one at a time --
+// row a + 1 cannot win before row a has given its first entry) and keeps its best head in registers, its rows' cursors
+// in a per-group scratch.  Lists live in global memory (a chunk's scratch).
+// k_forest_kbest_paths: one thread per derivation writes its AND nodes in pre-order: a node at offset o puts slot j's
+// node at o + size(L(j-1)[a]) (L0: o + 1), so every position is filled before the walk reaches it.
+// ---------------------------------------------------------------------------------------------------
+namespace {
+const uint32_t kFkNone = 0xFFFFFFFFu;
+const int kFkWarps = 4;  // warps per block
+struct FkArgs {
+  const uint64_t* node_off;  // [n_forests + 1] the batch's pre-order arrays
+  const uint32_t* next;
+  const uint32_t* label;
+  const uint8_t* backref;
+  const uint32_t* order;     // per forest, at its node_off: its real nodes by height, then pre-order index
+  const uint32_t* lvl;       // per forest, at lvl_base: n_levels + 1 offsets into its order
+  const uint64_t* lvl_base;  // [n_forests + 1]
+  const double* ln_w;
+  uint64_t f0, s0;           // first forest of the chunk and its first node (chunk-local node = batch node - s0)
+  uint32_t n_f, k;
+  // per chunk-local pre-order node: its own list (x*) and, for a child slot of an AND node, the fold through it (f*)
+  double* xs;
+  uint2* xb;
+  uint32_t *xz, *xl;
+  double* fs;
+  uint2* fb;
+  uint32_t *fz, *fl;
+  uint32_t* prv;   // child slot of an AND node -> the previous slot (kFkNone: the first)
+  uint32_t* lst;   // AND node with children -> its last slot
+  uint2* cur;      // per lane group: cstride (child node, cursor) rows
+  uint32_t cstride;
+  double* score;   // [n_f * k] this chunk's results
+  uint32_t* n_and;
+};
+
+__device__ __forceinline__ uint32_t fk_sat(uint32_t a, uint32_t b) {  // subtree sizes saturate at kFkNone
+  const uint32_t s = a + b;
+  return s < a ? kFkNone : s;
+}
+
+template <int G>
+__device__ __forceinline__ void fk_argmax(unsigned gmask, double& v, uint32_t& q) {  // score desc, then row asc
+#pragma unroll
+  for (int o = G / 2; o > 0; o >>= 1) {
+    const double ov = __shfl_xor_sync(gmask, v, o, G);
+    const uint32_t oq = __shfl_xor_sync(gmask, q, o, G);
+    if (ov > v || (ov == v && oq < q)) {
+      v = ov;
+      q = oq;
+    }
+  }
+}
+
+// Lj = top k { P[a] + S[b] } (ties by a, then b) into (os, ob, oz); returns its length
+template <int G>
+__device__ __forceinline__ uint32_t fk_fold(unsigned gmask, uint32_t g, uint32_t k, const double* __restrict__ ps, const uint32_t* __restrict__ pz,
+                            uint32_t la, const double* __restrict__ cs, const uint32_t* __restrict__ cz, uint32_t lc,
+                            double* __restrict__ os, uint2* __restrict__ ob, uint32_t* __restrict__ oz, uint2* __restrict__ C) {
+  if (!la || !lc) return 0;
+  uint32_t act = 1;  // open rows
+  if (g == 0) C[0].y = 0;
+  double bv = g == 0 ? ps[0] + cs[0] : -CUDART_INF;
+  uint32_t ba = g == 0 ? 0u : kFkNone;
+  uint32_t r = 0;
+  for (; r < k; ++r) {
+    double v = bv;
+    uint32_t a = ba;
+    fk_argmax<G>(gmask, v, a);
+    if (!(v > -CUDART_INF)) break;  // group-uniform: no candidate left
+    const bool opened = a + 1 == act && act < la;
+    if (opened) ++act;
+    const bool mine = a % G == g, gets_row = opened && (act - 1) % G == g;
+    if (mine) {
+      const uint32_t c0 = C[a].y;
+      os[r] = v;
+      ob[r] = make_uint2(a, c0);
+      oz[r] = fk_sat(pz[a], cz[c0]);
+      C[a].y = c0 + 1;
+    }
+    if (gets_row) C[act - 1].y = 0;
+    if (mine || gets_row) {
+      bv = -CUDART_INF;
+      ba = kFkNone;
+      for (uint32_t q = g; q < act; q += G) {
+        const uint32_t c = C[q].y;
+        if (c < lc) {
+          const double h = ps[q] + cs[c];
+          if (h > bv) {
+            bv = h;
+            ba = q;
+          }
+        }
+      }
+    }
+  }
+  return r;
+}
+
+template <int G>
+__global__ void __launch_bounds__(kFkWarps * 32, 1) k_forest_kbest(FkArgs A) {
+  const uint32_t lane = threadIdx.x & 31, g = lane % G, grp = lane / G;
+  const unsigned gmask = G == 32 ? 0xFFFFFFFFu : (((1u << G) - 1u) << (grp * G));
+  const uint32_t k = A.k;
+  const uint32_t gw = blockIdx.x * kFkWarps + threadIdx.x / 32, nw = gridDim.x * kFkWarps;
+  uint2* __restrict__ C = A.cur + ((uint64_t)gw * (32 / G) + grp) * A.cstride;
+  for (uint32_t w = gw; w < A.n_f; w += nw) {
+    const uint64_t f = A.f0 + w, nb = A.node_off[f], sb = nb - A.s0;
+    const uint32_t* __restrict__ nx = A.next + nb;
+    const uint32_t* __restrict__ lb = A.label + nb;
+    const uint8_t* __restrict__ br = A.backref + nb;
+    const uint32_t* __restrict__ ord = A.order + nb;
+    const uint32_t* __restrict__ lv = A.lvl + A.lvl_base[f];
+    const uint32_t nl = (uint32_t)(A.lvl_base[f + 1] - A.lvl_base[f]) - 1;
+    double* __restrict__ XS = A.xs + sb * k;
+    uint2* __restrict__ XB = A.xb + sb * k;
+    uint32_t* __restrict__ XZ = A.xz + sb * k;
+    uint32_t* __restrict__ XL = A.xl + sb;
+    double* __restrict__ FS = A.fs + sb * k;
+    uint2* __restrict__ FB = A.fb + sb * k;
+    uint32_t* __restrict__ FZ = A.fz + sb * k;
+    uint32_t* __restrict__ FL = A.fl + sb;
+    for (uint32_t l = 0; l < nl; ++l) {
+      const uint32_t j1 = lv[l + 1];
+      for (uint32_t j = lv[l] + grp; j < j1; j += 32 / G) {  // group-uniform
+        const uint32_t p = ord[j], e = nx[p], lab = lb[p];
+        if (lab) {  // AND node
+          const double wv = A.ln_w[lab];
+          if (e == p + 1) {  // a leaf rule
+            if (g == 0) {
+              const bool ok = wv > -CUDART_INF;
+              if (ok) {
+                XS[(uint64_t)p * k] = wv;
+                XB[(uint64_t)p * k] = make_uint2(0, 0);
+                XZ[(uint64_t)p * k] = 1;
+              }
+              XL[p] = ok ? 1 : 0;
+            }
+            continue;
+          }
+          uint32_t prev = kFkNone;
+          for (uint32_t b = p + 1; b < e;) {
+            const uint32_t c = br[b] ? lb[b] : b, b1 = nx[b];
+            const bool last = b1 >= e;
+            const uint64_t o = (uint64_t)(last ? p : b) * k;
+            double* os = (last ? XS : FS) + o;
+            uint2* ob = (last ? XB : FB) + o;
+            uint32_t* oz = (last ? XZ : FZ) + o;
+            const double* cs = XS + (uint64_t)c * k;
+            const uint32_t* cz = XZ + (uint64_t)c * k;
+            const uint32_t lc = XL[c];
+            uint32_t len;
+            if (prev == kFkNone) {  // L1 = [w] + s1: the slot's list shifted by the rule weight
+              len = wv > -CUDART_INF ? min(k, lc) : 0u;
+              for (uint32_t r = g; r < len; r += G) {
+                os[r] = wv + cs[r];
+                ob[r] = make_uint2(0, r);
+                oz[r] = fk_sat(1u, cz[r]);
+              }
+            } else {
+              len = fk_fold<G>(gmask, g, k, FS + (uint64_t)prev * k, FZ + (uint64_t)prev * k, FL[prev], cs, cz, lc, os, ob, oz, C);
+            }
+            if (g == 0) {
+              (last ? XL[p] : FL[b]) = len;
+              A.prv[sb + b] = prev;
+            }
+            __syncwarp(gmask);  // the next fold reads this one
+            prev = b;
+            b = b1;
+          }
+          if (g == 0) A.lst[sb + p] = prev;
+        } else {  // OR node: merge of the children's lists, one head per child
+          double bv = -CUDART_INF;
+          uint32_t bq = kFkNone, m = 0;
+          for (uint32_t b = p + 1; b < e; b = nx[b], ++m)
+            if (m % G == g) {
+              const uint32_t c = br[b] ? lb[b] : b;
+              C[m] = make_uint2(c, 0);
+              if (XL[c] && XS[(uint64_t)c * k] > bv) {
+                bv = XS[(uint64_t)c * k];
+                bq = m;
+              }
+            }
+          double* os = XS + (uint64_t)p * k;
+          uint2* ob = XB + (uint64_t)p * k;
+          uint32_t* oz = XZ + (uint64_t)p * k;
+          uint32_t r = 0;
+          for (; r < k; ++r) {
+            double v = bv;
+            uint32_t q = bq;
+            fk_argmax<G>(gmask, v, q);
+            if (!(v > -CUDART_INF)) break;
+            if (q % G == g) {  // the owner appends the winner, advances that child's cursor and rescans its rows
+              const uint2 cc = C[q];
+              os[r] = v;
+              ob[r] = cc;
+              oz[r] = XZ[(uint64_t)cc.x * k + cc.y];
+              C[q].y = cc.y + 1;
+              bv = -CUDART_INF;
+              bq = kFkNone;
+              for (uint32_t t = g; t < m; t += G) {
+                const uint2 d = C[t];
+                if (d.y < XL[d.x]) {
+                  const double h = XS[(uint64_t)d.x * k + d.y];
+                  if (h > bv) {
+                    bv = h;
+                    bq = t;
+                  }
+                }
+              }
+            }
+          }
+          if (g == 0) XL[p] = r;
+        }
+      }
+      __syncwarp();
+    }
+    const uint32_t L0 = XL[0];  // the root
+    for (uint32_t r = lane; r < k; r += 32) {
+      A.score[(uint64_t)w * k + r] = r < L0 ? XS[r] : -CUDART_INF;
+      A.n_and[(uint64_t)w * k + r] = r < L0 ? XZ[r] : 0u;
+    }
+    __syncwarp();
+  }
+}
+
+// derivation t = (chunk forest t / k, rank t % k): its AND nodes (in-forest pre-order indices) at out[obase[t] ..]
+__global__ void k_forest_kbest_paths(FkArgs A, const uint64_t* __restrict__ obase, uint32_t* __restrict__ out,
+                                     uint32_t* __restrict__ orank) {
+  const uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  const uint32_t k = A.k;
+  if (t >= (uint64_t)A.n_f * k) return;
+  const uint32_t n = A.n_and[t];
+  if (!n) return;
+  const uint64_t f = A.f0 + t / k, nb = A.node_off[f], sb = nb - A.s0;
+  const uint32_t* __restrict__ nx = A.next + nb;
+  const uint32_t* __restrict__ lb = A.label + nb;
+  const uint8_t* __restrict__ br = A.backref + nb;
+  const uint2* __restrict__ XB = A.xb + sb * k;
+  const uint2* __restrict__ FB = A.fb + sb * k;
+  const uint32_t* __restrict__ FZ = A.fz + sb * k;
+  const uint32_t* __restrict__ prv = A.prv + sb;
+  const uint32_t* __restrict__ lst = A.lst + sb;
+  uint32_t* __restrict__ o = out + obase[t];
+  uint32_t* __restrict__ rk = orank + obase[t];
+  auto put = [&](uint32_t c, uint32_t r, uint32_t at) {  // real node c's rank r, down to the AND node it stands for
+    while (!lb[c]) {
+      const uint2 x = XB[(uint64_t)c * k + r];
+      c = x.x;
+      r = x.y;
+    }
+    o[at] = c;
+    rk[at] = r;
+  };
+  put(0, (uint32_t)(t % k), 0);
+  for (uint32_t i = 0; i < n; ++i) {
+    const uint32_t p = o[i];
+    if (nx[p] == p + 1) continue;
+    uint32_t j = lst[p];
+    uint2 bp = XB[(uint64_t)p * k + rk[i]];  // the last fold is the node's own list
+    for (;;) {  // the slots, last to first
+      const uint32_t pj = prv[j];
+      put(br[j] ? lb[j] : j, bp.y, i + (pj == kFkNone ? 1u : FZ[(uint64_t)pj * k + bp.x]));
+      if (pj == kFkNone) break;
+      bp = FB[(uint64_t)pj * k + bp.x];
+      j = pj;
+    }
+  }
+}
+}  // namespace
+
+extern "C" int cml_forests_set_kbest_scratch_mb(cml_forests* f, uint64_t mb) {
+  if (!f) return CML_ERR_ARG;
+  F_REQUIRE(mb > 0, CML_ERR_ARG, "cml_forests_set_kbest_scratch_mb: the budget must be at least 1 MiB");
+  f->kbest_scratch_mb = mb;
+  return CML_OK;
+}
+
+extern "C" int cml_forests_kbest_stats(cml_forests* f, uint64_t* scratch_bytes, uint64_t* chunks, float* kernel_ms) {
+  if (!f) return CML_ERR_ARG;
+  if (scratch_bytes) *scratch_bytes = f->kbest_scratch;
+  if (chunks) *chunks = f->kbest_chunks;
+  if (kernel_ms) *kernel_ms = f->kbest_ms;
+  return CML_OK;
+}
+
+extern "C" int cml_forests_kbest(cml_forests* f, const cml_forest_batch* b, uint32_t k, double* ln_score, uint32_t* n_and,
+                                 uint64_t* base, uint32_t* nodes, uint64_t cap) {
+  if (!f || !b || !ln_score || !n_and || !base) return CML_ERR_ARG;
+  F_REQUIRE(f->have_params, CML_ERR_STATE, "cml_forests_kbest before cml_forests_set_params");
+  F_REQUIRE(k > 0, CML_ERR_ARG, "cml_forests_kbest: k must be at least 1");
+  const uint64_t nf = b->n_forests;
+  F_REQUIRE(nf == 0 || (b->node_off && b->next && b->label && b->backref), CML_ERR_ARG, "cml_forests_kbest: null array");
+  CML_CUDA(cudaSetDevice(f->device));
+  f->kbest_ms = 0;
+  f->kbest_scratch = 0;
+  f->kbest_chunks = 0;
+  base[0] = 0;
+  if (!nf) return CML_OK;
+  for (uint64_t i = 0; i < nf; ++i) {
+    F_REQUIRE(b->node_off[i] < b->node_off[i + 1], CML_ERR_ARG, "cml_forests_kbest: empty forest");
+    F_REQUIRE(b->node_off[i + 1] - b->node_off[i] < 0x7fffffffull, CML_ERR_ARG, "cml_forests_kbest: forest too large");
+  }
+  const uint64_t n_nodes = b->node_off[nf];
+  // levelise on the host: forest_pass1's heights, real nodes sorted by (height, pre-order index)
+  std::vector<FlatForest> ff(nf);
+  std::vector<uint32_t> order(n_nodes), maxdeg(nf, 0);
+  std::vector<std::vector<uint32_t>> lv(nf);
+  {
+    unsigned nt = std::max(1u, std::min(32u, std::thread::hardware_concurrency()));
+    if (nf < 64) nt = 1;
+    std::atomic<uint64_t> nextf(0);
+    auto work = [&]() {
+      ForestScratch S;
+      for (;;) {
+        const uint64_t i0 = nextf.fetch_add(64);
+        if (i0 >= nf) break;
+        for (uint64_t i = i0; i < std::min(nf, i0 + 64); ++i) {
+          const uint64_t o = b->node_off[i];
+          const uint32_t n = (uint32_t)(b->node_off[i + 1] - o);
+          const uint32_t *nx = b->next + o, *lb = b->label + o;
+          const uint8_t* br = b->backref + o;
+          forest_pass1(n, nx, lb, br, f->rulespace, S, ff[i]);
+          if (ff[i].error) continue;
+          std::vector<uint32_t>& L = lv[i];
+          L.assign(ff[i].n_levels + 1, 0);
+          for (uint32_t p = 0; p < n; ++p)
+            if (!br[p]) {
+              ++L[S.height[p] + 1];
+              if (!lb[p]) {
+                uint32_t m = 0;
+                for (uint32_t q = p + 1; q < nx[p]; q = nx[q]) ++m;
+                maxdeg[i] = std::max(maxdeg[i], m);
+              }
+            }
+          for (uint32_t h = 0; h < ff[i].n_levels; ++h) L[h + 1] += L[h];
+          S.cnt.assign(L.begin(), L.end() - 1);
+          for (uint32_t p = 0; p < n; ++p)
+            if (!br[p]) order[o + S.cnt[S.height[p]]++] = p;
+        }
+      }
+    };
+    std::vector<std::thread> th;
+    for (unsigned t = 1; t < nt; ++t) th.emplace_back(work);
+    work();
+    for (auto& t : th) t.join();
+  }
+  std::vector<uint64_t> lvl_base(nf + 1, 0);
+  uint32_t cstride = k;
+  for (uint64_t i = 0; i < nf; ++i) {
+    if (ff[i].error) {
+      f->err = "cml_forests_kbest: forest " + std::to_string(i) +
+               (ff[i].error == 2 ? " has a cyclic back reference" : ff[i].error == 3 ? " uses a rule id beyond rulespace" : " is malformed");
+      return ff[i].error == 2 ? CML_ERR_CYCLE : CML_ERR_ARG;
+    }
+    lvl_base[i + 1] = lvl_base[i] + lv[i].size();
+    cstride = std::max(cstride, maxdeg[i]);
+  }
+  std::vector<uint32_t> lvl(lvl_base[nf]);
+  for (uint64_t i = 0; i < nf; ++i) std::copy(lv[i].begin(), lv[i].end(), lvl.begin() + lvl_base[i]);
+  lv.clear();
+  lv.shrink_to_fit();
+  // chunks of consecutive forests whose scratch fits the budget (a larger forest gets a chunk of its own)
+  const uint64_t per_node = 40ull * k + 16, budget = f->kbest_scratch_mb << 20;
+  std::vector<uint64_t> chunk(1, 0);
+  uint64_t max_nodes = 0, max_forests = 0;
+  for (uint64_t i = 0; i < nf; ++i)
+    if (i > chunk.back() && (b->node_off[i + 1] - b->node_off[chunk.back()]) * per_node > budget) chunk.push_back(i);
+  chunk.push_back(nf);
+  const uint64_t n_chunks = chunk.size() - 1;
+  for (uint64_t c = 0; c < n_chunks; ++c) {
+    max_nodes = std::max(max_nodes, b->node_off[chunk[c + 1]] - b->node_off[chunk[c]]);
+    max_forests = std::max(max_forests, chunk[c + 1] - chunk[c]);
+  }
+  cudaStream_t s = f->stream;
+  const int G = k > 16 ? 32 : 8;
+  const unsigned max_blocks = (unsigned)f->sm_count * 16u;
+  const unsigned grid_cap = std::max(1u, std::min(f_cdiv(max_forests, kFkWarps), max_blocks));
+  const uint64_t n_groups = (uint64_t)grid_cap * kFkWarps * (32 / G);
+  DevArray<uint64_t> d_off, d_lvlb, d_obase;
+  DevArray<uint32_t> d_next, d_label, d_order, d_lvl, d_xz, d_xl, d_fz, d_fl, d_prv, d_lst, d_nand, d_out, d_rank;
+  DevArray<uint8_t> d_br;
+  DevArray<double> d_xs, d_fs, d_score;
+  DevArray<uint2> d_xb, d_fb, d_cur;
+  CML_CUDA(d_off.upload(b->node_off, nf + 1, s));
+  CML_CUDA(d_next.upload(b->next, n_nodes, s));
+  CML_CUDA(d_label.upload(b->label, n_nodes, s));
+  CML_CUDA(d_br.upload(b->backref, n_nodes, s));
+  CML_CUDA(d_order.upload(order.data(), n_nodes, s));
+  CML_CUDA(d_lvl.upload(lvl.data(), lvl.size(), s));
+  CML_CUDA(d_lvlb.upload(lvl_base.data(), nf + 1, s));
+  CML_CUDA(d_xs.alloc(max_nodes * k));
+  CML_CUDA(d_xb.alloc(max_nodes * k));
+  CML_CUDA(d_xz.alloc(max_nodes * k));
+  CML_CUDA(d_xl.alloc(max_nodes));
+  CML_CUDA(d_fs.alloc(max_nodes * k));
+  CML_CUDA(d_fb.alloc(max_nodes * k));
+  CML_CUDA(d_fz.alloc(max_nodes * k));
+  CML_CUDA(d_fl.alloc(max_nodes));
+  CML_CUDA(d_prv.alloc(max_nodes));
+  CML_CUDA(d_lst.alloc(max_nodes));
+  CML_CUDA(d_cur.alloc(n_groups * cstride));
+  CML_CUDA(d_score.alloc(max_forests * k));
+  CML_CUDA(d_nand.alloc(max_forests * k));
+  CML_CUDA(d_obase.alloc(max_forests * k));
+  f->kbest_chunks = n_chunks;
+  f->kbest_scratch = max_nodes * per_node + n_groups * cstride * sizeof(uint2);
+  FkArgs A{d_off.p, d_next.p, d_label.p, d_br.p, d_order.p, d_lvl.p, d_lvlb.p, f->ln_w.p, 0, 0, 0, k,
+           d_xs.p, d_xb.p, d_xz.p, d_xl.p, d_fs.p, d_fb.p, d_fz.p, d_fl.p, d_prv.p, d_lst.p, d_cur.p, cstride,
+           d_score.p, d_nand.p};
+  struct Events {
+    cudaEvent_t e[4] = {nullptr, nullptr, nullptr, nullptr};
+    ~Events() {
+      for (auto x : e)
+        if (x) cudaEventDestroy(x);
+    }
+  } ev;
+  for (auto& x : ev.e) CML_CUDA(cudaEventCreate(&x));
+  bool fits = true, too_big = false;
+  std::vector<uint64_t> obase;
+  for (uint64_t c = 0; c < n_chunks; ++c) {
+    const uint64_t f0 = chunk[c], nfc = chunk[c + 1] - f0, e0 = f0 * k, ne = nfc * k;
+    A.f0 = f0;
+    A.s0 = b->node_off[f0];
+    A.n_f = (uint32_t)nfc;
+    const unsigned grid = std::max(1u, std::min(f_cdiv(nfc, kFkWarps), grid_cap));
+    CML_CUDA(cudaEventRecord(ev.e[0], s));
+    if (G == 32)
+      k_forest_kbest<32><<<grid, kFkWarps * 32, 0, s>>>(A);
+    else
+      k_forest_kbest<8><<<grid, kFkWarps * 32, 0, s>>>(A);
+    ++f->launches;
+    CML_CUDA(cudaGetLastError());
+    CML_CUDA(cudaEventRecord(ev.e[1], s));
+    CML_CUDA(cudaMemcpyAsync(ln_score + e0, d_score.p, ne * sizeof(double), cudaMemcpyDeviceToHost, s));
+    CML_CUDA(cudaMemcpyAsync(n_and + e0, d_nand.p, ne * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+    CML_CUDA(cudaStreamSynchronize(s));
+    float ms = 0;
+    CML_CUDA(cudaEventElapsedTime(&ms, ev.e[0], ev.e[1]));
+    f->kbest_ms += ms;
+    obase.resize(ne);
+    for (uint64_t i = 0; i < ne; ++i) {
+      obase[i] = base[e0 + i] - base[e0];
+      too_big |= n_and[e0 + i] == kFkNone;
+      base[e0 + i + 1] = base[e0 + i] + n_and[e0 + i];
+    }
+    const uint64_t total = base[e0 + ne] - base[e0];
+    fits = fits && !too_big && (!nodes || base[e0 + ne] <= cap);
+    if (!nodes || !fits || !total) continue;
+    if (d_out.n < total) {
+      CML_CUDA(d_out.alloc(total));
+      CML_CUDA(d_rank.alloc(total));
+    }
+    CML_CUDA(cudaMemcpyAsync(d_obase.p, obase.data(), ne * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
+    CML_CUDA(cudaEventRecord(ev.e[2], s));
+    k_forest_kbest_paths<<<f_cdiv(ne, 256), 256, 0, s>>>(A, d_obase.p, d_out.p, d_rank.p);
+    ++f->launches;
+    CML_CUDA(cudaGetLastError());
+    CML_CUDA(cudaEventRecord(ev.e[3], s));
+    CML_CUDA(cudaMemcpyAsync(nodes + base[e0], d_out.p, total * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+    CML_CUDA(cudaStreamSynchronize(s));
+    CML_CUDA(cudaEventElapsedTime(&ms, ev.e[2], ev.e[3]));
+    f->kbest_ms += ms;
+  }
+  F_REQUIRE(!too_big, CML_ERR_ARG, "cml_forests_kbest: a derivation has more than 2^32 - 2 AND nodes");
+  F_REQUIRE(!nodes || base[nf * k] <= cap, CML_ERR_ARG,
+            "cml_forests_kbest: nodes buffer too small (need base[n_forests * k] = " + std::to_string(base[nf * k]) + ")");
+  return CML_OK;
 }

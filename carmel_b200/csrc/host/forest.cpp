@@ -664,23 +664,18 @@ void ForestJob::write_outputs(std::ostream& log) {
     b.next = forests.next.data() + o0;
     b.label = forests.label.data() + o0;
     b.backref = forests.backref.data() + o0;
-    std::vector<uint32_t> choice(nf ? off[nf] : 0);
-    ok(cml_forests_viterbi(ctx, &b, best.data(), choice.data()));
     std::ofstream o(opt.outviterbi_file);
-    for (uint64_t f = 0; f < nf; ++f) {
+    // write_viterbi_rec (forest.hpp:590-631) without recursion: a stack of (node, next child) for the AND nodes;
+    // and_of(slot) is the AND node a child slot (AND node, OR node or shared node) stands for in the derivation
+    auto write_tree = [&](uint64_t f, auto&& and_of) {
       const uint32_t* nx = b.next + off[f];
       const uint32_t* lb = b.label + off[f];
-      const uint8_t* br = b.backref + off[f];
-      const uint32_t* ch = choice.data() + off[f];
-      o << fmt_forest_weight(best[f], dbl, opt.human_probs) << '/' << fmt_forest_weight(sum[f], dbl, opt.human_probs) << '='
-        << 100 * std::exp(best[f] - sum[f]) << "% ";
-      // write_viterbi_rec (forest.hpp:590-631) without recursion: a stack of (node, next child) for the AND nodes
       std::vector<std::pair<uint32_t, uint32_t>> st;
       uint32_t cur = 0;
       bool have = true;
       while (have || !st.empty()) {
         if (have) {
-          while (br[cur] || lb[cur] == 0) cur = br[cur] ? lb[cur] : ch[cur];  // shared node / OR node: follow
+          cur = and_of(cur);
           if (nx[cur] == cur + 1) {
             o << lb[cur];
             have = false;
@@ -703,6 +698,49 @@ void ForestJob::write_outputs(std::ostream& log) {
         have = true;
       }
       o << '\n';
+    };
+    const uint32_t K = opt.kbest;
+    if (K == 1) {
+      std::vector<uint32_t> choice(nf ? off[nf] : 0);
+      ok(cml_forests_viterbi(ctx, &b, best.data(), choice.data()));
+      for (uint64_t f = 0; f < nf; ++f) {
+        const uint32_t* lb = b.label + off[f];
+        const uint8_t* br = b.backref + off[f];
+        const uint32_t* ch = choice.data() + off[f];
+        o << fmt_forest_weight(best[f], dbl, opt.human_probs) << '/' << fmt_forest_weight(sum[f], dbl, opt.human_probs) << '='
+          << 100 * std::exp(best[f] - sum[f]) << "% ";
+        write_tree(f, [&](uint32_t c) {
+          while (br[c] || lb[c] == 0) c = br[c] ? lb[c] : ch[c];  // shared node / OR node: follow
+          return c;
+        });
+      }
+    } else {  // n lines per forest, best first; a rank past the last derivation reads "0/<sum>=0% " with no tree
+      std::vector<double> score(nf * K);
+      std::vector<uint32_t> len(nf * K), nodes(std::max<uint64_t>(1, (nf ? off[nf] : 0) * K));
+      std::vector<uint64_t> base(nf * K + 1);
+      // a derivation without shared nodes has at most one AND node per forest node; shared nodes can need more
+      int rc = cml_forests_kbest(ctx, &b, K, score.data(), len.data(), base.data(), nodes.data(), nodes.size());
+      if (rc == CML_ERR_ARG && base[nf * K] > nodes.size()) {
+        nodes.resize(base[nf * K]);
+        rc = cml_forests_kbest(ctx, &b, K, score.data(), len.data(), base.data(), nodes.data(), nodes.size());
+      }
+      ok(rc);
+      uint64_t found = 0;
+      for (uint64_t f = 0; f < nf; ++f)
+        for (uint32_t r = 0; r < K; ++r) {
+          const uint64_t i = f * K + r;
+          if (!(score[i] > kNegInfD)) {
+            o << fmt_forest_weight(score[i], dbl, opt.human_probs) << '/' << fmt_forest_weight(sum[f], dbl, opt.human_probs)
+              << "=0% \n";
+            continue;
+          }
+          ++found;
+          o << fmt_forest_weight(score[i], dbl, opt.human_probs) << '/' << fmt_forest_weight(sum[f], dbl, opt.human_probs)
+            << '=' << 100 * std::exp(score[i] - sum[f]) << "% ";
+          const uint32_t* next_and = nodes.data() + base[i];
+          write_tree(f, [&](uint32_t) { return *next_and++; });
+        }
+      log << "Viterbi: " << K << "-best lists, " << found << " derivations found\n";
     }
   }
   if (!opt.history_file.empty()) {
@@ -731,6 +769,7 @@ int open_forest_job(int argc, const char* const* argv, ForestJob& job, std::ostr
       {"tempfile-prefix", 't'},   {"forest-tick-period", 'T'},   {"watch-period", 'W'},    {"random-seed", 's'},
       {"random-restarts", 'r'},   {"checkpoint-prefix", 'x'},    {"checkpoint-parameters", 'c'}, {"outviterbi-file", 'v'}};
   ForestOpts& a = job.opt;
+  bool have_kbest = false;
   try {
     for (int i = 1; i < argc; ++i) {
       const std::string s = argv[i];
@@ -753,6 +792,14 @@ int open_forest_job(int argc, const char* const* argv, ForestJob& job, std::ostr
           continue;
         }
         if (key == "gpu") { a.device = std::atoi(val.c_str()); continue; }
+        if (key == "kbest") {
+          char* end = nullptr;
+          const unsigned long long n = val.empty() || val[0] < '0' || val[0] > '9' ? 0 : std::strtoull(val.c_str(), &end, 10);
+          if (!n || *end || n > 0xFFFFFFFFull) throw std::runtime_error("--kbest=n needs a whole number of derivations >= 1 (got \"" + val + "\")");
+          a.kbest = (uint32_t)n;
+          have_kbest = true;
+          continue;
+        }
         if (key == "crp") { a.crp_iter = (unsigned)std::atol(val.c_str()); continue; }
         if (key == "burnin") { a.crp_burnin = (unsigned)std::atol(val.c_str()); continue; }
         if (key == "const-alpha") { a.crp_alpha = std::atof(val.c_str()); continue; }
@@ -821,6 +868,8 @@ int open_forest_job(int argc, const char* const* argv, ForestJob& job, std::ostr
         default: throw std::runtime_error(std::string("unknown option -") + c);
       }
     }
+    if (have_kbest && a.outviterbi_file.empty()) throw std::runtime_error("--kbest=n needs -v (outviterbi-file)");
+    if (have_kbest && a.shard_count > 1) throw std::runtime_error("--kbest decodes on one GPU (no --gpus / --shard)");
     if (a.max_iter && a.forests_file.empty()) throw std::runtime_error("Missing forests-file.");
     if (a.normgroups_file.empty() && (a.max_iter || a.normalize_initial)) throw std::runtime_error("Missing normgroups-file.\n");
     job.load();

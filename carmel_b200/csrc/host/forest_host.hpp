@@ -58,6 +58,7 @@ struct ForestOpts {
   int device = 0;                      // --gpu=n
   int shard_rank = 0, shard_count = 1;  // --shard=r/N
   int layout = CML_FOREST_LAYOUT_AUTO;  // --layout=auto|group|thread|level (device layout family, see cml_forests_set_layout)
+  uint32_t kbest = 1;                  // --kbest=n : -v writes the n best derivations per forest (cml_forests_kbest)
   bool parse_only = false;            // --parse-only : read (and --print-forests) without touching the GPU
   // checkpoints (forest-em.hpp:166-201,621-641; forest-em-params.hpp:138-145): on every "watch" iteration (the first
   // watch_period iterations, then every watch_period-th) write <prefix>.params / <prefix>.counts

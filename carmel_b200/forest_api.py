@@ -68,6 +68,10 @@ def _lib():
         lib.cml_forests_allreduce_counts.argtypes = [_vp]
         lib.cml_forests_maximize.argtypes = [_vp, C.POINTER(CmlForestNormOpts), _f64p, _u64p]
         lib.cml_forests_normalize_params.argtypes = [_vp]
+        lib.cml_forests_viterbi.argtypes = [_vp, C.POINTER(CmlForestBatch), _f64p, _u32p]
+        lib.cml_forests_kbest.argtypes = [_vp, C.POINTER(CmlForestBatch), C.c_uint32, _f64p, _u32p, _u64p, _u32p, C.c_uint64]
+        lib.cml_forests_set_kbest_scratch_mb.argtypes = [_vp, C.c_uint64]
+        lib.cml_forests_kbest_stats.argtypes = [_vp, _u64p, _u64p, C.POINTER(C.c_float)]
         lib.cml_forest_job_open.argtypes = [C.POINTER(_vp), C.c_int, C.POINTER(C.c_char_p)]
         lib.cml_forest_job_close.argtypes = [_vp]
         lib.cml_forest_job_close.restype = None
@@ -151,11 +155,63 @@ class Forests:
         self._ok(self.lib.cml_forests_get_params(self.h, w.ctypes.data_as(_f64p)))
         return w
 
-    def add(self, node_off, nxt, label, backref):
+    @staticmethod
+    def _batch(node_off, nxt, label, backref):
+        """(cml_forest_batch, the contiguous arrays it points into: keep them alive while the batch is used)"""
         no, nx, lb, br = _arr(node_off, np.uint64), _arr(nxt, np.uint32), _arr(label, np.uint32), _arr(backref, np.uint8)
         b = CmlForestBatch(len(no) - 1, no.ctypes.data_as(_u64p), nx.ctypes.data_as(_u32p), lb.ctypes.data_as(_u32p),
                            br.ctypes.data_as(_u8p))
+        return b, (no, nx, lb, br)
+
+    def add(self, node_off, nxt, label, backref):
+        b, keep = self._batch(node_off, nxt, label, backref)
         self._ok(self.lib.cml_forests_add(self.h, C.byref(b)))
+
+    def viterbi(self, node_off, nxt, label, backref):
+        """best derivation of every forest of the batch (cml_forests_viterbi): (ln score [n_forests], chosen child of
+        every OR node [n_nodes]: in-forest pre-order index, 0xFFFFFFFF elsewhere)"""
+        b, keep = self._batch(node_off, nxt, label, backref)
+        n = int(keep[0][-1])
+        root, best = np.empty(max(b.n_forests, 1)), np.empty(max(n, 1), np.uint32)
+        self._ok(self.lib.cml_forests_viterbi(self.h, C.byref(b), root.ctypes.data_as(_f64p), best.ctypes.data_as(_u32p)))
+        return root[:b.n_forests], best[:n]
+
+    def kbest(self, k: int, node_off, nxt, label, backref, nodes: bool = True, cap: int | None = None):
+        """the k best derivations of every forest of the batch (cml_forests_kbest): (ln_score [n_forests, k],
+        n_and [n_forests, k], base [n_forests * k + 1], nodes); derivation (i, r) is nodes[base[i*k+r]:][:n_and[i, r]],
+        in-forest pre-order indices of its AND nodes.  nodes=False asks for scores and sizes only (nodes is None).
+        cap: size of the node buffer handed to the library (default: k * n_nodes, grown once if that is too small)."""
+        b, keep = self._batch(node_off, nxt, label, backref)
+        nf, n = b.n_forests, int(keep[0][-1])
+        score, lens = np.empty(max(nf * k, 1)), np.empty(max(nf * k, 1), np.uint32)
+        base = np.zeros(nf * k + 1, np.uint64)
+
+        def call(buf, c):
+            return self.lib.cml_forests_kbest(self.h, C.byref(b), k, score.ctypes.data_as(_f64p), lens.ctypes.data_as(_u32p),
+                                              base.ctypes.data_as(_u64p), buf.ctypes.data_as(_u32p) if buf is not None else None, c)
+        out = None
+        if nodes:
+            c = k * n if cap is None else cap
+            out = np.empty(max(c, 1), np.uint32)
+            rc = call(out, c)
+            if rc == -1 and cap is None and int(base[-1]) > c:
+                c = int(base[-1])
+                out = np.empty(max(c, 1), np.uint32)
+                rc = call(out, c)
+            self._ok(rc)
+            out = out[:int(base[-1])]
+        else:
+            self._ok(call(None, 0))
+        return score[:nf * k].reshape(nf, k), lens[:nf * k].reshape(nf, k), base, out
+
+    def set_kbest_scratch_mb(self, mb: int):
+        self._ok(self.lib.cml_forests_set_kbest_scratch_mb(self.h, mb))
+
+    def kbest_stats(self) -> dict:
+        """the last kbest() call: scratch bytes of its largest chunk, chunks, kernel time (CUDA events, ms)"""
+        b, c, ms = C.c_uint64(), C.c_uint64(), C.c_float()
+        self._ok(self.lib.cml_forests_kbest_stats(self.h, C.byref(b), C.byref(c), C.byref(ms)))
+        return {"scratch_bytes": b.value, "chunks": c.value, "kernel_ms": ms.value}
 
     def totals(self):
         v = [C.c_uint64() for _ in range(4)]

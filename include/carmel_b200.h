@@ -540,6 +540,42 @@ int cml_forests_gibbs_get_state(cml_forests* f, double* count, double* cum, doub
  * forest's best derivation and, per node of `b` (the batch as given to cml_forests_add), the chosen child of OR nodes
  * (in-forest pre-order index, the first child that attains the maximum; 0xFFFFFFFF elsewhere), at the current weights */
 int cml_forests_viterbi(cml_forests* f, const cml_forest_batch* b, double* root_ln, uint32_t* best_child);
+/* The k best derivations of every forest of `b` (the batch as given to cml_forests_add) at the current weights, best
+ * first (forest-em -v FILE --kbest=n).  A derivation is returned as the AND nodes (rule applications) it uses, in
+ * derivation pre-order; the tree is rebuilt from the forest alone: each child slot of an AND node (its direct pre-order
+ * child: an AND node, an OR node or a back reference) takes the next listed node, the AND node the slot resolves to.
+ *   ln_score[n_forests * k]   ln score of derivation (i, r) at [i * k + r]; -inf where forest i has fewer than r + 1
+ *   n_and[n_forests * k]      AND nodes of derivation (i, r); 0 with -inf
+ *   base[n_forests * k + 1]   derivation (i, r) is nodes[base[i * k + r] .. + n_and[i * k + r])
+ *   nodes[cap]                in-forest pre-order indices of its AND nodes, or NULL for scores and sizes only
+ * Contract:
+ *   order        each forest's derivations come in non-increasing score
+ *   distinct     they are distinct choice sets (one child per OR node reached), so k counts derivations, not unique
+ *                trees; a back-referenced shared node is expanded independently at each use
+ *   zero weight  derivations of weight zero (ln -inf) are never listed; a forest of probability zero is all padding
+ *   scores       fp64, from the handle's fp64 weights whatever its precision (as cml_forests_viterbi)
+ *   ties         an OR node's list is the top k over its children's entries by score (descending), then child
+ *                pre-order position, then child rank; an AND node with rule weight w and slots s1..sm is the left fold
+ *                L0 = [w], Lj = top k { L(j-1)[a] + sj[b] } (ties by a, then b), summed in that order; a back reference
+ *                has its shared node's list
+ *   rank 0       for every forest with a finite Viterbi score it is bit-identical to cml_forests_viterbi: the same
+ *                double and the same OR choices
+ *   determinism  the same inputs give the same bytes on every run
+ *   nesting      no depth limit: a forest nested deeper than cml_forests_viterbi's 96 levels decodes
+ *   memory       device scratch of 40 B * k + 16 B per pre-order node (a node's list and the fold through a child slot,
+ *                each 20 B per entry: score, back pointer, subtree size) plus 8 B * max(k, largest OR fan-out) per lane
+ *                group; forests are processed in chunks of consecutive forests whose scratch fits the budget of
+ *                cml_forests_set_kbest_scratch_mb (a forest larger than that gets a chunk of its own).  Results do not
+ *                depend on the chunking.
+ * Errors: CML_ERR_STATE before cml_forests_set_params; CML_ERR_ARG for k == 0, for a malformed forest, or for a non-NULL
+ * `nodes` with cap < base[n_forests * k] -- then ln_score, n_and and base are still filled, so the caller can size the
+ * buffer and call again. */
+int cml_forests_kbest(cml_forests* f, const cml_forest_batch* b, uint32_t k, double* ln_score, uint32_t* n_and,
+                      uint64_t* base, uint32_t* nodes, uint64_t cap);
+int cml_forests_set_kbest_scratch_mb(cml_forests* f, uint64_t mb); /* scratch budget of one chunk (MiB); default 4096 */
+/* the last cml_forests_kbest call: device scratch bytes of its largest chunk, chunks, and the time of its derivation
+ * kernels from CUDA events (ms) */
+int cml_forests_kbest_stats(cml_forests* f, uint64_t* scratch_bytes, uint64_t* chunks, float* kernel_ms);
 int cml_forests_synchronize(cml_forests* f);
 int cml_forests_comm_init_rank(cml_forests* f, int n_ranks, int rank, const unsigned char id[CML_COMM_ID_BYTES]);
 int cml_forests_allreduce_counts(cml_forests* f);
