@@ -20,7 +20,7 @@ NO_GROUP = 0xFFFFFFFF
 LOCKED_GROUP = 0
 
 OPT_ARC_COUNTS, OPT_NO_ELL, OPT_LANE_MIN, OPT_NO_COUNTS, OPT_NO_FACTOR, OPT_NO_WIDE = 1, 2, 3, 4, 5, 6
-OPT_KBEST_SCRATCH_MB = 9
+OPT_KBEST_SCRATCH_MB, OPT_FREE_BUILD_SCRATCH_MB = 9, 10
 OK, ERR_ARG, ERR_CUDA, ERR_STATE, ERR_CYCLE, ERR_NODERIV, ERR_NOT_DENSE = 0, -1, -2, -3, -4, -5, -6
 
 _u32p = C.POINTER(C.c_uint32)
@@ -40,6 +40,22 @@ class CmlTrellisBatch(C.Structure):
         ("n_ex", C.c_uint64), ("ex_states", _u32p), ("ex_fin", _u32p), ("ex_weight", _f64p),
         ("arc_off", _u32p), ("arc_dst", _u32p), ("arc_id", _u32p),
     ]
+
+
+class CmlWfstView(C.Structure):
+    _fields_ = [("n_states", C.c_uint32), ("final_state", C.c_uint32), ("n_arcs", C.c_uint64),
+                ("state_arc_off", _u32p), ("arc_in", _u32p), ("arc_out", _u32p), ("arc_dest", _u32p)]
+
+
+class CmlStringBatch(C.Structure):
+    _fields_ = [("n", C.c_uint64), ("off", C.POINTER(C.c_uint64)), ("sym", _u32p)]
+
+
+class CmlBuiltTrellises(C.Structure):
+    _fields_ = [("batch", CmlTrellisBatch), ("kept_example", _u32p), ("n_dropped", C.c_uint64), ("dropped", _u32p),
+                ("pre_arcs", C.c_uint64), ("launches", C.c_uint32), ("peak_states", C.c_uint32),
+                ("peak_kept_arcs", C.c_uint32), ("peak_depth", C.c_uint32), ("seconds", C.c_double),
+                ("chunks", C.c_uint64), ("kernel_ms", C.c_double), ("owner", C.c_void_p)]
 
 
 class CmlDenseView(C.Structure):
@@ -117,6 +133,10 @@ def load_library(path: str | None = None) -> C.CDLL:
     lib.cml_viterbi.argtypes = [vp, _u32p, C.POINTER(C.c_uint64), _u32p, C.c_uint64, _f64p]
     lib.cml_kbest.argtypes = [vp, C.c_uint32, _u32p, C.POINTER(C.c_uint64), _u32p, C.c_uint64, _f64p]
     lib.cml_kbest_stats.argtypes = [vp, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.POINTER(C.c_float)]
+    lib.cml_build_free_trellises.argtypes = [vp, C.POINTER(CmlWfstView), C.POINTER(CmlStringBatch), C.c_int,
+                                             C.POINTER(C.POINTER(CmlBuiltTrellises))]
+    lib.cml_free_built_trellises.argtypes = [C.POINTER(CmlBuiltTrellises)]
+    lib.cml_free_built_trellises.restype = None
     lib.cml_get_example_layout.argtypes = [vp, C.c_uint64, _u32p, _u32p, _u32p]
     lib.cml_estimate.argtypes = [vp, C.POINTER(CmlEstimateResult)]
     lib.cml_estimate_launch.argtypes = [vp]
@@ -353,6 +373,49 @@ class Context:
         b, c, ms = C.c_uint64(), C.c_uint64(), C.c_float()
         self._check(self.lib.cml_kbest_stats(self.h, C.byref(b), C.byref(c), C.byref(ms)))
         return {"scratch_bytes": b.value, "chunks": c.value, "kernel_ms": ms.value}
+
+    def build_free_trellises(self, wfst: dict, strings, given: int) -> dict:
+        """the lattices of the given strings on tape `given` (0 input, 1 output) x the machine, the other tape free
+        (cml_build_free_trellises).  wfst: n_states, final_state, state_arc_off, arc_in, arc_out, arc_dest (arc-table
+        order, start = state 0); strings: a list of symbol-id sequences, or (off, sym) arrays as the C ABI takes them.
+        Returns the batch as numpy arrays (n_ex, ex_states, ex_fin, ex_weight, arc_off, arc_dst, arc_id), kept (string
+        index of every lattice), dropped, and the call's statistics; the size of the scratch of one chunk is the option
+        OPT_FREE_BUILD_SCRATCH_MB (set_option)."""
+        v = CmlWfstView()
+        soff, ain, aout, adst = (_u32(wfst[k]) for k in ("state_arc_off", "arc_in", "arc_out", "arc_dest"))
+        v.n_states, v.final_state, v.n_arcs = int(wfst["n_states"]), int(wfst["final_state"]), ain.size
+        v.state_arc_off, v.arc_in, v.arc_out, v.arc_dest = (_ptr(a, _u32p) for a in (soff, ain, aout, adst))
+        if isinstance(strings, tuple):
+            off, sym = np.ascontiguousarray(strings[0], np.uint64), _u32(strings[1])
+        else:
+            off = np.zeros(len(strings) + 1, np.uint64)
+            off[1:] = np.cumsum([len(q) for q in strings])
+            sym = _u32(np.concatenate([np.asarray(q, np.uint32) for q in strings]) if len(strings) else [])
+        sb = CmlStringBatch()
+        sb.n = off.size - 1
+        sb.off = off.ctypes.data_as(C.POINTER(C.c_uint64))
+        sb.sym = _ptr(sym if sym.size else np.zeros(1, np.uint32), _u32p)
+        out = C.POINTER(CmlBuiltTrellises)()
+        self._check(self.lib.cml_build_free_trellises(self.h, C.byref(v), C.byref(sb), int(given), C.byref(out)))
+        try:
+            b = out.contents
+            t = b.batch
+            n_ex = int(t.n_ex)
+            ex_states = np.ctypeslib.as_array(t.ex_states, (n_ex,)).copy() if n_ex else np.zeros(0, np.uint32)
+            rows = int(ex_states.astype(np.int64).sum()) + n_ex
+            take = lambda p, k, dt: np.ctypeslib.as_array(p, (k,)).copy() if k else np.zeros(0, dt)
+            arc_off = take(t.arc_off, rows, np.uint32)
+            ends = np.cumsum(ex_states.astype(np.int64) + 1) - 1  # each lattice's last row: its arc count
+            n_arcs = int(arc_off[ends].astype(np.int64).sum()) if n_ex else 0
+            return dict(n_ex=n_ex, ex_states=ex_states, ex_fin=take(t.ex_fin, n_ex, np.uint32),
+                        ex_weight=take(t.ex_weight, n_ex, np.float64), arc_off=arc_off,
+                        arc_dst=take(t.arc_dst, n_arcs, np.uint32), arc_id=take(t.arc_id, n_arcs, np.uint32),
+                        kept=take(b.kept_example, n_ex, np.uint32), dropped=take(b.dropped, int(b.n_dropped), np.uint32),
+                        stats=dict(launches=int(b.launches), peak_states=int(b.peak_states),
+                                   peak_kept_arcs=int(b.peak_kept_arcs), seconds=float(b.seconds),
+                                   chunks=int(b.chunks), kernel_ms=float(b.kernel_ms)))
+        finally:
+            self.lib.cml_free_built_trellises(out)
 
     def example_layout(self, e: int, n_states: int):
         nl = C.c_uint32()

@@ -278,6 +278,172 @@ __global__ void __launch_bounds__(128) k_build_trellis(BArgs A) {
   }
 }
 
+// ---- lattices of one given string, the other tape free (carmel_b200.h, cml_build_free_trellises) ---------------------
+// One warp per string over a cell grid (t, q), t in [0, |s|], q a machine state; cell (t, q) of string e is
+// cell_base[e] + t * Q + q in the three scratch arrays.  Pass 0 (count): forward reachability (fw), co-reachability of
+// the reachable cells (kept), then the state ids in (t, eps-level, q) order and the sizes.  Pass 1 (fill): the same
+// order again, each kept state's row offset and its kept arcs (eps group and s[t] group merged back into arc-table
+// order) written at the string's place in the chunk's output.
+constexpr int kFreeWarps = 4;  // warps per block
+
+struct FArgs {
+  const uint32_t* key_off;    // [Q + 1] per state: its range in keys
+  const uint32_t* keys;       // per state, ascending: the given-tape symbols its arcs carry (0 = *e* first)
+  const uint32_t* grp;        // per key: begin in ids (end = next entry)
+  const uint32_t* ids;        // arc-table ids grouped by (state, given symbol), each group in arc-table order
+  const uint32_t* dest;       // [n_arcs]
+  const uint32_t* order;      // [Q] states sorted by (eps-level, state)
+  const uint32_t* lvl_off;    // [L + 1] eps-level l is order[lvl_off[l] .. lvl_off[l + 1])
+  uint32_t Q, L, final_state;
+  const uint64_t* s_off;      // [n + 1]
+  const uint32_t* sym;
+  uint64_t e0;                // first string of the chunk
+  uint32_t n_list;            // strings of the chunk
+  const uint64_t* cell_base;  // [n] first cell of each string (relative to its chunk)
+  uint8_t* fw;
+  uint8_t* kept;
+  uint32_t* id;
+  uint32_t* n_st;             // [n] kept states (0: no derivation)
+  uint32_t* n_arc;            // [n] kept arcs
+  int fill;
+  const uint64_t* row_base;   // [n] first arc_off entry of the string in the chunk's output (fill)
+  const uint64_t* arc_base;   // [n] first arc (fill)
+  uint32_t* out_off;
+  uint32_t* out_dst;
+  uint32_t* out_id;
+};
+
+// [begin, end) in ids of the arcs of state q whose given-tape label is `symbol`
+__device__ __forceinline__ uint2 f_group(const uint32_t* __restrict__ key_off, const uint32_t* __restrict__ keys,
+                                         const uint32_t* __restrict__ grp, uint32_t q, uint32_t symbol) {
+  uint32_t lo = key_off[q], hi = key_off[q + 1];
+  const uint32_t end = hi;
+  while (lo < hi) {
+    const uint32_t mid = (lo + hi) >> 1;
+    if (keys[mid] < symbol) lo = mid + 1;
+    else hi = mid;
+  }
+  if (lo < end && keys[lo] == symbol) return make_uint2(grp[lo], grp[lo + 1]);
+  return make_uint2(0, 0);
+}
+
+__global__ void k_build_free(FArgs A) {
+  const uint32_t lane = threadIdx.x & 31;
+  const uint32_t Q = A.Q, L = A.L;
+  for (uint32_t w = blockIdx.x * kFreeWarps + threadIdx.x / 32; w < A.n_list; w += gridDim.x * kFreeWarps) {
+    const uint64_t e = A.e0 + w;
+    const uint32_t* __restrict__ s = A.sym + A.s_off[e];
+    const uint32_t n = (uint32_t)(A.s_off[e + 1] - A.s_off[e]);
+    const uint64_t cb = A.cell_base[e];
+    uint8_t* __restrict__ fw = A.fw + cb;
+    uint8_t* __restrict__ kept = A.kept + cb;
+    uint32_t* __restrict__ id = A.id + cb;
+    const uint32_t *key_off = A.key_off, *keys = A.keys, *grp = A.grp;
+    // the arcs of q leaving position t: the *e* group (same position), the s[t] group (next position)
+    auto eps_group = [=](uint32_t q) { return f_group(key_off, keys, grp, q, 0u); };
+    auto sym_group = [=](uint32_t q, uint32_t t) {
+      return (t < n && s[t] != 0u) ? f_group(key_off, keys, grp, q, s[t]) : make_uint2(0, 0);
+    };
+    if (!A.fill) {
+      // forward: reachability from (0, 0); the cells are zero on entry
+      if (lane == 0) fw[0] = 1;
+      __syncwarp();
+      for (uint32_t t = 0; t <= n; ++t) {
+        const uint64_t row = (uint64_t)t * Q;
+        for (uint32_t l = 0; l < L; ++l) {
+          for (uint32_t j = A.lvl_off[l] + lane; j < A.lvl_off[l + 1]; j += 32) {
+            const uint32_t q = A.order[j];
+            if (!fw[row + q]) continue;
+            const uint2 ge = eps_group(q), gs = sym_group(q, t);
+            for (uint32_t k = ge.x; k < ge.y; ++k) fw[row + A.dest[A.ids[k]]] = 1;  // a later eps-level of this position
+            for (uint32_t k = gs.x; k < gs.y; ++k) fw[row + Q + A.dest[A.ids[k]]] = 1;
+          }
+          __syncwarp();
+        }
+      }
+      // backward: a reachable cell is kept when it is the goal or an arc leads to a kept cell
+      for (uint32_t t = n + 1; t-- > 0;) {
+        const uint64_t row = (uint64_t)t * Q;
+        for (uint32_t l = L; l-- > 0;) {
+          for (uint32_t j = A.lvl_off[l] + lane; j < A.lvl_off[l + 1]; j += 32) {
+            const uint32_t q = A.order[j];
+            uint8_t k = 0;
+            if (fw[row + q]) {
+              k = (t == n && q == A.final_state);
+              const uint2 ge = eps_group(q), gs = sym_group(q, t);
+              for (uint32_t a = ge.x; a < ge.y && !k; ++a) k = kept[row + A.dest[A.ids[a]]];
+              for (uint32_t a = gs.x; a < gs.y && !k; ++a) k = kept[row + Q + A.dest[A.ids[a]]];
+            }
+            kept[row + q] = k;
+          }
+          __syncwarp();
+        }
+      }
+    }
+    if (!kept[0]) {  // (0, 0) does not reach the goal: no derivation
+      if (!A.fill && lane == 0) A.n_st[e] = A.n_arc[e] = 0;
+      continue;
+    }
+    // numbering in (t, eps-level, q) order; arcs counted (pass 0) or written (pass 1) in the same order
+    uint32_t* __restrict__ off = A.fill ? A.out_off + A.row_base[e] : nullptr;
+    uint32_t* __restrict__ odst = A.fill ? A.out_dst + A.arc_base[e] : nullptr;
+    uint32_t* __restrict__ oid = A.fill ? A.out_id + A.arc_base[e] : nullptr;
+    uint32_t next_id = 0, next_arc = 0;
+    for (uint32_t t = 0; t <= n; ++t) {
+      const uint64_t row = (uint64_t)t * Q;
+      for (uint32_t j0 = 0; j0 < Q; j0 += 32) {
+        const uint32_t j = j0 + lane;
+        const uint32_t q = j < Q ? A.order[j] : 0u;
+        const bool k = j < Q && kept[row + q];
+        uint2 ge = make_uint2(0, 0), gs = make_uint2(0, 0);
+        uint32_t cnt = 0;
+        if (k) {
+          ge = eps_group(q);
+          gs = sym_group(q, t);
+          for (uint32_t a = ge.x; a < ge.y; ++a) cnt += kept[row + A.dest[A.ids[a]]];
+          for (uint32_t a = gs.x; a < gs.y; ++a) cnt += kept[row + Q + A.dest[A.ids[a]]];
+        }
+        const unsigned bal = __ballot_sync(0xFFFFFFFFu, k);
+        uint32_t incl = cnt;  // inclusive warp scan of the arc counts
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+          const uint32_t v = __shfl_up_sync(0xFFFFFFFFu, incl, o);
+          if ((int)lane >= o) incl += v;
+        }
+        if (k) {
+          const uint32_t my_id = next_id + __popc(bal & ((1u << lane) - 1u));
+          if (!A.fill) {
+            id[row + q] = my_id;
+          } else {  // row offset, then the eps group and the s[t] group merged back into arc-table order
+            uint32_t p = next_arc + incl - cnt;
+            off[my_id] = p;
+            uint32_t a = ge.x, b = gs.x;
+            while (a < ge.y || b < gs.y) {
+              const bool take_e = b >= gs.y || (a < ge.y && A.ids[a] < A.ids[b]);
+              const uint32_t arc = take_e ? A.ids[a++] : A.ids[b++];
+              const uint64_t dc = (take_e ? row : row + Q) + A.dest[arc];
+              if (!kept[dc]) continue;
+              odst[p] = id[dc];
+              oid[p] = arc;
+              ++p;
+            }
+          }
+        }
+        next_id += __popc(bal);
+        next_arc += __shfl_sync(0xFFFFFFFFu, incl, 31);
+      }
+    }
+    if (lane == 0) {
+      if (A.fill)
+        off[next_id] = next_arc;
+      else {
+        A.n_st[e] = next_id;
+        A.n_arc[e] = next_arc;
+      }
+    }
+  }
+}
+
 struct BuiltOwner {
   std::vector<uint32_t> ex_states, ex_fin, arc_off, arc_dst, arc_id, kept_example, dropped;
   std::vector<double> ex_weight;
@@ -522,6 +688,265 @@ extern "C" int cml_build_trellises(cml_ctx* ctx, const cml_wfst_view* x, const c
   P.peak_states = peak[0];
   P.peak_kept_arcs = peak[1];
   P.peak_depth = peak[2];
+  P.seconds = std::chrono::duration<double>(std::chrono::steady_clock::now() - t_start).count();
+  P.owner = own.get();
+  *out = &own.release()->pub;
+  return CML_OK;
+}
+
+extern "C" int cml_build_free_trellises(cml_ctx* ctx, const cml_wfst_view* x, const cml_string_batch* sb, int given_tape,
+                                        cml_built_trellises** out) {
+  if (!ctx) return CML_ERR_ARG;
+  CML_REQUIRE(x && sb && out, CML_ERR_ARG, "cml_build_free_trellises: null argument");
+  *out = nullptr;
+  CML_REQUIRE(given_tape == 0 || given_tape == 1, CML_ERR_ARG, "cml_build_free_trellises: the given tape must be 0 (input) or 1 (output)");
+  CML_REQUIRE(x->n_states >= 1 && x->state_arc_off && (x->n_arcs == 0 || (x->arc_in && x->arc_out && x->arc_dest)), CML_ERR_ARG,
+              "cml_build_free_trellises: incomplete transducer view");
+  CML_REQUIRE(x->final_state < x->n_states, CML_ERR_ARG, "cml_build_free_trellises: final state out of range");
+  CML_REQUIRE(x->n_arcs < 0xFFFFFFFFull, CML_ERR_ARG, "cml_build_free_trellises: too many arcs");
+  const auto t_start = std::chrono::steady_clock::now();
+  const uint32_t Q = x->n_states;
+  const uint64_t n_arcs = x->n_arcs, n = sb->n;
+  CML_REQUIRE(x->state_arc_off[0] == 0 && x->state_arc_off[Q] == n_arcs, CML_ERR_ARG,
+              "cml_build_free_trellises: state_arc_off must run from 0 to n_arcs");
+  for (uint32_t q = 0; q < Q; ++q)
+    CML_REQUIRE(x->state_arc_off[q] <= x->state_arc_off[q + 1], CML_ERR_ARG, "cml_build_free_trellises: state_arc_off not monotone");
+  for (uint64_t a = 0; a < n_arcs; ++a)
+    CML_REQUIRE(x->arc_dest[a] < Q, CML_ERR_ARG, "cml_build_free_trellises: arc destination out of range");
+  CML_REQUIRE(n < 0xFFFFFFFFull, CML_ERR_ARG, "cml_build_free_trellises: too many strings");
+  CML_REQUIRE(n == 0 || (sb->off && sb->off[0] == 0 && (sb->off[n] == 0 || sb->sym)), CML_ERR_ARG,
+              "cml_build_free_trellises: incomplete string batch (off[0] must be 0)");
+  for (uint64_t e = 0; e < n; ++e) {
+    CML_REQUIRE(sb->off[e] <= sb->off[e + 1], CML_ERR_ARG, "cml_build_free_trellises: string offsets not monotone");
+    CML_REQUIRE((sb->off[e + 1] - sb->off[e] + 1) * Q < 0xFFFFFFFFull, CML_ERR_ARG,
+                "cml_build_free_trellises: a string's lattice would have more than 2^32 states");
+    // (|s| + 1) * n_arcs bounds the lattice's arcs, which the kernel counts in 32 bits (and arc_off holds)
+    CML_REQUIRE((sb->off[e + 1] - sb->off[e] + 1) * n_arcs < 0xFFFFFFFFull, CML_ERR_ARG,
+                "cml_build_free_trellises: a string's lattice could have more than 2^32 arcs");
+  }
+  const uint32_t* glab = given_tape == 0 ? x->arc_in : x->arc_out;
+  // ---- eps-levels: longest-path depth in the subgraph of the arcs with *e* on the given tape (Kahn's order)
+  std::vector<uint32_t> level(Q, 0), indeg(Q, 0), topo;
+  for (uint64_t a = 0; a < n_arcs; ++a)
+    if (glab[a] == 0) ++indeg[x->arc_dest[a]];
+  topo.reserve(Q);
+  for (uint32_t q = 0; q < Q; ++q)
+    if (!indeg[q]) topo.push_back(q);
+  for (size_t i = 0; i < topo.size(); ++i) {
+    const uint32_t q = topo[i];
+    for (uint32_t a = x->state_arc_off[q]; a < x->state_arc_off[q + 1]; ++a) {
+      if (glab[a] != 0) continue;
+      const uint32_t d = x->arc_dest[a];
+      level[d] = std::max(level[d], level[q] + 1);
+      if (--indeg[d] == 0) topo.push_back(d);
+    }
+  }
+  CML_REQUIRE(topo.size() == Q, CML_ERR_CYCLE,
+              std::string("cml_build_free_trellises: the arcs with *e* on the given ") + (given_tape ? "output" : "input") +
+                  " tape form a cycle, so a string would have unboundedly many derivations (given-*e* cycles are not decoded)");
+  std::vector<uint32_t> order(Q);
+  std::iota(order.begin(), order.end(), 0u);
+  std::stable_sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return level[a] < level[b]; });
+  const uint32_t L = level[order.back()] + 1;
+  std::vector<uint32_t> lvl_off(L + 1, 0);
+  for (uint32_t q = 0; q < Q; ++q) ++lvl_off[level[q] + 1];
+  for (uint32_t l = 0; l < L; ++l) lvl_off[l + 1] += lvl_off[l];
+  // ---- given-symbol index: per state the arc-table ids grouped by given-tape symbol, groups ascending, ids of a group
+  // in arc-table order
+  std::vector<uint32_t> key_off(Q + 1, 0), keys, grp, ids;
+  {
+    std::vector<std::pair<uint32_t, uint32_t>> tmp;
+    ids.reserve(n_arcs);
+    for (uint32_t q = 0; q < Q; ++q) {
+      tmp.clear();
+      for (uint32_t a = x->state_arc_off[q]; a < x->state_arc_off[q + 1]; ++a) tmp.emplace_back(glab[a], a);
+      std::stable_sort(tmp.begin(), tmp.end(), [](auto const& p, auto const& r) { return p.first < r.first; });
+      for (size_t i = 0; i < tmp.size(); ++i) {
+        if (i == 0 || tmp[i].first != tmp[i - 1].first) {
+          keys.push_back(tmp[i].first);
+          grp.push_back((uint32_t)ids.size());
+        }
+        ids.push_back(tmp[i].second);
+      }
+      key_off[q + 1] = (uint32_t)keys.size();
+    }
+    grp.push_back((uint32_t)ids.size());
+  }
+  // ---- chunks of consecutive strings whose cells (6 B each) fit the budget
+  const uint64_t budget = (uint64_t)ctx->opt_free_build_scratch_mb << 20;
+  std::vector<uint64_t> cell_base(n + 1, 0), chunk_begin(1, 0);
+  uint64_t cells = 0, max_cells = 0;
+  for (uint64_t e = 0; e < n; ++e) {
+    const uint64_t c = (sb->off[e + 1] - sb->off[e] + 1) * Q;
+    if (cells && (cells + c) * 6 > budget) {
+      chunk_begin.push_back(e);
+      max_cells = std::max(max_cells, cells);
+      cells = 0;
+    }
+    cell_base[e] = cells;
+    cells += c;
+  }
+  max_cells = std::max(max_cells, cells);
+  chunk_begin.push_back(n);
+  const uint64_t n_chunks = chunk_begin.size() - 1;
+
+  CML_CUDA(cudaSetDevice(ctx->device));
+  cudaStream_t st = ctx->stream;
+  DevArray<uint32_t> d_key_off, d_keys, d_grp, d_ids, d_dest, d_order, d_lvl_off, d_sym, d_nst, d_narc;
+  DevArray<uint64_t> d_soff, d_cell_base, d_row_base, d_arc_base;
+  DevArray<uint8_t> d_fw, d_kept;
+  DevArray<uint32_t> d_id, d_off, d_dst, d_aid;
+  CML_CUDA(d_key_off.upload(key_off.data(), key_off.size(), st));
+  CML_CUDA(d_keys.upload(keys.data(), keys.size(), st));
+  CML_CUDA(d_grp.upload(grp.data(), grp.size(), st));
+  CML_CUDA(d_ids.upload(ids.data(), ids.size(), st));
+  CML_CUDA(d_dest.upload(x->arc_dest, n_arcs, st));
+  CML_CUDA(d_order.upload(order.data(), Q, st));
+  CML_CUDA(d_lvl_off.upload(lvl_off.data(), lvl_off.size(), st));
+  static const uint64_t zero1[1] = {0};
+  CML_CUDA(d_soff.upload(n ? sb->off : zero1, n + 1, st));
+  CML_CUDA(d_sym.upload(sb->sym, n ? sb->off[n] : 0, st));
+  CML_CUDA(d_cell_base.upload(cell_base.data(), n + 1, st));
+  CML_CUDA(d_nst.alloc(n + 1));
+  CML_CUDA(d_narc.alloc(n + 1));
+  CML_CUDA(d_row_base.alloc(n + 1));
+  CML_CUDA(d_arc_base.alloc(n + 1));
+  CML_CUDA(d_fw.alloc(std::max<uint64_t>(1, max_cells)));
+  CML_CUDA(d_kept.alloc(std::max<uint64_t>(1, max_cells)));
+  CML_CUDA(d_id.alloc(std::max<uint64_t>(1, max_cells)));
+  struct Events {
+    cudaEvent_t a = nullptr, b = nullptr;
+    ~Events() {
+      if (a) cudaEventDestroy(a);
+      if (b) cudaEventDestroy(b);
+    }
+  } ev;
+  CML_CUDA(cudaEventCreate(&ev.a));
+  CML_CUDA(cudaEventCreate(&ev.b));
+
+  std::unique_ptr<BuiltOwner> own(new BuiltOwner());
+  std::vector<uint32_t> nst(n + 1), narc(n + 1);
+  std::vector<uint64_t> row_base(n + 1, 0), arc_base(n + 1, 0);
+  uint32_t launches = 0, peak_states = 0, peak_arcs = 0;
+  double kernel_ms = 0;
+  FArgs A{};
+  A.key_off = d_key_off.p;
+  A.keys = d_keys.p;
+  A.grp = d_grp.p;
+  A.ids = d_ids.p;
+  A.dest = d_dest.p;
+  A.order = d_order.p;
+  A.lvl_off = d_lvl_off.p;
+  A.Q = Q;
+  A.L = L;
+  A.final_state = x->final_state;
+  A.s_off = d_soff.p;
+  A.sym = d_sym.p;
+  A.cell_base = d_cell_base.p;
+  A.fw = d_fw.p;
+  A.kept = d_kept.p;
+  A.id = d_id.p;
+  A.n_st = d_nst.p;
+  A.n_arc = d_narc.p;
+  A.row_base = d_row_base.p;
+  A.arc_base = d_arc_base.p;
+  const unsigned max_blocks = (unsigned)ctx->sm_count * 16u;
+  for (uint64_t c = 0; c < n_chunks; ++c) {
+    const uint64_t e0 = chunk_begin[c], e1 = chunk_begin[c + 1];
+    if (e0 == e1) continue;
+    const uint64_t chunk_cells = (e1 < n ? cell_base[e1 - 1] + (sb->off[e1] - sb->off[e1 - 1] + 1) * Q : cells);
+    CML_CUDA(cudaMemsetAsync(d_fw.p, 0, chunk_cells, st));
+    A.e0 = e0;
+    A.n_list = (uint32_t)(e1 - e0);
+    const unsigned grid = std::max(1u, std::min(cdiv(e1 - e0, kFreeWarps), max_blocks));
+    float ms = 0;
+    // pass 0: reachability, ids, sizes
+    A.fill = 0;
+    CML_CUDA(cudaEventRecord(ev.a, st));
+    k_build_free<<<grid, kFreeWarps * 32, 0, st>>>(A);
+    CML_CUDA(cudaGetLastError());
+    CML_CUDA(cudaEventRecord(ev.b, st));
+    ++launches;
+    ++ctx->launches;
+    CML_CUDA(cudaMemcpyAsync(nst.data() + e0, d_nst.p + e0, (e1 - e0) * 4, cudaMemcpyDeviceToHost, st));
+    CML_CUDA(cudaMemcpyAsync(narc.data() + e0, d_narc.p + e0, (e1 - e0) * 4, cudaMemcpyDeviceToHost, st));
+    CML_CUDA(cudaStreamSynchronize(st));
+    CML_CUDA(cudaEventElapsedTime(&ms, ev.a, ev.b));
+    kernel_ms += ms;
+    // exclusive scan of the kept lattices' sizes: their places in the chunk's output
+    uint64_t rows = 0, arcs = 0;
+    for (uint64_t e = e0; e < e1; ++e) {
+      row_base[e] = rows;
+      arc_base[e] = arcs;
+      if (nst[e]) {
+        rows += (uint64_t)nst[e] + 1;
+        arcs += narc[e];
+        peak_states = std::max(peak_states, nst[e]);
+        peak_arcs = std::max(peak_arcs, narc[e]);
+      }
+    }
+    if (!rows) {
+      for (uint64_t e = e0; e < e1; ++e) own->dropped.push_back((uint32_t)e);
+      continue;
+    }
+    // pass 1: rows and arcs at their places (the cells of pass 0 are still in the scratch)
+    CML_CUDA(cudaMemcpyAsync(d_row_base.p + e0, row_base.data() + e0, (e1 - e0) * 8, cudaMemcpyHostToDevice, st));
+    CML_CUDA(cudaMemcpyAsync(d_arc_base.p + e0, arc_base.data() + e0, (e1 - e0) * 8, cudaMemcpyHostToDevice, st));
+    if (d_off.n < rows) CML_CUDA(d_off.alloc(rows));
+    if (d_dst.n < std::max<uint64_t>(1, arcs)) {
+      CML_CUDA(d_dst.alloc(std::max<uint64_t>(1, arcs)));
+      CML_CUDA(d_aid.alloc(std::max<uint64_t>(1, arcs)));
+    }
+    A.fill = 1;
+    A.out_off = d_off.p;
+    A.out_dst = d_dst.p;
+    A.out_id = d_aid.p;
+    CML_CUDA(cudaEventRecord(ev.a, st));
+    k_build_free<<<grid, kFreeWarps * 32, 0, st>>>(A);
+    CML_CUDA(cudaGetLastError());
+    CML_CUDA(cudaEventRecord(ev.b, st));
+    ++launches;
+    ++ctx->launches;
+    const size_t r0 = own->arc_off.size(), a0 = own->arc_dst.size();
+    own->arc_off.resize(r0 + rows);
+    own->arc_dst.resize(a0 + arcs);
+    own->arc_id.resize(a0 + arcs);
+    CML_CUDA(cudaMemcpyAsync(own->arc_off.data() + r0, d_off.p, rows * 4, cudaMemcpyDeviceToHost, st));
+    if (arcs) {
+      CML_CUDA(cudaMemcpyAsync(own->arc_dst.data() + a0, d_dst.p, arcs * 4, cudaMemcpyDeviceToHost, st));
+      CML_CUDA(cudaMemcpyAsync(own->arc_id.data() + a0, d_aid.p, arcs * 4, cudaMemcpyDeviceToHost, st));
+    }
+    CML_CUDA(cudaStreamSynchronize(st));
+    CML_CUDA(cudaEventElapsedTime(&ms, ev.a, ev.b));
+    kernel_ms += ms;
+    for (uint64_t e = e0; e < e1; ++e) {
+      if (!nst[e]) {
+        own->dropped.push_back((uint32_t)e);
+        continue;
+      }
+      own->kept_example.push_back((uint32_t)e);
+      own->ex_states.push_back(nst[e]);
+      own->ex_fin.push_back(nst[e] - 1);
+      own->ex_weight.push_back(1.0);
+    }
+  }
+  cml_built_trellises& P = own->pub;
+  std::memset(&P, 0, sizeof(P));
+  P.batch.n_ex = own->kept_example.size();
+  P.batch.ex_states = own->ex_states.data();
+  P.batch.ex_fin = own->ex_fin.data();
+  P.batch.ex_weight = own->ex_weight.data();
+  P.batch.arc_off = own->arc_off.data();
+  P.batch.arc_dst = own->arc_dst.data();
+  P.batch.arc_id = own->arc_id.data();
+  P.kept_example = own->kept_example.data();
+  P.n_dropped = own->dropped.size();
+  P.dropped = own->dropped.data();
+  P.launches = launches;
+  P.peak_states = peak_states;
+  P.peak_kept_arcs = peak_arcs;
+  P.chunks = n_chunks;
+  P.kernel_ms = kernel_ms;
   P.seconds = std::chrono::duration<double>(std::chrono::steady_clock::now() - t_start).count();
   P.owner = own.get();
   *out = &own.release()->pub;

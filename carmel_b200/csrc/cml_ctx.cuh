@@ -140,6 +140,7 @@ struct cml_ctx {
   int opt_no_factor = 0;     // CML_OPT_NO_FACTOR: keep per-arc weight records (no arc classes; round-1 kernels)
   int opt_no_wide = 0;       // CML_OPT_NO_WIDE: wide lattices stay on the k_fb_ell classes
   int opt_kbest_scratch_mb = 4096;  // CML_OPT_KBEST_SCRATCH_MB: list scratch of one cml_kbest chunk
+  int opt_free_build_scratch_mb = 4096;  // CML_OPT_FREE_BUILD_SCRATCH_MB: cell scratch of one cml_build_free_trellises chunk
   // last cml_kbest / cml_viterbi call (cml_kbest_stats)
   uint64_t kbest_scratch = 0, kbest_chunks = 0;
   float kbest_ms = 0;

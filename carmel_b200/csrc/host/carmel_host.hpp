@@ -90,6 +90,9 @@ struct Corpus {
   double total_weight = 0, n_input = 0, n_output = 0;
   void count();
   void read(std::istream& in, Wfst& x);
+  // one string per line (an empty line is the empty string) on tape 0 (input) or 1 (output) of x: the strings
+  // --decode reads, kept as examples whose other side is empty
+  void read_strings(std::istream& in, Wfst& x, int tape);
 };
 
 // ---- cascade: composed arc -> chain of original parameters (cascade.h) --------------------------
@@ -160,6 +163,7 @@ struct TrainOpts {
   uint64_t seed = 1;                // -R seed : the restarts' generator (the reference seeds boost's lagged Fibonacci; draws differ)
   std::string kbest_arg;            // -k n : derivations per example written by --viterbi (unused when training)
   uint32_t kbest = 1;
+  int given_tape = -1;              // --given=input|output : the tape --decode reads its strings on (0 / 1)
   TrainOpts();
 };
 // WFST::random_restart_acceptor (fst.h:999-1044): a further start must be, after its first iteration, within a
@@ -240,6 +244,7 @@ struct TrainJob {
   void export_fem_tables(std::ostream& log);        // --fem-norm / --fem-param, after training (fem.cpp)
   void export_fem_forest(TrellisBatch const& tb, std::ostream& log);  // --fem-forest, from prepare()
   void load_fem_param(std::string const& file);     // --load-fem-param
+  void prepare_model();  // context, model, parameters after the initial normalisation (the first part of prepare)
   void prepare();
   bool try_dense(int tape, Corpus const& local, std::vector<uint32_t>& kept, std::vector<uint32_t>& dropped);
   double estimate(double& ln_unweighted);
@@ -250,6 +255,10 @@ struct TrainJob {
   // kept example: ln weight, number of arcs, arc-table ids; then, per arc, the (input:output) labels of the cascade
   // members' arcs it stands for (decode side: carmel -k 1 on the composed machine, fst.h:769-800)
   void run_viterbi(std::ostream& log, std::string const& path);
+  // --decode=FILE --given=input|output: the -k n best derivations of every string of the corpus file on the given tape
+  // with the other tape free (carmel -sri / -sli ... -k n), n lines per string in file order: the --viterbi line, then
+  // " ||" and the free-tape labels of the path; "-inf 0 | ||" past the last derivation or for a string without one
+  void run_decode(std::ostream& log, std::string const& path);
   void attach_dense_sampler();  // batched --crp on position-synchronous lattices: cml_gibbs_attach_dense  // lattices + CRP parameters on the GPU, counts = priors; no sweep yet
   bool gibbs_prepared = false;
   std::vector<uint32_t> g_norm;  // CRP normalisation group of every parameter (kNoGroup = fixed probability)

@@ -8,6 +8,7 @@
 // sweep (gibbs.hpp:712-742) is a strictly sequential product over the corpus and is computed here from
 // the downloaded sample paths.
 #include <algorithm>
+#include <chrono>
 #include <fstream>
 #include <iostream>
 #include <stdexcept>
@@ -317,6 +318,35 @@ TrainResult const& TrainJob::run_gibbs(std::ostream& log) {
   return res;
 }
 
+namespace {
+
+// labels of every parameter's member arc (parameters are numbered member by member, state by state, arc by arc)
+std::vector<std::string> param_labels(std::vector<Wfst*> const& members) {
+  std::vector<std::string> plabel;
+  for (Wfst* m : members)
+    for (auto& st : m->states)
+      for (Arc& a : st) plabel.push_back(m->alph[0]->names[a.in] + ":" + m->alph[1]->names[a.out]);
+  return plabel;
+}
+
+// one decode line without its newline: ln weight, number of arcs, arc-table ids, "|", then per arc the (input:output)
+// labels of the cascade members' arcs it stands for
+void write_derivation(std::ostream& o, double lnw, const uint32_t* arcs, uint32_t len, std::vector<std::string> const& plabel,
+                      bool using_cascade, ModelArrays const& M) {
+  o << lnw << " " << len;
+  for (uint32_t k = 0; k < len; ++k) o << " " << arcs[k];
+  o << " |";
+  for (uint32_t k = 0; k < len; ++k) {
+    const uint32_t a = arcs[k];
+    const uint32_t k0 = using_cascade ? M.chain_off[a] : a, k1 = using_cascade ? M.chain_off[a + 1] : a + 1;
+    o << " (";
+    for (uint32_t c = k0; c < k1; ++c) o << (c > k0 ? " " : "") << plabel[using_cascade ? M.chain_param[c] : c];
+    o << ")";
+  }
+}
+
+}  // namespace
+
 // Decode: the -k n best derivations per training pair (cml_viterbi for n = 1, cml_kbest otherwise), n lines per example
 // in corpus order, best first; ranks past the number of derivations read "-inf 0 |".  The weights are the model's as
 // read, after the same normalisation a training run starts from (train.cc:509); no training happens.
@@ -335,27 +365,14 @@ void TrainJob::run_viterbi(std::ostream& log, std::string const& path) {
   std::vector<double> lnw(n_ex * K);
   if (n_ex && K == 1) ok(cml_viterbi(ctx, len.data(), base.data(), arcs.data(), arcs.size(), lnw.data()));
   if (n_ex && K > 1) ok(cml_kbest(ctx, (uint32_t)K, len.data(), base.data(), arcs.data(), arcs.size(), lnw.data()));
-  // labels of every parameter's member arc (parameters are numbered member by member, state by state, arc by arc)
-  std::vector<std::string> plabel;
-  for (Wfst* m : members)
-    for (auto& st : m->states)
-      for (Arc& a : st) plabel.push_back(m->alph[0]->names[a.in] + ":" + m->alph[1]->names[a.out]);
+  const std::vector<std::string> plabel = param_labels(members);
   std::ofstream o(path);
   if (!o) throw std::runtime_error("cannot write " + path);
   o.precision(17);
   double total = 0;
   uint64_t found = 0;
   for (uint64_t i = 0; i < n_ex * K; ++i) {
-    o << lnw[i] << " " << len[i];
-    for (uint32_t k = 0; k < len[i]; ++k) o << " " << arcs[base[i] + k];
-    o << " |";
-    for (uint32_t k = 0; k < len[i]; ++k) {
-      const uint32_t a = arcs[base[i] + k];
-      const uint32_t k0 = using_cascade ? M.chain_off[a] : a, k1 = using_cascade ? M.chain_off[a + 1] : a + 1;
-      o << " (";
-      for (uint32_t c = k0; c < k1; ++c) o << (c > k0 ? " " : "") << plabel[using_cascade ? M.chain_param[c] : c];
-      o << ")";
-    }
+    write_derivation(o, lnw[i], arcs.data() + base[i], len[i], plabel, using_cascade, M);
     o << "\n";
     if (i % K == 0) total += lnw[i];
     if (lnw[i] > kNegInf) ++found;
@@ -363,6 +380,96 @@ void TrainJob::run_viterbi(std::ostream& log, std::string const& path) {
   if (!opt.quiet) {
     log << "Viterbi: best derivations of " << n_ex << " examples, product of their weights=" << format_base2(total) << "\n";
     if (K > 1) log << "Viterbi: " << K << "-best lists, " << found << " derivations found\n";
+  }
+}
+
+// Decode new strings: the lattice of every string on the given tape x the composed machine, the other tape free, built on
+// the GPU (cml_build_free_trellises), then the same decoders and line format as run_viterbi.  The model is set up as for
+// --viterbi (prepare_model: the weights as read, normalised as a training run starts from them).
+void TrainJob::run_decode(std::ostream& log, std::string const& path) {
+  opt.precision = 64;
+  opt.space = CML_SPACE_LOG;
+  opt.no_ell = true;
+  opt.dense = -1;
+  if (opt.shard_count > 1) throw std::runtime_error("--decode decodes on one GPU");
+  prepare_model();
+  const int g = opt.given_tape;
+  std::vector<uint32_t> soff, ain, aout, adest;
+  x->arc_offsets(soff);
+  for (auto const& st : x->states)
+    for (Arc const& a : st) {
+      ain.push_back(a.in);
+      aout.push_back(a.out);
+      adest.push_back(a.dest);
+    }
+  const size_t n = corpus.examples.size();
+  std::vector<uint64_t> off(n + 1, 0);
+  std::vector<uint32_t> sym;
+  for (size_t e = 0; e < n; ++e) {
+    auto const& v = g ? corpus.examples[e].out : corpus.examples[e].in;
+    sym.insert(sym.end(), v.begin(), v.end());
+    off[e + 1] = sym.size();
+  }
+  cml_wfst_view xv{};
+  xv.n_states = x->num_states();
+  xv.final_state = x->final_state;
+  xv.n_arcs = ain.size();
+  xv.state_arc_off = soff.data();
+  xv.arc_in = ain.data();
+  xv.arc_out = aout.data();
+  xv.arc_dest = adest.data();
+  cml_string_batch sb{n, off.data(), sym.data()};
+  cml_built_trellises* b = nullptr;
+  ok(cml_build_free_trellises(ctx, &xv, &sb, g, &b));
+  std::unique_ptr<cml_built_trellises, void (*)(cml_built_trellises*)> hold(b, cml_free_built_trellises);
+  auto t0 = std::chrono::steady_clock::now();
+  if (b->batch.n_ex) ok(cml_add_trellises(ctx, &b->batch));
+  const double add_s = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
+  const uint64_t K = opt.kbest;
+  uint64_t n_ex = 0, n_states = 0, n_arcs = 0, n_levels = 0;
+  ok(cml_trellis_totals(ctx, &n_ex, &n_states, &n_arcs, &n_levels));
+  std::vector<uint32_t> len(n_ex * K), arcs(std::max<uint64_t>(1, n_levels * K));
+  std::vector<uint64_t> base(n_ex * K + 1);
+  std::vector<double> lnw(n_ex * K);
+  t0 = std::chrono::steady_clock::now();
+  if (n_ex && K == 1) ok(cml_viterbi(ctx, len.data(), base.data(), arcs.data(), arcs.size(), lnw.data()));
+  if (n_ex && K > 1) ok(cml_kbest(ctx, (uint32_t)K, len.data(), base.data(), arcs.data(), arcs.size(), lnw.data()));
+  const double dec_s = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
+  float dec_ms = 0;
+  ok(cml_kbest_stats(ctx, nullptr, nullptr, &dec_ms));
+  std::vector<int64_t> lat_of(n, -1);
+  for (uint64_t i = 0; i < b->batch.n_ex; ++i) lat_of[b->kept_example[i]] = (int64_t)i;
+  const std::vector<std::string> plabel = param_labels(members);
+  const std::vector<uint32_t>& free_label = g ? ain : aout;
+  const std::vector<std::string>& free_name = x->alph[1 - g]->names;
+  std::ofstream o(path);
+  if (!o) throw std::runtime_error("cannot write " + path);
+  o.precision(17);
+  double total = 0;
+  uint64_t found = 0;
+  for (size_t e = 0; e < n; ++e)
+    for (uint64_t r = 0; r < K; ++r) {
+      if (lat_of[e] < 0) {
+        o << "-inf 0 | ||\n";
+        continue;
+      }
+      const uint64_t i = (uint64_t)lat_of[e] * K + r;
+      const uint32_t* p = arcs.data() + base[i];
+      write_derivation(o, lnw[i], p, len[i], plabel, using_cascade, M);
+      o << " ||";
+      for (uint32_t k = 0; k < len[i]; ++k)
+        if (free_label[p[k]] != kEps) o << " " << free_name[free_label[p[k]]];
+      o << "\n";
+      if (r == 0) total += lnw[i];
+      if (lnw[i] > kNegInf) ++found;
+    }
+  if (!opt.quiet && !flags[(unsigned)'q']) {
+    log << "Decode: " << n << " strings on the " << (g ? "output" : "input") << " tape, " << b->n_dropped
+        << " without a derivation; product of the best weights of the others=" << format_base2(total) << "\n";
+    if (K > 1) log << "Decode: " << K << "-best lists, " << found << " derivations found\n";
+    log << "Decode: lattices built on the GPU in " << b->seconds << " s (k_build_free " << b->kernel_ms << " ms, "
+        << b->chunks << " chunk(s); " << n_states << " states, " << n_arcs << " arcs), cml_add_trellises " << add_s
+        << " s, decode " << dec_s << " s (kernels " << dec_ms << " ms)\n";
   }
 }
 

@@ -90,6 +90,32 @@ int open_job(int argc, const char* const* argv, TrainJob& job, std::ostream& err
       err << "carmel-b200: -" << c << " is not implemented on the training path\n";
       return -11;
     }
+  // --decode=FILE --given=input|output: decode the strings of the first file with the other tape free (in place of -t)
+  const bool decode = lopt.count("decode") > 0;
+  if (decode) {
+    const std::string g = lopt.count("given") ? lopt["given"] : "";
+    if (g != "input" && g != "output") {
+      err << "carmel-b200: --decode needs --given=input or --given=output (the tape the strings are on)\n";
+      return -9;
+    }
+    if (lopt.count("viterbi") || lopt.count("crp")) {
+      err << "carmel-b200: --decode cannot be combined with --viterbi or --crp\n";
+      return -9;
+    }
+    // --decode decodes instead of training: switches that train, or write what only training writes, are refused
+    // rather than ignored
+    for (const char c : {'t', 'F', 'M', '!'})
+      if (flags[(unsigned char)c]) {
+        err << "carmel-b200: --decode cannot be combined with -" << c << " (it decodes instead of training)\n";
+        return -9;
+      }
+    for (const char* k : {"trellis-only", "dump-trellis", "history", "fem-forest", "fem-norm", "fem-param", "dump-samples"})
+      if (lopt.count(k)) {
+        err << "carmel-b200: --decode cannot be combined with --" << k << "\n";
+        return -9;
+      }
+    topt.given_tape = g == "input" ? 0 : 1;
+  }
   // --crp forces -t and --train-cascade (carmel.cc:255-304 parse_gibbs_opts)
   const bool crp = lopt.count("crp") > 0;
   const bool trainc = lopt.count("train-cascade") > 0 || crp;
@@ -123,7 +149,7 @@ int open_job(int argc, const char* const* argv, TrainJob& job, std::ostream& err
     g.expectation = lopt.count("expectation") > 0;
     if (lopt.count("dump-samples")) g.dump_samples_file = lopt["dump-samples"];
   }
-  if (!flags[(unsigned)'t']) {
+  if (!flags[(unsigned)'t'] && !decode) {
     err << "carmel-b200 implements carmel's training path only: use -t (or --train-cascade)\n";
     return -11;
   }
@@ -164,7 +190,7 @@ int open_job(int argc, const char* const* argv, TrainJob& job, std::ostream& err
 
   job.corpus_file = files[0];
   job.fst_files.assign(files.begin() + 1, files.end());
-  if (lopt.count("viterbi") && flags[(unsigned)'k']) {  // -k n with --viterbi: n derivations per example
+  if ((lopt.count("viterbi") || decode) && flags[(unsigned)'k']) {  // -k n with --viterbi / --decode: n derivations each
     char* end = nullptr;
     const unsigned long long n = std::strtoull(topt.kbest_arg.c_str(), &end, 10);
     if (topt.kbest_arg.empty() || *end || topt.kbest_arg[0] == '-' || n < 1 || n > 0xFFFFFFFFull) {
@@ -247,7 +273,10 @@ int open_job(int argc, const char* const* argv, TrainJob& job, std::ostream& err
     err << "File " << job.corpus_file << " could not be opened for input.\n";
     return -9;
   }
-  job.corpus.read(cf, *result);
+  if (decode)
+    job.corpus.read_strings(cf, *result, topt.given_tape);
+  else
+    job.corpus.read(cf, *result);
   return 0;
 }
 

@@ -7,6 +7,7 @@
 //   carmel-b200 -t [-HJ] [-M n] [-e w] [-X w] [-f w] [-U] [-o g] [-j|-u] [-d] [-K] [-F out]
 //               [--train-cascade] [--normby=JCN] [--priors=w,w] [--float] [--scaled] [--gpu=n]
 //               [--dump-trellis=file] [--history=file] [--trellis-only] corpus wfst [wfst ...]
+//   carmel-b200 --decode=out --given=input|output [-k n] [--train-cascade] strings wfst [wfst ...]
 #include <cstring>
 #include <fstream>
 #include <iostream>
@@ -39,7 +40,10 @@ static void usage() {
                "           per example, normalisation groups, parameters after training (-M -1: the normalised input weights)\n"
                "  --load-fem-param=f  read cascade weights written by --fem-param\n"
                "  --viterbi=file [-k n]  decode only: the n best derivations (default 1) of every training pair, n lines per\n"
-               "           example, best first (\"-inf 0 |\" past the last derivation)\n";
+               "           example, best first (\"-inf 0 |\" past the last derivation)\n"
+               "  --decode=file --given=input|output [-k n]  in place of -t: the corpus file holds one string per line on the\n"
+               "           given tape; the n best derivations (default 1) with the other tape free, n lines per string, best\n"
+               "           first: the --viterbi line, \" ||\" and the decoded free-tape string (\"-inf 0 | ||\" when there is none)\n";
 }
 
 // carmel-b200 --gpus=N ...: N jobs in one process, job r keeps block r of the corpus on GPU r (--shard=r/N --gpu=r); the
@@ -47,10 +51,11 @@ static void usage() {
 // ranks take the same decisions (the reduced table and likelihood are identical everywhere); rank 0 logs and writes.
 static int run_multi_gpu(int argc, char** argv, int n_gpus) {
   for (int i = 1; i < argc; ++i)
-    if (std::strncmp(argv[i], "--viterbi", 9) == 0) {
-      std::cerr << "ERROR: --viterbi decodes on one GPU (no --gpus)\n";
-      return -11;
-    }
+    for (const char* d : {"--viterbi", "--decode"})
+      if (std::strncmp(argv[i], d, std::strlen(d)) == 0) {
+        std::cerr << "ERROR: " << d << " decodes on one GPU (no --gpus)\n";
+        return -11;
+      }
   unsigned char id[CML_COMM_ID_BYTES];
   if (cml_comm_unique_id(id) != CML_OK) {
     std::cerr << "ERROR: --gpus needs NCCL (libnccl.so.2 could not be loaded)\n";
@@ -124,6 +129,10 @@ int main(int argc, char** argv) {
     if (job.lopt.count("load-fem-param")) {  // carmel.cc:792-800
       std::cerr << "Reading cascade weights from --load-fem-param=" << job.lopt["load-fem-param"] << std::endl;
       job.load_fem_param(job.lopt["load-fem-param"]);
+    }
+    if (job.lopt.count("decode")) {  // decode new strings, the other tape free
+      job.run_decode(std::cerr, job.lopt["decode"]);
+      return 0;
     }
     if (job.lopt.count("trellis-only")) {  // host-side lattice construction only (no GPU work): parity tests
       TrellisBatch tb;

@@ -234,10 +234,8 @@ bool TrainJob::try_dense(int tape, Corpus const& local, std::vector<uint32_t>& k
   return true;
 }
 
-// Everything up to the first E-step: model tables, initial normalisation, prior counts, derivation
-// lattices (this rank's shard) flattened and resident on the GPU.
-void TrainJob::prepare() {
-  if (prepared) return;
+// The model on the GPU: context, model tables, parameters after the initial normalisation, prior counts.
+void TrainJob::prepare_model() {
   build_model();
   if (cml_create(&ctx, opt.device, opt.precision, opt.space) != CML_OK)
     throw std::runtime_error(std::string("carmel_b200: ") + cml_last_error(nullptr));
@@ -296,6 +294,13 @@ void TrainJob::prepare() {
     ok(cml_set_model(ctx, &mm));  // (no lattices are resident yet)
     ok(cml_set_params(ctx, w.data()));
   }
+}
+
+// Everything up to the first E-step: the model (prepare_model), derivation lattices (this rank's shard) flattened and
+// resident on the GPU.
+void TrainJob::prepare() {
+  if (prepared) return;
+  prepare_model();
 
   // ---- derivation lattices: built once, resident on the GPU (carmel's -: cache semantics) ----
   // With --shard=r/N only a contiguous block of the corpus (balanced by string length) is built and

@@ -451,4 +451,14 @@ void Corpus::read(std::istream& in, Wfst& x) {
   count();
 }
 
+void Corpus::read_strings(std::istream& in, Wfst& x, int tape) {
+  std::string line;
+  while (std::getline(in, line)) {
+    Example e;
+    symbols_of_line(line, *x.alph[tape], tape ? e.out : e.in);
+    examples.push_back(std::move(e));
+  }
+  count();
+}
+
 }  // namespace cb

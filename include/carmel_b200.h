@@ -75,7 +75,8 @@ enum cml_option {
   CML_OPT_ALLOW_EMPTY = 7, /* a rank of a sharded job whose block holds no usable example still takes part in every
                              collective: its E-step contributes zeros instead of failing with CML_ERR_NODERIV */
   CML_OPT_NO_GRAPH = 8,   /* cml_em_step enqueues its launches one by one instead of replaying a CUDA graph */
-  CML_OPT_KBEST_SCRATCH_MB = 9 /* device scratch budget (MiB) of one cml_kbest chunk; default 4096 */
+  CML_OPT_KBEST_SCRATCH_MB = 9, /* device scratch budget (MiB) of one cml_kbest chunk; default 4096 */
+  CML_OPT_FREE_BUILD_SCRATCH_MB = 10 /* device scratch budget (MiB) of one cml_build_free_trellises chunk; default 4096 */
 };
 int cml_set_option(cml_ctx* ctx, int option, int value);
 
@@ -189,10 +190,47 @@ typedef struct cml_built_trellises {
   uint32_t launches;             /* kernel launches (capacity rounds of the sizing pass + the fill pass) */
   uint32_t peak_states, peak_kept_arcs, peak_depth; /* largest walk: states / kept arcs before pruning, DFS depth */
   double seconds;                /* wall time of the call (index, upload, both passes, download) */
+  uint64_t chunks;               /* cml_build_free_trellises: chunks of strings processed (0 for cml_build_trellises) */
+  double kernel_ms;              /* cml_build_free_trellises: time of its k_build_free launches, CUDA events (0 otherwise) */
   void* owner;
 } cml_built_trellises;
 int cml_build_trellises(cml_ctx* ctx, const cml_wfst_view* x, const cml_corpus_view* c, cml_built_trellises** out);
 void cml_free_built_trellises(cml_built_trellises* b);
+/* ---- lattices of one given string, the other tape free (carmel -sri / -sli ... -k n: decode new strings) ---------- *
+ * The lattice of  string s on tape g  x  transducer x, with the other tape free:
+ *   x        the composed machine's arc table as a cml_wfst_view (arc-table order, symbol 0 = *e*, start = state 0)
+ *   g        the given tape: 0 = input, 1 = output
+ *   s        symbol ids on tape g
+ * States     pairs (q, t) of a machine state q and a position t in [0, |s|], kept when reachable from (0, 0) and
+ *            co-reachable to (final_state, |s|).
+ * Arcs       machine arc a of q leads from (q, t) to (dest, t) when its tape-g label is *e*, and to (dest, t + 1) when
+ *            that label equals s[t] (a symbol 0 in s matches no arc).  Its label on the free tape is not looked at.
+ * eps-level  of a machine state: its longest-path depth in the subgraph of the arcs with *e* on tape g.  When that
+ *            subgraph has a cycle the call fails with CML_ERR_CYCLE before any device work (such a model has strings
+ *            with unboundedly many derivations, and the decoders need acyclic lattices).
+ * Numbering  kept states are numbered in the order (t, eps-level(q), q): (0, 0) is state 0 and (final, |s|) the last
+ *            state (ex_fin = ex_states - 1); each state's out-arcs are its kept arcs in arc-table order; arc_id is the
+ *            machine arc id, as cml_add_trellises and the weights expect.
+ * Strings without a derivation (the empty lattice, symbols the tape never uses, ids out of range) are left out and
+ * listed in `dropped`; kept_example gives the string index of each kept lattice.  ex_weight is 1.
+ * The result is host memory in the form cml_add_trellises takes (release it with cml_free_built_trellises).  Of the
+ * statistics, `launches`, `peak_states` / `peak_kept_arcs` (the largest kept lattice), `seconds`, `chunks` and
+ * `kernel_ms` are filled in; `pre_arcs` and `peak_depth` are 0.
+ * GPU work: kernel k_build_free, one warp per string: reachability forward and co-reachability backward over the
+ * positions, the eps-levels of one position in order and the states of one eps-level across the lanes; then a counting
+ * pass, an exclusive scan on the host and a fill pass.  Device scratch is 6 B per (position, machine state) cell;
+ * strings are processed in chunks of consecutive strings whose scratch fits CML_OPT_FREE_BUILD_SCRATCH_MB (a string
+ * larger than that gets a chunk of its own).  Results do not depend on the chunking.
+ * Errors: CML_ERR_ARG for a null pointer, a tape other than 0 / 1, an incomplete or inconsistent transducer view,
+ * string offsets that do not start at 0 or decrease, or a string s with (|s| + 1) * n_states or (|s| + 1) * n_arcs of
+ * 2^32 or more (the bounds of its lattice's states and arcs, which are counted in 32 bits); CML_ERR_CYCLE as above. */
+typedef struct cml_string_batch {
+  uint64_t n;           /* strings */
+  const uint64_t* off;  /* [n + 1] string i is sym[off[i] .. off[i + 1]) */
+  const uint32_t* sym;
+} cml_string_batch;
+int cml_build_free_trellises(cml_ctx* ctx, const cml_wfst_view* x, const cml_string_batch* s, int given_tape,
+                             cml_built_trellises** out);
 int cml_trellis_totals(cml_ctx* ctx, uint64_t* n_ex, uint64_t* n_states, uint64_t* n_arcs, uint64_t* n_levels);
 int cml_cyclic_stats(cml_ctx* ctx, uint64_t* n_examples, uint64_t* n_back_edges);
 /* Best derivation of every resident lattice at the current parameters -- the decode carmel does with `-k 1` on the
