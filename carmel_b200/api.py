@@ -133,6 +133,9 @@ def load_library(path: str | None = None) -> C.CDLL:
     lib.cml_viterbi.argtypes = [vp, _u32p, C.POINTER(C.c_uint64), _u32p, C.c_uint64, _f64p]
     lib.cml_kbest.argtypes = [vp, C.c_uint32, _u32p, C.POINTER(C.c_uint64), _u32p, C.c_uint64, _f64p]
     lib.cml_kbest_stats.argtypes = [vp, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.POINTER(C.c_float)]
+    lib.cml_sample.argtypes = [vp, C.c_uint32, C.c_uint64, C.POINTER(C.c_uint64), _u32p, C.POINTER(C.c_uint64), _u32p,
+                               C.c_uint64, _f64p, _f64p]
+    lib.cml_sample_stats.argtypes = [vp, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.POINTER(C.c_float)]
     lib.cml_build_free_trellises.argtypes = [vp, C.POINTER(CmlWfstView), C.POINTER(CmlStringBatch), C.c_int,
                                              C.POINTER(C.POINTER(CmlBuiltTrellises))]
     lib.cml_free_built_trellises.argtypes = [C.POINTER(CmlBuiltTrellises)]
@@ -372,6 +375,38 @@ class Context:
         """the last decode call: scratch bytes of its largest chunk, chunks, kernel time (CUDA events, ms)"""
         b, c, ms = C.c_uint64(), C.c_uint64(), C.c_float()
         self._check(self.lib.cml_kbest_stats(self.h, C.byref(b), C.byref(c), C.byref(ms)))
+        return {"scratch_bytes": b.value, "chunks": c.value, "kernel_ms": ms.value}
+
+    def sample(self, n: int, seed: int, keys=None, cap: int | None = None):
+        """the total weight of every resident lattice and n derivations of each drawn in proportion to their weight
+        (cml_sample): (ln_total [n_ex], ln_weight [n_ex, n], path_len [n_ex, n], path_base [n_ex * n + 1], path_arcs);
+        sample (e, r) is path_arcs[path_base[e*n+r]:][:path_len[e, r]].  keys: the key of each lattice's uniforms
+        (default: its index); cap (default: n * total lattice levels) is the size of the arc buffer handed to the
+        library.  n = 0 computes ln_total only."""
+        t = self.trellis_totals()
+        n_ex, n = t["examples"], int(n)
+        m = n_ex * n
+        ln_total = np.zeros(max(n_ex, 1))
+        ln_w, lens = np.zeros(max(m, 1)), np.zeros(max(m, 1), np.uint32)
+        base = np.zeros(m + 1, np.uint64)
+        if cap is None:
+            cap = n * t["levels"]
+        arcs = np.zeros(max(cap, 1), np.uint32)
+        kp = None
+        if keys is not None:
+            keys = np.ascontiguousarray(keys, np.uint64)
+            assert keys.size == n_ex, (keys.size, n_ex)
+            kp = keys.ctypes.data_as(C.POINTER(C.c_uint64))
+        bp = base.ctypes.data_as(C.POINTER(C.c_uint64)) if n else None
+        self._check(self.lib.cml_sample(self.h, n, C.c_uint64(int(seed)), kp, _ptr(lens, _u32p) if n else None, bp,
+                                        _ptr(arcs, _u32p) if n else None, cap, _ptr(ln_w, _f64p) if n else None,
+                                        _ptr(ln_total, _f64p)))
+        return ln_total[:n_ex], ln_w[:m].reshape(n_ex, n), lens[:m].reshape(n_ex, n), base, arcs
+
+    def sample_stats(self) -> dict:
+        """the last sample() call: scratch bytes of its largest chunk, chunks, kernel time (CUDA events, ms)"""
+        b, c, ms = C.c_uint64(), C.c_uint64(), C.c_float()
+        self._check(self.lib.cml_sample_stats(self.h, C.byref(b), C.byref(c), C.byref(ms)))
         return {"scratch_bytes": b.value, "chunks": c.value, "kernel_ms": ms.value}
 
     def build_free_trellises(self, wfst: dict, strings, given: int) -> dict:

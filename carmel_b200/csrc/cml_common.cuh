@@ -33,6 +33,14 @@ struct __align__(16) CmlExDesc {
   double ln_weight;     // ln(weight)
 };
 
+// splitmix64 finaliser: the mixing step of every counter-based uniform (Gibbs samplers, cml_sample)
+__host__ __device__ __forceinline__ uint64_t mix64(uint64_t x) {
+  x += 0x9E3779B97F4A7C15ull;
+  x = (x ^ (x >> 30)) * 0xBF58476D1CE4E5B9ull;
+  x = (x ^ (x >> 27)) * 0x94D049BB133111EBull;
+  return x ^ (x >> 31);
+}
+
 template <typename T>
 struct DevArray {
   T* p = nullptr;

@@ -139,11 +139,14 @@ struct cml_ctx {
   int opt_no_counts = 0;     // CML_OPT_NO_COUNTS: profiling only, the sweeps skip their count REDs (lane kernel)
   int opt_no_factor = 0;     // CML_OPT_NO_FACTOR: keep per-arc weight records (no arc classes; round-1 kernels)
   int opt_no_wide = 0;       // CML_OPT_NO_WIDE: wide lattices stay on the k_fb_ell classes
-  int opt_kbest_scratch_mb = 4096;  // CML_OPT_KBEST_SCRATCH_MB: list scratch of one cml_kbest chunk
+  int opt_kbest_scratch_mb = 4096;  // CML_OPT_KBEST_SCRATCH_MB: scratch of one cml_kbest / cml_sample chunk
   int opt_free_build_scratch_mb = 4096;  // CML_OPT_FREE_BUILD_SCRATCH_MB: cell scratch of one cml_build_free_trellises chunk
   // last cml_kbest / cml_viterbi call (cml_kbest_stats)
   uint64_t kbest_scratch = 0, kbest_chunks = 0;
   float kbest_ms = 0;
+  // last cml_sample call (cml_sample_stats)
+  uint64_t sample_scratch = 0, sample_chunks = 0;
+  float sample_ms = 0;
 
   // model
   bool have_model = false, trivial = true;
@@ -231,6 +234,18 @@ struct cml_ctx {
 };
 
 int cml_dense_estimate_launch(cml_ctx* ctx);  // cml_dense.cu
+
+// Per-lattice decoders over the layered CSR (cml_kbest.cu; cml_kbest, cml_sample): the chunks of desc slots one call
+// walks, and the arc-table ids of the internal arc ids.
+struct DecodeChunks {
+  std::vector<uint64_t> st_base, cur_base;  // [desc slot] first state / in-arc of the lattice in its chunk's scratch
+  std::vector<uint32_t> list;               // chunk c = list[begin[c] .. begin[c + 1]); in-degree > 8 from mid[c] on
+  std::vector<uint64_t> begin, mid;
+  uint64_t max_states = 0, max_arcs = 0;    // of the largest chunk
+  DevArray<uint32_t> orig;                  // internal arc id -> arc-table id
+};
+int cml_decode_setup(cml_ctx* ctx, Batch& bt, uint64_t state_bytes, uint64_t arc_bytes, DecodeChunks& C);
+std::vector<uint64_t> cml_path_slots(Batch const& bt, uint32_t n, uint64_t* path_base);
 
 #define CML_REQUIRE(cond, code, msg) \
   do {                               \

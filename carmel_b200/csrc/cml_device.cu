@@ -2160,7 +2160,7 @@ extern "C" const char* const* cml_exported_symbols(size_t* n) {
       "cml_normalize_params", "cml_exported_symbols", "cml_job_open", "cml_job_close", "cml_job_error",
       "cml_job_set_comm", "cml_job_set_allreduce", "cml_job_prepare", "cml_job_context", "cml_job_train", "cml_job_write", "cml_job_stats", "cml_gibbs_init", "cml_gibbs_attach_dense", "cml_gibbs_sweep",
       "cml_gibbs_sample_capacity", "cml_gibbs_get_samples", "cml_gibbs_get_state", "cml_gibbs_get_block_logprob", "cml_forests_create", "cml_forests_destroy",
-      "cml_forests_last_error", "cml_forests_set_stream", "cml_forests_set_layout", "cml_forests_layout_stats", "cml_forests_level_stats", "cml_build_trellises", "cml_build_free_trellises", "cml_free_built_trellises", "cml_cyclic_stats", "cml_viterbi", "cml_kbest", "cml_kbest_stats",
+      "cml_forests_last_error", "cml_forests_set_stream", "cml_forests_set_layout", "cml_forests_layout_stats", "cml_forests_level_stats", "cml_build_trellises", "cml_build_free_trellises", "cml_free_built_trellises", "cml_cyclic_stats", "cml_viterbi", "cml_kbest", "cml_kbest_stats", "cml_sample", "cml_sample_stats",
       "cml_forests_launch_count", "cml_forests_set_rules",
       "cml_forests_set_params", "cml_forests_get_params", "cml_forests_add", "cml_forests_totals", "cml_forests_estimate",
       "cml_forests_estimate_launch", "cml_forests_estimate_finish", "cml_forests_last_time_ms", "cml_forests_get_inside",

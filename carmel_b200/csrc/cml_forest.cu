@@ -2242,15 +2242,9 @@ extern "C" int cml_forests_viterbi(cml_forests* f, const cml_forest_batch* b, do
 // reference's fp64 logweight (pairwise log-add in child order).
 // ---------------------------------------------------------------------------------------------------
 const int kGibbsDepth = 96, kGibbsStack = 384;
-__device__ __forceinline__ uint64_t fg_mix64(uint64_t x) {
-  x += 0x9E3779B97F4A7C15ull;
-  x = (x ^ (x >> 30)) * 0xBF58476D1CE4E5B9ull;
-  x = (x ^ (x >> 27)) * 0x94D049BB133111EBull;
-  return x ^ (x >> 31);
-}
 __device__ __forceinline__ double fg_uniform(uint64_t seed, uint32_t sweep, uint32_t block, uint32_t draw) {
-  uint64_t h = fg_mix64(seed ^ fg_mix64(((uint64_t)sweep << 32) | block));
-  h = fg_mix64(h + draw);
+  uint64_t h = mix64(seed ^ mix64(((uint64_t)sweep << 32) | block));
+  h = mix64(h + draw);
   return (double)(h >> 11) * (1.0 / 9007199254740992.0);
 }
 struct FGibbsArgs {

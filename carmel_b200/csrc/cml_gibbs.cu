@@ -25,12 +25,6 @@
 
 namespace {
 
-__device__ __forceinline__ uint64_t mix64(uint64_t x) {
-  x += 0x9E3779B97F4A7C15ull;
-  x = (x ^ (x >> 30)) * 0xBF58476D1CE4E5B9ull;
-  x = (x ^ (x >> 27)) * 0x94D049BB133111EBull;
-  return x ^ (x >> 31);
-}
 __device__ __forceinline__ double gibbs_uniform(uint64_t seed, uint32_t sweep, uint32_t block, uint32_t draw) {
   uint64_t h = mix64(seed ^ mix64(((uint64_t)sweep << 32) | block));
   h = mix64(h + draw);

@@ -172,6 +172,83 @@ __global__ void k_kbest_shape(const CmlExDesc* __restrict__ desc, uint32_t n, co
 
 }  // namespace
 
+// the path slots of n derivations per lattice: a derivation has at most (levels - 1) arcs; example e's derivation r
+// starts at n * lvl_pre[e] + r * levels(e).  Fills path_base[n_ex * n + 1] when non-null and returns lvl_pre[n_ex + 1].
+std::vector<uint64_t> cml_path_slots(Batch const& bt, uint32_t n, uint64_t* path_base) {
+  const uint64_t n_ex = bt.n_ex;
+  std::vector<uint64_t> lvl_pre(n_ex + 1, 0);
+  for (uint64_t e = 0; e < n_ex; ++e) lvl_pre[e + 1] = lvl_pre[e] + bt.h_nlevels[e];
+  if (path_base) {
+    for (uint64_t e = 0; e < n_ex; ++e)
+      for (uint32_t r = 0; r < n; ++r) path_base[e * n + r] = lvl_pre[e] * n + (uint64_t)r * bt.h_nlevels[e];
+    path_base[n_ex * n] = lvl_pre[n_ex] * n;
+  }
+  return lvl_pre;
+}
+
+// What every per-lattice decoder needs before its launches: the ln arc weights at the current parameters (arc_w_real),
+// the way back from internal arc ids to arc-table ids (C.orig), and chunks of consecutive desc slots whose scratch
+// (state_bytes per state, arc_bytes per in-arc) fits CML_OPT_KBEST_SCRATCH_MB; a lattice larger than the budget gets a
+// chunk of its own.  Within a chunk the slots whose largest in-degree is <= 8 come first (k_kbest's G = 8 part).
+int cml_decode_setup(cml_ctx* ctx, Batch& bt, uint64_t state_bytes, uint64_t arc_bytes, DecodeChunks& C) {
+  cudaStream_t s = ctx->stream;
+  const uint64_t n_ex = bt.n_ex;
+  if (ctx->arc_slot_code.n < (size_t)ctx->n_arcs + 1) {
+    CML_CUDA(ctx->arc_slot_code.alloc((size_t)ctx->n_arcs + 1));
+    CML_CUDA(cudaMemsetAsync(ctx->arc_slot_code.p, 0xFF, ((size_t)ctx->n_arcs + 1) * sizeof(uint32_t), s));
+  }
+  cmlk::k_arc_weights<double, false, cmlk::WS<double>><<<cdiv(ctx->n_arcs + 1, 256), 256, 0, s>>>(
+      ctx->n_arcs, ctx->trivial ? nullptr : ctx->chain_off.p, ctx->chain_param.p, ctx->ln_w.p, ctx->arc_slot_code.p,
+      ctx->arc_perm.p, ctx->arc_lnw.p, (double*)ctx->arc_w_real.p, (cmlk::WS<double>*)ctx->arc_ws.p);
+  ++ctx->launches;
+  std::vector<uint32_t> orig((size_t)ctx->n_arcs + 1, 0);
+  for (uint32_t a = 0; a < ctx->n_arcs; ++a) orig[ctx->h_perm[a]] = a;
+  CML_CUDA(C.orig.upload(orig.data(), orig.size(), s));
+  // lattice shapes (by desc slot) decide the lane-group width and the chunks
+  DevArray<uint2> d_shape;
+  CML_CUDA(d_shape.alloc(n_ex));
+  k_kbest_shape<<<cdiv(n_ex, 128), 128, 0, s>>>(bt.desc.p, (uint32_t)n_ex, bt.in_off.p, d_shape.p);
+  ++ctx->launches;
+  CML_CUDA(cudaGetLastError());
+  std::vector<uint2> shape(n_ex);
+  std::vector<CmlExDesc> desc(n_ex);
+  CML_CUDA(cudaMemcpyAsync(shape.data(), d_shape.p, n_ex * sizeof(uint2), cudaMemcpyDeviceToHost, s));
+  CML_CUDA(cudaMemcpyAsync(desc.data(), bt.desc.p, n_ex * sizeof(CmlExDesc), cudaMemcpyDeviceToHost, s));
+  CML_CUDA(cudaStreamSynchronize(s));
+  const uint64_t budget = (uint64_t)ctx->opt_kbest_scratch_mb << 20;
+  C.st_base.assign(n_ex, 0);
+  C.cur_base.assign(n_ex, 0);
+  C.list.clear();
+  C.begin.assign(1, 0);
+  C.mid.clear();
+  C.max_states = C.max_arcs = 0;
+  uint64_t ns = 0, na = 0;
+  std::vector<uint32_t> wide;
+  auto close_chunk = [&]() {
+    C.mid.push_back(C.list.size());
+    C.list.insert(C.list.end(), wide.begin(), wide.end());
+    wide.clear();
+    C.begin.push_back(C.list.size());
+    C.max_states = std::max(C.max_states, ns);
+    C.max_arcs = std::max(C.max_arcs, na);
+    ns = na = 0;
+  };
+  for (uint64_t t = 0; t < n_ex; ++t) {
+    const uint64_t st = desc[t].n_states, ar = shape[t].y;
+    if ((ns || na) && ((ns + st) * state_bytes + (na + ar) * arc_bytes > budget)) close_chunk();
+    C.st_base[t] = ns;
+    C.cur_base[t] = na;
+    ns += st;
+    na += ar;
+    if (shape[t].x <= 8)
+      C.list.push_back((uint32_t)t);
+    else
+      wide.push_back((uint32_t)t);
+  }
+  close_chunk();
+  return CML_OK;
+}
+
 extern "C" int cml_kbest(cml_ctx* ctx, uint32_t k, uint32_t* path_len, uint64_t* path_base, uint32_t* path_arcs,
                          uint64_t cap, double* ln_weight) {
   if (!ctx || !path_len || !path_base || !ln_weight) return CML_ERR_ARG;
@@ -186,78 +263,25 @@ extern "C" int cml_kbest(cml_ctx* ctx, uint32_t k, uint32_t* path_len, uint64_t*
   cudaSetDevice(ctx->device);
   cudaStream_t s = ctx->stream;
   const uint64_t n_ex = bt.n_ex;
-  // path slots: a derivation has at most (levels - 1) arcs; example e's rank r starts at k * lvl_pre[e] + r * levels(e)
-  std::vector<uint64_t> lvl_pre(n_ex + 1, 0);
-  for (uint64_t e = 0; e < n_ex; ++e) lvl_pre[e + 1] = lvl_pre[e] + bt.h_nlevels[e];
-  for (uint64_t e = 0; e < n_ex; ++e)
-    for (uint32_t r = 0; r < k; ++r) path_base[e * k + r] = lvl_pre[e] * k + (uint64_t)r * bt.h_nlevels[e];
-  path_base[n_ex * k] = lvl_pre[n_ex] * k;
+  const std::vector<uint64_t> lvl_pre = cml_path_slots(bt, k, path_base);
   CML_REQUIRE(!path_arcs || cap >= lvl_pre[n_ex] * k, CML_ERR_ARG,
               "path_arcs too small (need k times the total number of lattice levels)");
   ctx->kbest_ms = 0;
   ctx->kbest_chunks = 0;
   ctx->kbest_scratch = 0;
   if (!n_ex) return CML_OK;
-  if (ctx->arc_slot_code.n < (size_t)ctx->n_arcs + 1) {
-    CML_CUDA(ctx->arc_slot_code.alloc((size_t)ctx->n_arcs + 1));
-    CML_CUDA(cudaMemsetAsync(ctx->arc_slot_code.p, 0xFF, ((size_t)ctx->n_arcs + 1) * sizeof(uint32_t), s));
-  }
-  cmlk::k_arc_weights<double, false, cmlk::WS<double>><<<cdiv(ctx->n_arcs + 1, 256), 256, 0, s>>>(
-      ctx->n_arcs, ctx->trivial ? nullptr : ctx->chain_off.p, ctx->chain_param.p, ctx->ln_w.p, ctx->arc_slot_code.p,
-      ctx->arc_perm.p, ctx->arc_lnw.p, (double*)ctx->arc_w_real.p, (cmlk::WS<double>*)ctx->arc_ws.p);
-  ++ctx->launches;
-  std::vector<uint32_t> orig((size_t)ctx->n_arcs + 1, 0);
-  for (uint32_t a = 0; a < ctx->n_arcs; ++a) orig[ctx->h_perm[a]] = a;
-  // lattice shapes (by desc slot) decide the lane-group width and the chunks
-  DevArray<uint2> d_shape;
-  CML_CUDA(d_shape.alloc(n_ex));
-  k_kbest_shape<<<cdiv(n_ex, 128), 128, 0, s>>>(bt.desc.p, (uint32_t)n_ex, bt.in_off.p, d_shape.p);
-  ++ctx->launches;
-  CML_CUDA(cudaGetLastError());
-  std::vector<uint2> shape(n_ex);
-  std::vector<CmlExDesc> desc(n_ex);
-  CML_CUDA(cudaMemcpyAsync(shape.data(), d_shape.p, n_ex * sizeof(uint2), cudaMemcpyDeviceToHost, s));
-  CML_CUDA(cudaMemcpyAsync(desc.data(), bt.desc.p, n_ex * sizeof(CmlExDesc), cudaMemcpyDeviceToHost, s));
-  CML_CUDA(cudaStreamSynchronize(s));
-  // chunks of consecutive slots whose scratch (k list entries of 16 B and a length per state, a cursor per in-arc)
-  // fits the budget; a lattice larger than the budget gets a chunk of its own
-  const uint64_t budget = (uint64_t)ctx->opt_kbest_scratch_mb << 20;
-  std::vector<uint64_t> st_base(n_ex), cur_base(n_ex);
-  std::vector<uint32_t> list;                      // per chunk: the G = 8 slots, then the G = 32 slots
-  std::vector<uint64_t> chunk_begin(1, 0), chunk_mid;  // offsets into list
-  uint64_t max_states = 0, max_arcs = 0, ns = 0, na = 0;
-  std::vector<uint32_t> wide;
-  auto close_chunk = [&]() {
-    chunk_mid.push_back(list.size());
-    list.insert(list.end(), wide.begin(), wide.end());
-    wide.clear();
-    chunk_begin.push_back(list.size());
-    max_states = std::max(max_states, ns);
-    max_arcs = std::max(max_arcs, na);
-    ns = na = 0;
-  };
-  for (uint64_t t = 0; t < n_ex; ++t) {
-    const uint64_t st = desc[t].n_states, ar = shape[t].y;
-    if ((ns || na) && ((ns + st) * (16ull * k + 4) + (na + ar) * 4 > budget)) close_chunk();
-    st_base[t] = ns;
-    cur_base[t] = na;
-    ns += st;
-    na += ar;
-    if (shape[t].x <= 8)
-      list.push_back((uint32_t)t);
-    else
-      wide.push_back((uint32_t)t);
-  }
-  close_chunk();
-  const uint64_t n_chunks = chunk_mid.size();
-  DevArray<uint32_t> d_orig, d_list, d_len, d_plen, d_path, d_cur;
+  // chunk scratch: k list entries of 16 B and a length per state, a cursor per in-arc
+  DecodeChunks P;
+  const int rc = cml_decode_setup(ctx, bt, 16ull * k + 4, 4, P);
+  if (rc != CML_OK) return rc;
+  const uint64_t n_chunks = P.mid.size(), max_states = P.max_states, max_arcs = P.max_arcs;
+  DevArray<uint32_t> d_list, d_len, d_plen, d_path, d_cur;
   DevArray<uint64_t> d_stb, d_curb, d_pre;
   DevArray<double> d_sc, d_lnw;
   DevArray<uint2> d_bp;
-  CML_CUDA(d_orig.upload(orig.data(), orig.size(), s));
-  CML_CUDA(d_list.upload(list.data(), list.size(), s));
-  CML_CUDA(d_stb.upload(st_base.data(), n_ex, s));
-  CML_CUDA(d_curb.upload(cur_base.data(), n_ex, s));
+  CML_CUDA(d_list.upload(P.list.data(), P.list.size(), s));
+  CML_CUDA(d_stb.upload(P.st_base.data(), n_ex, s));
+  CML_CUDA(d_curb.upload(P.cur_base.data(), n_ex, s));
   CML_CUDA(d_pre.upload(lvl_pre.data(), lvl_pre.size(), s));
   CML_CUDA(d_sc.alloc(std::max<uint64_t>(1, max_states * k)));
   CML_CUDA(d_bp.alloc(std::max<uint64_t>(1, max_states * k)));
@@ -269,7 +293,7 @@ extern "C" int cml_kbest(cml_ctx* ctx, uint32_t k, uint32_t* path_len, uint64_t*
   ctx->kbest_chunks = n_chunks;
   ctx->kbest_scratch = max_states * (16ull * k + 4) + max_arcs * 4;
   KbestArgs A{bt.desc.p, nullptr, 0, k, bt.lvl_off.p, bt.in_off.p, bt.in_arc.p, (const double*)ctx->arc_w_real.p,
-              d_orig.p, d_stb.p, d_curb.p, d_pre.p, d_sc.p, d_bp.p, d_len.p, d_cur.p, d_plen.p,
+              P.orig.p, d_stb.p, d_curb.p, d_pre.p, d_sc.p, d_bp.p, d_len.p, d_cur.p, d_plen.p,
               path_arcs ? d_path.p : nullptr, d_lnw.p};
   struct Events {
     cudaEvent_t a = nullptr, b = nullptr;
@@ -284,7 +308,7 @@ extern "C" int cml_kbest(cml_ctx* ctx, uint32_t k, uint32_t* path_len, uint64_t*
   const unsigned max_blocks = (unsigned)ctx->sm_count * 16u;
   for (uint64_t c = 0; c < n_chunks; ++c) {
     for (int wide_part = 0; wide_part < 2; ++wide_part) {
-      const uint64_t b0 = wide_part ? chunk_mid[c] : chunk_begin[c], b1 = wide_part ? chunk_begin[c + 1] : chunk_mid[c];
+      const uint64_t b0 = wide_part ? P.mid[c] : P.begin[c], b1 = wide_part ? P.begin[c + 1] : P.mid[c];
       if (b1 == b0) continue;
       A.list = d_list.p + b0;
       A.n_list = (uint32_t)(b1 - b0);

@@ -164,6 +164,8 @@ struct TrainOpts {
   std::string kbest_arg;            // -k n : derivations per example written by --viterbi (unused when training)
   uint32_t kbest = 1;
   int given_tape = -1;              // --given=input|output : the tape --decode reads its strings on (0 / 1)
+  uint32_t sample = 0;              // --sample=n : with --viterbi / --decode, n derivations drawn per example (seed -R)
+  std::string sum_file;             // --sum=FILE : with --viterbi / --decode, ln of every example's total weight
   TrainOpts();
 };
 // WFST::random_restart_acceptor (fst.h:999-1044): a further start must be, after its first iteration, within a
@@ -238,6 +240,8 @@ struct TrainJob {
   std::vector<Wfst*> members;
   bool using_cascade = false, prepared = false;
   TrainResult res;
+  std::vector<uint32_t> kept_example;  // prepare(): corpus index of each resident lattice
+  uint64_t corpus_size = 0;            // prepare(): examples read, with or without a derivation
 
   ~TrainJob();
   void build_model();  // parameters, chains, normalisation groups (host only; fem.cpp)
@@ -253,7 +257,9 @@ struct TrainJob {
   void prepare_gibbs();
   // --viterbi=FILE: the best derivation of every training pair under the (normalised) model as given, one line per
   // kept example: ln weight, number of arcs, arc-table ids; then, per arc, the (input:output) labels of the cascade
-  // members' arcs it stands for (decode side: carmel -k 1 on the composed machine, fst.h:769-800)
+  // members' arcs it stands for (decode side: carmel -k 1 on the composed machine, fst.h:769-800).  With --sample=n the
+  // file holds n derivations drawn per example instead, in corpus order (examples without a derivation included); with
+  // --sum=FILE that file gets ln of every example's total weight.
   void run_viterbi(std::ostream& log, std::string const& path);
   // --decode=FILE --given=input|output: the -k n best derivations of every string of the corpus file on the given tape
   // with the other tape free (carmel -sri / -sli ... -k n), n lines per string in file order: the --viterbi line, then

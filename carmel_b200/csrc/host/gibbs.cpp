@@ -9,6 +9,7 @@
 // the downloaded sample paths.
 #include <algorithm>
 #include <chrono>
+#include <cstdio>
 #include <fstream>
 #include <iostream>
 #include <stdexcept>
@@ -345,6 +346,53 @@ void write_derivation(std::ostream& o, double lnw, const uint32_t* arcs, uint32_
   }
 }
 
+// --sample / --sum: ln of the total weight of every resident lattice and, for n > 0, n derivations drawn from each in
+// proportion to their weight (cml_sample), the uniforms of lattice i keyed by key[i]
+struct Drawn {
+  std::vector<uint32_t> len, arcs;
+  std::vector<uint64_t> base;
+  std::vector<double> lnw, total;
+  float kernel_ms = 0;
+};
+int draw_samples(cml_ctx* ctx, uint32_t n, uint64_t seed, std::vector<uint64_t> const& key, Drawn& d) {
+  uint64_t n_ex = 0, n_states = 0, n_arcs = 0, n_levels = 0;
+  int rc = cml_trellis_totals(ctx, &n_ex, &n_states, &n_arcs, &n_levels);
+  if (rc != CML_OK) return rc;
+  d.len.assign(n_ex * n, 0);
+  d.arcs.assign(std::max<uint64_t>(1, n_levels * n), 0);
+  d.base.assign(n_ex * n + 1, 0);
+  d.lnw.assign(n_ex * n, 0.);
+  d.total.assign(n_ex, 0.);
+  if (!n_ex) return CML_OK;
+  rc = cml_sample(ctx, n, seed, key.data(), d.len.data(), d.base.data(), d.arcs.data(), d.arcs.size(), d.lnw.data(),
+                  d.total.data());
+  if (rc != CML_OK) return rc;
+  return cml_sample_stats(ctx, nullptr, nullptr, &d.kernel_ms);
+}
+
+// --sum=FILE: one line per example (lat_of[e] < 0: no lattice), ln of its total weight as %.17g, or -inf; the log line
+// gives the product of the totals of the examples with a derivation
+void write_sums(std::ostream& log, bool quiet, std::string const& path, std::vector<int64_t> const& lat_of,
+                std::vector<double> const& total, const char* what) {
+  std::ofstream o(path);
+  if (!o) throw std::runtime_error("cannot write " + path);
+  double prod = 0;
+  uint64_t none = 0;
+  char buf[64];
+  for (int64_t i : lat_of) {
+    const double t = i < 0 ? kNegInf : total[i];
+    std::snprintf(buf, sizeof buf, "%.17g", t);
+    o << buf << "\n";
+    if (t > kNegInf)
+      prod += t;
+    else
+      ++none;
+  }
+  if (!quiet)
+    log << "Sum: total weights of " << lat_of.size() << " " << what << ", " << none
+        << " without a derivation; product of the others=" << format_base2(prod) << "\n";
+}
+
 }  // namespace
 
 // Decode: the -k n best derivations per training pair (cml_viterbi for n = 1, cml_kbest otherwise), n lines per example
@@ -357,6 +405,32 @@ void TrainJob::run_viterbi(std::ostream& log, std::string const& path) {
   opt.dense = -1;
   if (opt.shard_count > 1) throw std::runtime_error("--viterbi decodes on one GPU");
   prepare();
+  std::vector<int64_t> lat_of(corpus_size, -1);
+  std::vector<uint64_t> key(kept_example.begin(), kept_example.end());  // the example's index in the corpus
+  for (size_t i = 0; i < kept_example.size(); ++i) lat_of[kept_example[i]] = (int64_t)i;
+  const std::vector<std::string> plabel = param_labels(members);
+  Drawn d;
+  if (opt.sample || !opt.sum_file.empty()) ok(draw_samples(ctx, opt.sample, opt.seed, key, d));
+  if (!opt.sum_file.empty()) write_sums(log, opt.quiet, opt.sum_file, lat_of, d.total, "examples");
+  if (opt.sample) {  // n lines per example in corpus order, "-inf 0 |" for an example without a derivation
+    const uint32_t n = opt.sample;
+    std::ofstream o(path);
+    if (!o) throw std::runtime_error("cannot write " + path);
+    o.precision(17);
+    for (int64_t i : lat_of)
+      for (uint32_t r = 0; r < n; ++r) {
+        const uint64_t j = i < 0 ? 0 : (uint64_t)i * n + r;
+        if (i < 0)
+          write_derivation(o, kNegInf, nullptr, 0, plabel, using_cascade, M);
+        else
+          write_derivation(o, d.lnw[j], d.arcs.data() + d.base[j], d.len[j], plabel, using_cascade, M);
+        o << "\n";
+      }
+    if (!opt.quiet)
+      log << "Sample: " << n << " derivations drawn per example (seed " << opt.seed << ") from " << kept_example.size()
+          << " of " << corpus_size << " examples (kernels " << d.kernel_ms << " ms)\n";
+    return;
+  }
   const uint64_t K = opt.kbest;
   uint64_t n_ex = 0, n_states = 0, n_arcs = 0, n_levels = 0;
   ok(cml_trellis_totals(ctx, &n_ex, &n_states, &n_arcs, &n_levels));
@@ -365,7 +439,6 @@ void TrainJob::run_viterbi(std::ostream& log, std::string const& path) {
   std::vector<double> lnw(n_ex * K);
   if (n_ex && K == 1) ok(cml_viterbi(ctx, len.data(), base.data(), arcs.data(), arcs.size(), lnw.data()));
   if (n_ex && K > 1) ok(cml_kbest(ctx, (uint32_t)K, len.data(), base.data(), arcs.data(), arcs.size(), lnw.data()));
-  const std::vector<std::string> plabel = param_labels(members);
   std::ofstream o(path);
   if (!o) throw std::runtime_error("cannot write " + path);
   o.precision(17);
@@ -425,20 +498,33 @@ void TrainJob::run_decode(std::ostream& log, std::string const& path) {
   auto t0 = std::chrono::steady_clock::now();
   if (b->batch.n_ex) ok(cml_add_trellises(ctx, &b->batch));
   const double add_s = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
-  const uint64_t K = opt.kbest;
+  const uint64_t K = opt.sample ? opt.sample : opt.kbest;
   uint64_t n_ex = 0, n_states = 0, n_arcs = 0, n_levels = 0;
   ok(cml_trellis_totals(ctx, &n_ex, &n_states, &n_arcs, &n_levels));
+  std::vector<int64_t> lat_of(n, -1);
+  for (uint64_t i = 0; i < b->batch.n_ex; ++i) lat_of[b->kept_example[i]] = (int64_t)i;
+  // --sample / --sum: keyed by the string's line, so a string's draws do not depend on the other lines
+  const std::vector<uint64_t> key(b->kept_example, b->kept_example + b->batch.n_ex);
+  Drawn d;
+  if (!opt.sum_file.empty() && !opt.sample) ok(draw_samples(ctx, 0, opt.seed, key, d));
   std::vector<uint32_t> len(n_ex * K), arcs(std::max<uint64_t>(1, n_levels * K));
   std::vector<uint64_t> base(n_ex * K + 1);
   std::vector<double> lnw(n_ex * K);
   t0 = std::chrono::steady_clock::now();
-  if (n_ex && K == 1) ok(cml_viterbi(ctx, len.data(), base.data(), arcs.data(), arcs.size(), lnw.data()));
-  if (n_ex && K > 1) ok(cml_kbest(ctx, (uint32_t)K, len.data(), base.data(), arcs.data(), arcs.size(), lnw.data()));
+  if (opt.sample) {
+    ok(draw_samples(ctx, opt.sample, opt.seed, key, d));
+    len.swap(d.len);
+    arcs.swap(d.arcs);
+    base.swap(d.base);
+    lnw.swap(d.lnw);
+  }
+  if (n_ex && K == 1 && !opt.sample) ok(cml_viterbi(ctx, len.data(), base.data(), arcs.data(), arcs.size(), lnw.data()));
+  if (n_ex && K > 1 && !opt.sample)
+    ok(cml_kbest(ctx, (uint32_t)K, len.data(), base.data(), arcs.data(), arcs.size(), lnw.data()));
   const double dec_s = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
-  float dec_ms = 0;
-  ok(cml_kbest_stats(ctx, nullptr, nullptr, &dec_ms));
-  std::vector<int64_t> lat_of(n, -1);
-  for (uint64_t i = 0; i < b->batch.n_ex; ++i) lat_of[b->kept_example[i]] = (int64_t)i;
+  float dec_ms = d.kernel_ms;
+  if (!opt.sample) ok(cml_kbest_stats(ctx, nullptr, nullptr, &dec_ms));
+  if (!opt.sum_file.empty()) write_sums(log, opt.quiet || flags[(unsigned)'q'], opt.sum_file, lat_of, d.total, "strings");
   const std::vector<std::string> plabel = param_labels(members);
   const std::vector<uint32_t>& free_label = g ? ain : aout;
   const std::vector<std::string>& free_name = x->alph[1 - g]->names;
@@ -465,8 +551,13 @@ void TrainJob::run_decode(std::ostream& log, std::string const& path) {
     }
   if (!opt.quiet && !flags[(unsigned)'q']) {
     log << "Decode: " << n << " strings on the " << (g ? "output" : "input") << " tape, " << b->n_dropped
-        << " without a derivation; product of the best weights of the others=" << format_base2(total) << "\n";
-    if (K > 1) log << "Decode: " << K << "-best lists, " << found << " derivations found\n";
+        << " without a derivation";
+    if (opt.sample)
+      log << "; " << K << " derivations drawn per string (seed " << opt.seed << ")\n";
+    else
+      log << "; product of the best weights of the others=" << format_base2(total) << "\n";
+    if (K > 1 && !opt.sample)
+      log << "Decode: " << K << "-best lists, " << found << " derivations found\n";
     log << "Decode: lattices built on the GPU in " << b->seconds << " s (k_build_free " << b->kernel_ms << " ms, "
         << b->chunks << " chunk(s); " << n_states << " states, " << n_arcs << " arcs), cml_add_trellises " << add_s
         << " s, decode " << dec_s << " s (kernels " << dec_ms << " ms)\n";

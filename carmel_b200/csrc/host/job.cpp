@@ -190,6 +190,29 @@ int open_job(int argc, const char* const* argv, TrainJob& job, std::ostream& err
 
   job.corpus_file = files[0];
   job.fst_files.assign(files.begin() + 1, files.end());
+  // --sample=n / --sum=FILE with --viterbi / --decode: draw n derivations per example instead of the best ones / write
+  // ln of every example's total weight (without --viterbi / --decode they are unknown long options, accepted and unused)
+  if ((lopt.count("viterbi") || decode) && lopt.count("sample")) {
+    if (flags[(unsigned)'k']) {
+      err << "carmel-b200: --sample cannot be combined with -k (it draws derivations instead of listing the best)\n";
+      return -9;
+    }
+    const std::string v = lopt["sample"];
+    char* end = nullptr;
+    const unsigned long long n = std::strtoull(v.c_str(), &end, 10);
+    if (v.empty() || *end || v[0] == '-' || n < 1 || n > 0xFFFFFFFFull) {
+      err << "carmel-b200: --sample needs a whole number of derivations >= 1 (got \"" << v << "\")\n";
+      return -9;
+    }
+    topt.sample = (uint32_t)n;
+  }
+  if ((lopt.count("viterbi") || decode) && lopt.count("sum")) {
+    if (lopt["sum"].empty()) {
+      err << "carmel-b200: --sum needs a file name (--sum=FILE)\n";
+      return -9;
+    }
+    topt.sum_file = lopt["sum"];
+  }
   if ((lopt.count("viterbi") || decode) && flags[(unsigned)'k']) {  // -k n with --viterbi / --decode: n derivations each
     char* end = nullptr;
     const unsigned long long n = std::strtoull(topt.kbest_arg.c_str(), &end, 10);

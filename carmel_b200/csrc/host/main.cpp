@@ -7,7 +7,7 @@
 //   carmel-b200 -t [-HJ] [-M n] [-e w] [-X w] [-f w] [-U] [-o g] [-j|-u] [-d] [-K] [-F out]
 //               [--train-cascade] [--normby=JCN] [--priors=w,w] [--float] [--scaled] [--gpu=n]
 //               [--dump-trellis=file] [--history=file] [--trellis-only] corpus wfst [wfst ...]
-//   carmel-b200 --decode=out --given=input|output [-k n] [--train-cascade] strings wfst [wfst ...]
+//   carmel-b200 --decode=out --given=input|output [-k n | --sample=n [-R seed]] [--sum=file] [--train-cascade] strings wfst ...
 #include <cstring>
 #include <fstream>
 #include <iostream>
@@ -43,7 +43,10 @@ static void usage() {
                "           example, best first (\"-inf 0 |\" past the last derivation)\n"
                "  --decode=file --given=input|output [-k n]  in place of -t: the corpus file holds one string per line on the\n"
                "           given tape; the n best derivations (default 1) with the other tape free, n lines per string, best\n"
-               "           first: the --viterbi line, \" ||\" and the decoded free-tape string (\"-inf 0 | ||\" when there is none)\n";
+               "           first: the --viterbi line, \" ||\" and the decoded free-tape string (\"-inf 0 | ||\" when there is none)\n"
+               "  --sum=file    with --viterbi / --decode: ln of every example's total weight, one line per example or string\n"
+               "  --sample=n    with --viterbi / --decode (not -k): n derivations drawn per example or string in proportion to\n"
+               "           their weight, seed -R (default 1), in place of the best ones\n";
 }
 
 // carmel-b200 --gpus=N ...: N jobs in one process, job r keeps block r of the corpus on GPU r (--shard=r/N --gpu=r); the

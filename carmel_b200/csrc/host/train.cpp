@@ -347,6 +347,9 @@ void TrainJob::prepare() {
         build_trellises(*x, local, tb, dropped);
       kept = tb.kept_example;
     }
+    corpus_size = e1 - e0;
+    kept_example.clear();
+    for (uint32_t e : kept) kept_example.push_back((uint32_t)(e0 + e));
     for (uint32_t e : dropped)  // cached_derivs.h:53-57,87-93
       std::cerr << "No derivations in transducer for input/output #" << e0 + e + 1 << ":\n";
     std::vector<Example> keep;

@@ -75,7 +75,7 @@ enum cml_option {
   CML_OPT_ALLOW_EMPTY = 7, /* a rank of a sharded job whose block holds no usable example still takes part in every
                              collective: its E-step contributes zeros instead of failing with CML_ERR_NODERIV */
   CML_OPT_NO_GRAPH = 8,   /* cml_em_step enqueues its launches one by one instead of replaying a CUDA graph */
-  CML_OPT_KBEST_SCRATCH_MB = 9, /* device scratch budget (MiB) of one cml_kbest chunk; default 4096 */
+  CML_OPT_KBEST_SCRATCH_MB = 9, /* device scratch budget (MiB) of one cml_kbest or cml_sample chunk; default 4096 */
   CML_OPT_FREE_BUILD_SCRATCH_MB = 10 /* device scratch budget (MiB) of one cml_build_free_trellises chunk; default 4096 */
 };
 int cml_set_option(cml_ctx* ctx, int option, int value);
@@ -269,6 +269,39 @@ int cml_kbest(cml_ctx* ctx, uint32_t k, uint32_t* path_len, uint64_t* path_base,
 /* the last cml_kbest / cml_viterbi call: device scratch bytes of its largest chunk, number of chunks, and the time of
  * its derivation kernels from CUDA events (ms) */
 int cml_kbest_stats(cml_ctx* ctx, uint64_t* scratch_bytes, uint64_t* chunks, float* kernel_ms);
+/* The total weight of every resident lattice, and n derivations of each drawn in proportion to their weight,
+ * P(d | lattice) = w(d) / sum of w over its derivations.  Same preconditions and errors as cml_kbest (an fp64
+ * CML_SPACE_LOG context whose lattices are all in the layered-CSR layout; CML_ERR_CYCLE for a lattice with a cycle), and
+ * CML_ERR_ARG for a cap below n * the total number of lattice levels, a null ln_total, or n > 0 with a null output.
+ *   ln_total[n_ex]          beta(start) of lattice e, where beta(s) = ln of the sum over the paths s -> goal of the
+ *                           product of their arc weights: fp64, a max-shifted log-sum-exp over each state's out-arcs;
+ *                           -inf when the lattice has no derivation of non-zero weight
+ *   n = 0                   computes ln_total only; ex_key and the path arrays may then be null
+ *   ex_key[n_ex]            the key of lattice e's uniforms, or null for key = e
+ *   path_len, path_base, path_arcs, cap
+ *                           as in cml_kbest with k = n: sample r of lattice e is path_arcs[path_base[e * n + r] ..
+ *                           + path_len[e * n + r]), arc-table ids in path order
+ *   ln_weight[n_ex * n]     the sum of the sample's arc ln weights, in path order
+ * Sample r of lattice e walks from the start state to the goal.  At step t (0, 1, ...) it draws
+ *   u = sample_uniform(seed, key, r, t):  h = mix64(seed ^ mix64(key)); h = mix64(h + ((uint64_t)r << 32 | t));
+ *                                          u = (h >> 11) * 2^-53
+ * (mix64 = the splitmix64 finaliser: x += 0x9E3779B97F4A7C15; x = (x ^ x >> 30) * 0xBF58476D1CE4E5B9;
+ *  x = (x ^ x >> 27) * 0x94D049BB133111EB; x ^ x >> 31), sets c = u, and goes through state s's out-arcs in the order
+ * cml_add_trellises received them: arc j has p_j = exp(lnw_j + beta(dst_j) - beta(s)), c -= p_j, and the first arc after
+ * which c < 0 is taken.  When rounding leaves c >= 0 after the last arc, the last arc with p_j > 0 is taken.  An arc of
+ * weight zero, or whose destination has beta = -inf, is never taken.  A lattice with ln_total = -inf gives n entries
+ * with path_len 0 and ln_weight -inf.
+ *   determinism the same inputs give the same bytes on every run; results do not depend on the chunking or the launch
+ *               shape, and a lattice's samples do not depend on the other lattices
+ *   memory      device scratch of 8 B per lattice state (beta); the lattices are processed in chunks of consecutive
+ *               lattices whose scratch fits CML_OPT_KBEST_SCRATCH_MB (a lattice larger than that gets a chunk of its own)
+ * GPU work: kernel k_sample, one warp per lattice: a backward pass over the levels from the top, the states of one
+ * level across the lanes, then lane j draws samples j, j + 32, ... */
+int cml_sample(cml_ctx* ctx, uint32_t n, uint64_t seed, const uint64_t* ex_key, uint32_t* path_len, uint64_t* path_base,
+               uint32_t* path_arcs, uint64_t cap, double* ln_weight, double* ln_total);
+/* the last cml_sample call: device scratch bytes of its largest chunk, number of chunks, and the time of its k_sample
+ * launches from CUDA events (ms) */
+int cml_sample_stats(cml_ctx* ctx, uint64_t* scratch_bytes, uint64_t* chunks, float* kernel_ms);
 /* how the resident lattices are stored: examples / arcs / padded records in the level-sliced ELL layout
  * (throughput kernel) and examples in the layered-CSR layout (general kernels) */
 int cml_layout_stats(cml_ctx* ctx, uint64_t* ell_examples, uint64_t* ell_arcs, uint64_t* ell_records,
