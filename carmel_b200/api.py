@@ -344,15 +344,21 @@ class Context:
         return dict(zip(("examples", "states", "arcs", "levels"), (int(x.value) for x in v)))
 
     # ---- decode (cml_viterbi / cml_kbest) ----
-    def _decode(self, k: int | None, cap: int | None):
+    def _path_arrays(self, n: int, cap: int | None):
+        """n_ex, the arc buffer size cap (default: n * total lattice levels) and the zeroed output arrays of n
+        derivations per resident lattice: ln_weight, path_len, path_base, path_arcs"""
         t = self.trellis_totals()
-        n_ex, kk = t["examples"], 1 if k is None else k
-        n = n_ex * kk
-        ln_w, lens = np.zeros(max(n, 1)), np.zeros(max(n, 1), np.uint32)
-        base = np.zeros(n + 1, np.uint64)
+        n_ex = t["examples"]
+        m = n_ex * n
         if cap is None:
-            cap = kk * t["levels"]
-        arcs = np.zeros(max(cap, 1), np.uint32)
+            cap = n * t["levels"]
+        return (n_ex, cap, np.zeros(max(m, 1)), np.zeros(max(m, 1), np.uint32), np.zeros(m + 1, np.uint64),
+                np.zeros(max(cap, 1), np.uint32))
+
+    def _decode(self, k: int | None, cap: int | None):
+        kk = 1 if k is None else k
+        n_ex, cap, ln_w, lens, base, arcs = self._path_arrays(kk, cap)
+        n = n_ex * kk
         bp = base.ctypes.data_as(C.POINTER(C.c_uint64))
         if k is None:
             rc = self.lib.cml_viterbi(self.h, _ptr(lens, _u32p), bp, _ptr(arcs, _u32p), cap, _ptr(ln_w, _f64p))
@@ -371,11 +377,14 @@ class Context:
         """the best derivation of every resident lattice (cml_viterbi), in kbest()'s shapes with k = 1"""
         return self._decode(None, None)
 
+    def _decode_stats(self, fn) -> dict:
+        b, c, ms = C.c_uint64(), C.c_uint64(), C.c_float()
+        self._check(fn(self.h, C.byref(b), C.byref(c), C.byref(ms)))
+        return {"scratch_bytes": b.value, "chunks": c.value, "kernel_ms": ms.value}
+
     def kbest_stats(self) -> dict:
         """the last decode call: scratch bytes of its largest chunk, chunks, kernel time (CUDA events, ms)"""
-        b, c, ms = C.c_uint64(), C.c_uint64(), C.c_float()
-        self._check(self.lib.cml_kbest_stats(self.h, C.byref(b), C.byref(c), C.byref(ms)))
-        return {"scratch_bytes": b.value, "chunks": c.value, "kernel_ms": ms.value}
+        return self._decode_stats(self.lib.cml_kbest_stats)
 
     def sample(self, n: int, seed: int, keys=None, cap: int | None = None):
         """the total weight of every resident lattice and n derivations of each drawn in proportion to their weight
@@ -383,15 +392,10 @@ class Context:
         sample (e, r) is path_arcs[path_base[e*n+r]:][:path_len[e, r]].  keys: the key of each lattice's uniforms
         (default: its index); cap (default: n * total lattice levels) is the size of the arc buffer handed to the
         library.  n = 0 computes ln_total only."""
-        t = self.trellis_totals()
-        n_ex, n = t["examples"], int(n)
+        n = int(n)
+        n_ex, cap, ln_w, lens, base, arcs = self._path_arrays(n, cap)
         m = n_ex * n
         ln_total = np.zeros(max(n_ex, 1))
-        ln_w, lens = np.zeros(max(m, 1)), np.zeros(max(m, 1), np.uint32)
-        base = np.zeros(m + 1, np.uint64)
-        if cap is None:
-            cap = n * t["levels"]
-        arcs = np.zeros(max(cap, 1), np.uint32)
         kp = None
         if keys is not None:
             keys = np.ascontiguousarray(keys, np.uint64)
@@ -405,9 +409,7 @@ class Context:
 
     def sample_stats(self) -> dict:
         """the last sample() call: scratch bytes of its largest chunk, chunks, kernel time (CUDA events, ms)"""
-        b, c, ms = C.c_uint64(), C.c_uint64(), C.c_float()
-        self._check(self.lib.cml_sample_stats(self.h, C.byref(b), C.byref(c), C.byref(ms)))
-        return {"scratch_bytes": b.value, "chunks": c.value, "kernel_ms": ms.value}
+        return self._decode_stats(self.lib.cml_sample_stats)
 
     def build_free_trellises(self, wfst: dict, strings, given: int) -> dict:
         """the lattices of the given strings on tape `given` (0 input, 1 output) x the machine, the other tape free

@@ -814,15 +814,8 @@ extern "C" int cml_build_free_trellises(cml_ctx* ctx, const cml_wfst_view* x, co
   CML_CUDA(d_fw.alloc(std::max<uint64_t>(1, max_cells)));
   CML_CUDA(d_kept.alloc(std::max<uint64_t>(1, max_cells)));
   CML_CUDA(d_id.alloc(std::max<uint64_t>(1, max_cells)));
-  struct Events {
-    cudaEvent_t a = nullptr, b = nullptr;
-    ~Events() {
-      if (a) cudaEventDestroy(a);
-      if (b) cudaEventDestroy(b);
-    }
-  } ev;
-  CML_CUDA(cudaEventCreate(&ev.a));
-  CML_CUDA(cudaEventCreate(&ev.b));
+  EventPair ev;
+  CML_CUDA(ev.create());
 
   std::unique_ptr<BuiltOwner> own(new BuiltOwner());
   std::vector<uint32_t> nst(n + 1), narc(n + 1);

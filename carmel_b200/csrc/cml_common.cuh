@@ -41,6 +41,22 @@ __host__ __device__ __forceinline__ uint64_t mix64(uint64_t x) {
   return x ^ (x >> 31);
 }
 
+// Two CUDA events that bracket a call's kernels (its kernel time), destroyed on every return path
+struct EventPair {
+  cudaEvent_t a = nullptr, b = nullptr;
+  cudaError_t create() {
+    const cudaError_t e = cudaEventCreate(&a);
+    return e != cudaSuccess ? e : cudaEventCreate(&b);
+  }
+  ~EventPair() {
+    if (a) cudaEventDestroy(a);
+    if (b) cudaEventDestroy(b);
+  }
+  EventPair() {}
+  EventPair(EventPair const&) = delete;
+  EventPair& operator=(EventPair const&) = delete;
+};
+
 template <typename T>
 struct DevArray {
   T* p = nullptr;

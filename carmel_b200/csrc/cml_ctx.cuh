@@ -122,6 +122,18 @@ struct DenseState {
   }
 };
 
+// what cml_kbest_stats / cml_sample_stats report: device scratch bytes of the largest chunk, chunks, kernel time
+struct DecodeStats {
+  uint64_t scratch = 0, chunks = 0;
+  float ms = 0;
+  int get(uint64_t* scratch_bytes, uint64_t* n_chunks, float* kernel_ms) const {
+    if (scratch_bytes) *scratch_bytes = scratch;
+    if (n_chunks) *n_chunks = chunks;
+    if (kernel_ms) *kernel_ms = ms;
+    return CML_OK;
+  }
+};
+
 struct cml_ctx {
   int device = 0;
   int precision = 64;
@@ -141,12 +153,7 @@ struct cml_ctx {
   int opt_no_wide = 0;       // CML_OPT_NO_WIDE: wide lattices stay on the k_fb_ell classes
   int opt_kbest_scratch_mb = 4096;  // CML_OPT_KBEST_SCRATCH_MB: scratch of one cml_kbest / cml_sample chunk
   int opt_free_build_scratch_mb = 4096;  // CML_OPT_FREE_BUILD_SCRATCH_MB: cell scratch of one cml_build_free_trellises chunk
-  // last cml_kbest / cml_viterbi call (cml_kbest_stats)
-  uint64_t kbest_scratch = 0, kbest_chunks = 0;
-  float kbest_ms = 0;
-  // last cml_sample call (cml_sample_stats)
-  uint64_t sample_scratch = 0, sample_chunks = 0;
-  float sample_ms = 0;
+  DecodeStats kbest, sample;  // last cml_kbest / cml_viterbi call; last cml_sample call
 
   // model
   bool have_model = false, trivial = true;
@@ -235,17 +242,23 @@ struct cml_ctx {
 
 int cml_dense_estimate_launch(cml_ctx* ctx);  // cml_dense.cu
 
-// Per-lattice decoders over the layered CSR (cml_kbest.cu; cml_kbest, cml_sample): the chunks of desc slots one call
-// walks, and the arc-table ids of the internal arc ids.
+// Host code shared by the per-lattice decoders over the layered CSR (cml_decode.cu: cml_viterbi, cml_kbest;
+// cml_sample.cu: cml_sample).
+int cml_decode_batch(cml_ctx* ctx, const char* name, const char* cycle_msg, Batch** bt);
+std::vector<uint64_t> cml_path_slots(Batch const& bt, uint32_t n, uint64_t* path_base);
+int cml_arc_weights_f64(cml_ctx* ctx, const double* lnp);  // also cml_gibbs_sweep's per-arc table
+int cml_upload_arc_orig(cml_ctx* ctx, DevArray<uint32_t>& orig);
+// the chunks of desc slots one cml_kbest / cml_sample call walks
 struct DecodeChunks {
   std::vector<uint64_t> st_base, cur_base;  // [desc slot] first state / in-arc of the lattice in its chunk's scratch
   std::vector<uint32_t> list;               // chunk c = list[begin[c] .. begin[c + 1]); in-degree > 8 from mid[c] on
   std::vector<uint64_t> begin, mid;
   uint64_t max_states = 0, max_arcs = 0;    // of the largest chunk
-  DevArray<uint32_t> orig;                  // internal arc id -> arc-table id
 };
-int cml_decode_setup(cml_ctx* ctx, Batch& bt, uint64_t state_bytes, uint64_t arc_bytes, DecodeChunks& C);
-std::vector<uint64_t> cml_path_slots(Batch const& bt, uint32_t n, uint64_t* path_base);
+int cml_decode_chunks(cml_ctx* ctx, Batch& bt, uint64_t state_bytes, uint64_t arc_bytes, DecodeChunks& C);
+int cml_decode_download(cml_ctx* ctx, uint64_t m, uint32_t* path_len, const uint32_t* d_len, double* ln_weight,
+                        const double* d_lnw, uint64_t n_path, uint32_t* path_arcs, const uint32_t* d_path,
+                        EventPair const& ev, float* ms);
 
 #define CML_REQUIRE(cond, code, msg) \
   do {                               \

@@ -3035,14 +3035,9 @@ extern "C" int cml_forests_kbest(cml_forests* f, const cml_forest_batch* b, uint
   FkArgs A{d_off.p, d_next.p, d_label.p, d_br.p, d_order.p, d_lvl.p, d_lvlb.p, f->ln_w.p, 0, 0, 0, k,
            d_xs.p, d_xb.p, d_xz.p, d_xl.p, d_fs.p, d_fb.p, d_fz.p, d_fl.p, d_prv.p, d_lst.p, d_cur.p, cstride,
            d_score.p, d_nand.p};
-  struct Events {
-    cudaEvent_t e[4] = {nullptr, nullptr, nullptr, nullptr};
-    ~Events() {
-      for (auto x : e)
-        if (x) cudaEventDestroy(x);
-    }
-  } ev;
-  for (auto& x : ev.e) CML_CUDA(cudaEventCreate(&x));
+  EventPair ev, ev_paths;  // k_forest_kbest, k_forest_kbest_paths
+  CML_CUDA(ev.create());
+  CML_CUDA(ev_paths.create());
   bool fits = true, too_big = false;
   std::vector<uint64_t> obase;
   for (uint64_t c = 0; c < n_chunks; ++c) {
@@ -3051,19 +3046,19 @@ extern "C" int cml_forests_kbest(cml_forests* f, const cml_forest_batch* b, uint
     A.s0 = b->node_off[f0];
     A.n_f = (uint32_t)nfc;
     const unsigned grid = std::max(1u, std::min(f_cdiv(nfc, kFkWarps), grid_cap));
-    CML_CUDA(cudaEventRecord(ev.e[0], s));
+    CML_CUDA(cudaEventRecord(ev.a, s));
     if (G == 32)
       k_forest_kbest<32><<<grid, kFkWarps * 32, 0, s>>>(A);
     else
       k_forest_kbest<8><<<grid, kFkWarps * 32, 0, s>>>(A);
     ++f->launches;
     CML_CUDA(cudaGetLastError());
-    CML_CUDA(cudaEventRecord(ev.e[1], s));
+    CML_CUDA(cudaEventRecord(ev.b, s));
     CML_CUDA(cudaMemcpyAsync(ln_score + e0, d_score.p, ne * sizeof(double), cudaMemcpyDeviceToHost, s));
     CML_CUDA(cudaMemcpyAsync(n_and + e0, d_nand.p, ne * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
     CML_CUDA(cudaStreamSynchronize(s));
     float ms = 0;
-    CML_CUDA(cudaEventElapsedTime(&ms, ev.e[0], ev.e[1]));
+    CML_CUDA(cudaEventElapsedTime(&ms, ev.a, ev.b));
     f->kbest_ms += ms;
     obase.resize(ne);
     for (uint64_t i = 0; i < ne; ++i) {
@@ -3079,14 +3074,14 @@ extern "C" int cml_forests_kbest(cml_forests* f, const cml_forest_batch* b, uint
       CML_CUDA(d_rank.alloc(total));
     }
     CML_CUDA(cudaMemcpyAsync(d_obase.p, obase.data(), ne * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
-    CML_CUDA(cudaEventRecord(ev.e[2], s));
+    CML_CUDA(cudaEventRecord(ev_paths.a, s));
     k_forest_kbest_paths<<<f_cdiv(ne, 256), 256, 0, s>>>(A, d_obase.p, d_out.p, d_rank.p);
     ++f->launches;
     CML_CUDA(cudaGetLastError());
-    CML_CUDA(cudaEventRecord(ev.e[3], s));
+    CML_CUDA(cudaEventRecord(ev_paths.b, s));
     CML_CUDA(cudaMemcpyAsync(nodes + base[e0], d_out.p, total * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
     CML_CUDA(cudaStreamSynchronize(s));
-    CML_CUDA(cudaEventElapsedTime(&ms, ev.e[2], ev.e[3]));
+    CML_CUDA(cudaEventElapsedTime(&ms, ev_paths.a, ev_paths.b));
     f->kbest_ms += ms;
   }
   F_REQUIRE(!too_big, CML_ERR_ARG, "cml_forests_kbest: a derivation has more than 2^32 - 2 AND nodes");

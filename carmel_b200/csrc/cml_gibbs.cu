@@ -21,7 +21,6 @@
 #include <cmath>
 
 #include "cml_ctx.cuh"
-#include "cml_kernels_model.cuh"
 
 namespace {
 
@@ -770,14 +769,7 @@ extern "C" int cml_gibbs_sweep(cml_ctx* ctx, const cml_gibbs_sweep_opts* o) {
       CML_REQUIRE(ctx->have_params, CML_ERR_STATE, "init_from_params needs cml_set_params");
     CML_REQUIRE(ctx->precision == 64 && ctx->space == CML_SPACE_LOG, CML_ERR_STATE,
                 "Gibbs sampling runs in fp64 log space (create the context with precision 64, CML_SPACE_LOG)");
-    if (ctx->arc_slot_code.n < (size_t)ctx->n_arcs + 1) {
-      CML_CUDA(ctx->arc_slot_code.alloc((size_t)ctx->n_arcs + 1));
-      CML_CUDA(cudaMemsetAsync(ctx->arc_slot_code.p, 0xFF, ((size_t)ctx->n_arcs + 1) * sizeof(uint32_t), s));
-    }
-    cmlk::k_arc_weights<double, false, cmlk::WS<double>><<<cdiv(ctx->n_arcs + 1, 256), 256, 0, s>>>(
-        ctx->n_arcs, ctx->trivial ? nullptr : ctx->chain_off.p, ctx->chain_param.p, lnp, ctx->arc_slot_code.p,
-        ctx->arc_perm.p, ctx->arc_lnw.p, (double*)ctx->arc_w_real.p, (cmlk::WS<double>*)ctx->arc_ws.p);
-    ++ctx->launches;
+    if (const int rc = cml_arc_weights_f64(ctx, lnp)) return rc;
     A.arc_lnw = (const double*)ctx->arc_w_real.p;
   }
   // batched modes: the sweep's count update, summed over the ranks when the context has a communicator
@@ -973,118 +965,5 @@ extern "C" int cml_gibbs_get_state(cml_ctx* ctx, double* count, double* cum, dou
   if (normsum)
     CML_CUDA(cudaMemcpyAsync(normsum, ctx->g_normsum.p, ctx->g_norms * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
   CML_CUDA(cudaStreamSynchronize(ctx->stream));
-  return CML_OK;
-}
-
-// ---------------------------------------------------------------------------------------------------
-// Best derivation of every resident lattice (decode side: what `carmel -k 1` yields on the composed
-// string x transducer x string machine, graehl/shared/kbest.h via fst.h:769-800): a max-plus forward pass over the
-// layered CSR -- states in layered (topological) order, each state's out-arcs in the reference's stored order, a
-// destination takes a new best only on a STRICT improvement -- then a walk back from the goal.  One thread per lattice
-// (a decode runs once after training).  Needs the lattices in the layered-CSR layout of a fp64 log-space context, like
-// the samplers; lattices with a cycle are refused.
-// ---------------------------------------------------------------------------------------------------
-namespace {
-__global__ void k_viterbi(const CmlExDesc* __restrict__ desc, uint32_t n_ex, const uint32_t* __restrict__ out_off,
-                          const uint2* __restrict__ out_arc, const double* __restrict__ arc_lnw,
-                          const uint32_t* __restrict__ arc_orig, const uint64_t* __restrict__ state_base,
-                          const uint64_t* __restrict__ path_base, double* __restrict__ best, uint32_t* __restrict__ bp_src,
-                          uint32_t* __restrict__ bp_arc, uint32_t* __restrict__ path_len, uint32_t* __restrict__ path_arcs,
-                          double* __restrict__ ln_weight) {
-  const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
-  if (t >= n_ex) return;
-  const CmlExDesc d = desc[t];
-  const uint32_t e = d.ex_index, n = d.n_states;
-  const uint32_t* __restrict__ ooff = out_off + d.row_base;
-  const uint2* __restrict__ oarc = out_arc + d.arc_base;
-  double* __restrict__ b = best + state_base[e];
-  uint32_t* __restrict__ ps = bp_src + state_base[e];
-  uint32_t* __restrict__ pa = bp_arc + state_base[e];
-  for (uint32_t j = 0; j < n; ++j) b[j] = -CUDART_INF;
-  b[0] = 0.;  // the start state has layered index 0
-  for (uint32_t j = 0; j < n; ++j) {
-    const double bj = b[j];
-    if (!(bj > -CUDART_INF)) continue;
-    for (uint32_t k = ooff[j]; k < ooff[j + 1]; ++k) {
-      const uint2 a = oarc[k];
-      const double c = bj + arc_lnw[a.y];
-      if (c > b[a.x]) {
-        b[a.x] = c;
-        ps[a.x] = j;
-        pa[a.x] = a.y;
-      }
-    }
-  }
-  ln_weight[e] = b[d.fin];
-  uint32_t len = 0;
-  if (b[d.fin] > -CUDART_INF)
-    for (uint32_t s = d.fin; s != 0; s = ps[s]) ++len;
-  path_len[e] = len;
-  uint32_t* __restrict__ out = path_arcs + path_base[e];
-  uint32_t i = len;
-  if (len)
-    for (uint32_t s = d.fin; s != 0; s = ps[s]) out[--i] = arc_orig[pa[s]];
-}
-}  // namespace
-
-extern "C" int cml_viterbi(cml_ctx* ctx, uint32_t* path_len, uint64_t* path_base, uint32_t* path_arcs, uint64_t cap, double* ln_weight) {
-  if (!ctx || !path_len || !path_base || !ln_weight) return CML_ERR_ARG;
-  CML_REQUIRE(ctx->have_model && ctx->have_params, CML_ERR_STATE, "cml_set_model and cml_set_params first");
-  CML_REQUIRE(ctx->precision == 64 && ctx->space == CML_SPACE_LOG, CML_ERR_STATE,
-              "cml_viterbi runs in fp64 log space (create the context with precision 64, CML_SPACE_LOG)");
-  CML_REQUIRE(ctx->batches.size() == 1 && ctx->batches[0]->ell_ex == 0 && ctx->batches[0]->lane_ex == 0, CML_ERR_STATE,
-              "cml_viterbi needs the lattices in ONE batch in the layered-CSR layout");
-  Batch& bt = *ctx->batches[0];
-  CML_REQUIRE(bt.cyc_ex == 0, CML_ERR_CYCLE, "best derivation of a lattice with a cycle is not built");
-  cudaSetDevice(ctx->device);
-  cudaStream_t s = ctx->stream;
-  const uint64_t n_ex = bt.n_ex;
-  // path slots: a derivation has at most (levels - 1) arcs
-  std::vector<uint64_t> pbase(n_ex + 1, 0);
-  for (uint64_t e = 0; e < n_ex; ++e) pbase[e + 1] = pbase[e] + bt.h_nlevels[e];
-  for (uint64_t e = 0; e <= n_ex; ++e) path_base[e] = pbase[e];
-  CML_REQUIRE(!path_arcs || cap >= pbase[n_ex], CML_ERR_ARG, "path_arcs too small (need the total number of lattice levels)");
-  // per-arc ln weights in internal order (the same table the log-space sweeps use) and the way back to arc-table ids
-  if (ctx->arc_slot_code.n < (size_t)ctx->n_arcs + 1) {
-    CML_CUDA(ctx->arc_slot_code.alloc((size_t)ctx->n_arcs + 1));
-    CML_CUDA(cudaMemsetAsync(ctx->arc_slot_code.p, 0xFF, ((size_t)ctx->n_arcs + 1) * sizeof(uint32_t), s));
-  }
-  cmlk::k_arc_weights<double, false, cmlk::WS<double>><<<cdiv(ctx->n_arcs + 1, 256), 256, 0, s>>>(
-      ctx->n_arcs, ctx->trivial ? nullptr : ctx->chain_off.p, ctx->chain_param.p, ctx->ln_w.p, ctx->arc_slot_code.p,
-      ctx->arc_perm.p, ctx->arc_lnw.p, (double*)ctx->arc_w_real.p, (cmlk::WS<double>*)ctx->arc_ws.p);
-  ++ctx->launches;
-  std::vector<uint32_t> orig((size_t)ctx->n_arcs + 1, 0);
-  for (uint32_t a = 0; a < ctx->n_arcs; ++a) orig[ctx->h_perm[a]] = a;
-  DevArray<uint32_t> d_orig, d_src, d_arc, d_len, d_path;
-  DevArray<uint64_t> d_sbase, d_pbase;
-  DevArray<double> d_best, d_lnw;
-  CML_CUDA(d_orig.upload(orig.data(), orig.size(), s));
-  CML_CUDA(d_sbase.upload(bt.h_state_base.data(), bt.h_state_base.size(), s));
-  CML_CUDA(d_pbase.upload(pbase.data(), pbase.size(), s));
-  CML_CUDA(d_best.alloc(std::max<uint64_t>(1, bt.n_states)));
-  CML_CUDA(d_src.alloc(std::max<uint64_t>(1, bt.n_states)));
-  CML_CUDA(d_arc.alloc(std::max<uint64_t>(1, bt.n_states)));
-  CML_CUDA(d_len.alloc(std::max<uint64_t>(1, n_ex)));
-  CML_CUDA(d_lnw.alloc(std::max<uint64_t>(1, n_ex)));
-  CML_CUDA(d_path.alloc(std::max<uint64_t>(1, pbase[n_ex])));
-  cudaEvent_t ev0 = nullptr, ev1 = nullptr;  // kernel time for cml_kbest_stats
-  CML_CUDA(cudaEventCreate(&ev0));
-  CML_CUDA(cudaEventCreate(&ev1));
-  CML_CUDA(cudaEventRecord(ev0, s));
-  k_viterbi<<<cdiv(n_ex, 64), 64, 0, s>>>(bt.desc.p, (uint32_t)n_ex, bt.out_off.p, bt.out_arc.p, (const double*)ctx->arc_w_real.p,
-                                         d_orig.p, d_sbase.p, d_pbase.p, d_best.p, d_src.p, d_arc.p, d_len.p, d_path.p, d_lnw.p);
-  cudaEventRecord(ev1, s);
-  ++ctx->launches;
-  CML_CUDA(cudaGetLastError());
-  CML_CUDA(cudaMemcpyAsync(path_len, d_len.p, n_ex * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
-  CML_CUDA(cudaMemcpyAsync(ln_weight, d_lnw.p, n_ex * sizeof(double), cudaMemcpyDeviceToHost, s));
-  if (path_arcs && pbase[n_ex])
-    CML_CUDA(cudaMemcpyAsync(path_arcs, d_path.p, pbase[n_ex] * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
-  CML_CUDA(cudaStreamSynchronize(s));
-  ctx->kbest_chunks = 1;
-  ctx->kbest_scratch = bt.n_states * (sizeof(double) + 2 * sizeof(uint32_t));
-  cudaEventElapsedTime(&ctx->kbest_ms, ev0, ev1);
-  cudaEventDestroy(ev0);
-  cudaEventDestroy(ev1);
   return CML_OK;
 }

@@ -126,26 +126,23 @@ __global__ void __launch_bounds__(kSampleWarps * 32) k_sample(SampleArgs A) {
 extern "C" int cml_sample(cml_ctx* ctx, uint32_t n, uint64_t seed, const uint64_t* ex_key, uint32_t* path_len,
                           uint64_t* path_base, uint32_t* path_arcs, uint64_t cap, double* ln_weight, double* ln_total) {
   if (!ctx || !ln_total || (n && (!path_len || !path_base || !path_arcs || !ln_weight))) return CML_ERR_ARG;
-  CML_REQUIRE(ctx->have_model && ctx->have_params, CML_ERR_STATE, "cml_set_model and cml_set_params first");
-  CML_REQUIRE(ctx->precision == 64 && ctx->space == CML_SPACE_LOG, CML_ERR_STATE,
-              "cml_sample runs in fp64 log space (create the context with precision 64, CML_SPACE_LOG)");
-  CML_REQUIRE(ctx->batches.size() == 1 && ctx->batches[0]->ell_ex == 0 && ctx->batches[0]->lane_ex == 0, CML_ERR_STATE,
-              "cml_sample needs the lattices in ONE batch in the layered-CSR layout");
-  Batch& bt = *ctx->batches[0];
-  CML_REQUIRE(bt.cyc_ex == 0, CML_ERR_CYCLE, "derivations of a lattice with a cycle are not sampled");
+  Batch* b = nullptr;
+  if (const int rc = cml_decode_batch(ctx, "cml_sample", "derivations of a lattice with a cycle are not sampled", &b))
+    return rc;
+  Batch& bt = *b;
   cudaSetDevice(ctx->device);
   cudaStream_t s = ctx->stream;
   const uint64_t n_ex = bt.n_ex;
   const std::vector<uint64_t> lvl_pre = cml_path_slots(bt, n, path_base);
   CML_REQUIRE(!n || cap >= lvl_pre[n_ex] * n, CML_ERR_ARG,
               "path_arcs too small (need n times the total number of lattice levels)");
-  ctx->sample_ms = 0;
-  ctx->sample_chunks = 0;
-  ctx->sample_scratch = 0;
+  ctx->sample = DecodeStats();
   if (!n_ex) return CML_OK;
+  if (const int rc = cml_arc_weights_f64(ctx, ctx->ln_w.p)) return rc;
+  DevArray<uint32_t> d_orig;
+  if (const int rc = cml_upload_arc_orig(ctx, d_orig)) return rc;
   DecodeChunks P;  // chunk scratch: beta, 8 B per state
-  const int rc = cml_decode_setup(ctx, bt, sizeof(double), 0, P);
-  if (rc != CML_OK) return rc;
+  if (const int rc = cml_decode_chunks(ctx, bt, sizeof(double), 0, P)) return rc;
   const uint64_t n_chunks = P.mid.size();
   DevArray<uint32_t> d_list, d_plen, d_path;
   DevArray<uint64_t> d_stb, d_pre, d_key;
@@ -159,20 +156,13 @@ extern "C" int cml_sample(cml_ctx* ctx, uint32_t n, uint64_t seed, const uint64_
   CML_CUDA(d_plen.alloc(std::max<uint64_t>(1, n_ex * n)));
   CML_CUDA(d_lnw.alloc(std::max<uint64_t>(1, n_ex * n)));
   CML_CUDA(d_path.alloc(std::max<uint64_t>(1, lvl_pre[n_ex] * n)));
-  ctx->sample_chunks = n_chunks;
-  ctx->sample_scratch = P.max_states * sizeof(double);
+  ctx->sample.chunks = n_chunks;
+  ctx->sample.scratch = P.max_states * sizeof(double);
   SampleArgs A{bt.desc.p, nullptr, 0, n, seed, ex_key ? d_key.p : nullptr, bt.lvl_off.p, bt.out_off.p, bt.out_arc.p,
-               (const double*)ctx->arc_w_real.p, P.orig.p, d_stb.p, d_pre.p, d_beta.p, d_tot.p, d_plen.p, d_path.p,
+               (const double*)ctx->arc_w_real.p, d_orig.p, d_stb.p, d_pre.p, d_beta.p, d_tot.p, d_plen.p, d_path.p,
                d_lnw.p};
-  struct Events {
-    cudaEvent_t a = nullptr, b = nullptr;
-    ~Events() {
-      if (a) cudaEventDestroy(a);
-      if (b) cudaEventDestroy(b);
-    }
-  } ev;
-  CML_CUDA(cudaEventCreate(&ev.a));
-  CML_CUDA(cudaEventCreate(&ev.b));
+  EventPair ev;
+  CML_CUDA(ev.create());
   CML_CUDA(cudaEventRecord(ev.a, s));
   const unsigned max_blocks = (unsigned)ctx->sm_count * 16u;
   for (uint64_t c = 0; c < n_chunks; ++c) {
@@ -186,21 +176,11 @@ extern "C" int cml_sample(cml_ctx* ctx, uint32_t n, uint64_t seed, const uint64_
   }
   CML_CUDA(cudaEventRecord(ev.b, s));
   CML_CUDA(cudaMemcpyAsync(ln_total, d_tot.p, n_ex * sizeof(double), cudaMemcpyDeviceToHost, s));
-  if (n) {
-    CML_CUDA(cudaMemcpyAsync(path_len, d_plen.p, n_ex * n * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
-    CML_CUDA(cudaMemcpyAsync(ln_weight, d_lnw.p, n_ex * n * sizeof(double), cudaMemcpyDeviceToHost, s));
-    if (lvl_pre[n_ex])
-      CML_CUDA(cudaMemcpyAsync(path_arcs, d_path.p, lvl_pre[n_ex] * n * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
-  }
-  CML_CUDA(cudaStreamSynchronize(s));
-  CML_CUDA(cudaEventElapsedTime(&ctx->sample_ms, ev.a, ev.b));
-  return CML_OK;
+  // n = 0: the totals only (the counts below are 0, nothing else is copied)
+  return cml_decode_download(ctx, n_ex * n, path_len, d_plen.p, ln_weight, d_lnw.p, lvl_pre[n_ex] * n, path_arcs, d_path.p,
+                             ev, &ctx->sample.ms);
 }
 
 extern "C" int cml_sample_stats(cml_ctx* ctx, uint64_t* scratch_bytes, uint64_t* chunks, float* kernel_ms) {
-  if (!ctx) return CML_ERR_ARG;
-  if (scratch_bytes) *scratch_bytes = ctx->sample_scratch;
-  if (chunks) *chunks = ctx->sample_chunks;
-  if (kernel_ms) *kernel_ms = ctx->sample_ms;
-  return CML_OK;
+  return ctx ? ctx->sample.get(scratch_bytes, chunks, kernel_ms) : CML_ERR_ARG;
 }

@@ -255,15 +255,16 @@ struct TrainJob {
   TrainResult const& run(std::ostream& log);        // EM (WFST::train)
   TrainResult const& run_gibbs(std::ostream& log);  // --crp (WFST::train_gibbs)
   void prepare_gibbs();
-  // --viterbi=FILE: the best derivation of every training pair under the (normalised) model as given, one line per
-  // kept example: ln weight, number of arcs, arc-table ids; then, per arc, the (input:output) labels of the cascade
-  // members' arcs it stands for (decode side: carmel -k 1 on the composed machine, fst.h:769-800).  With --sample=n the
-  // file holds n derivations drawn per example instead, in corpus order (examples without a derivation included); with
-  // --sum=FILE that file gets ln of every example's total weight.
+  // --viterbi=FILE (decode.cpp): the best derivation of every training pair under the (normalised) model as given, one
+  // line per kept example: ln weight, number of arcs, arc-table ids; then, per arc, the (input:output) labels of the
+  // cascade members' arcs it stands for (decode side: carmel -k 1 on the composed machine, fst.h:769-800).  With -k n,
+  // n lines per kept example.  With --sample=n the file holds n derivations drawn per example instead, in corpus order
+  // (examples without a derivation included); with --sum=FILE that file gets ln of every example's total weight.
   void run_viterbi(std::ostream& log, std::string const& path);
-  // --decode=FILE --given=input|output: the -k n best derivations of every string of the corpus file on the given tape
-  // with the other tape free (carmel -sri / -sli ... -k n), n lines per string in file order: the --viterbi line, then
-  // " ||" and the free-tape labels of the path; "-inf 0 | ||" past the last derivation or for a string without one
+  // --decode=FILE --given=input|output (decode.cpp): the -k n best derivations of every string of the corpus file on the
+  // given tape with the other tape free (carmel -sri / -sli ... -k n), n lines per string in file order: the --viterbi
+  // line, then " ||" and the free-tape labels of the path; "-inf 0 | ||" past the last derivation or for a string
+  // without one
   void run_decode(std::ostream& log, std::string const& path);
   void attach_dense_sampler();  // batched --crp on position-synchronous lattices: cml_gibbs_attach_dense  // lattices + CRP parameters on the GPU, counts = priors; no sweep yet
   bool gibbs_prepared = false;

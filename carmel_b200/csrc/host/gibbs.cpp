@@ -8,8 +8,6 @@
 // sweep (gibbs.hpp:712-742) is a strictly sequential product over the corpus and is computed here from
 // the downloaded sample paths.
 #include <algorithm>
-#include <chrono>
-#include <cstdio>
 #include <fstream>
 #include <iostream>
 #include <stdexcept>
@@ -317,251 +315,6 @@ TrainResult const& TrainJob::run_gibbs(std::ostream& log) {
       }
   finish();
   return res;
-}
-
-namespace {
-
-// labels of every parameter's member arc (parameters are numbered member by member, state by state, arc by arc)
-std::vector<std::string> param_labels(std::vector<Wfst*> const& members) {
-  std::vector<std::string> plabel;
-  for (Wfst* m : members)
-    for (auto& st : m->states)
-      for (Arc& a : st) plabel.push_back(m->alph[0]->names[a.in] + ":" + m->alph[1]->names[a.out]);
-  return plabel;
-}
-
-// one decode line without its newline: ln weight, number of arcs, arc-table ids, "|", then per arc the (input:output)
-// labels of the cascade members' arcs it stands for
-void write_derivation(std::ostream& o, double lnw, const uint32_t* arcs, uint32_t len, std::vector<std::string> const& plabel,
-                      bool using_cascade, ModelArrays const& M) {
-  o << lnw << " " << len;
-  for (uint32_t k = 0; k < len; ++k) o << " " << arcs[k];
-  o << " |";
-  for (uint32_t k = 0; k < len; ++k) {
-    const uint32_t a = arcs[k];
-    const uint32_t k0 = using_cascade ? M.chain_off[a] : a, k1 = using_cascade ? M.chain_off[a + 1] : a + 1;
-    o << " (";
-    for (uint32_t c = k0; c < k1; ++c) o << (c > k0 ? " " : "") << plabel[using_cascade ? M.chain_param[c] : c];
-    o << ")";
-  }
-}
-
-// --sample / --sum: ln of the total weight of every resident lattice and, for n > 0, n derivations drawn from each in
-// proportion to their weight (cml_sample), the uniforms of lattice i keyed by key[i]
-struct Drawn {
-  std::vector<uint32_t> len, arcs;
-  std::vector<uint64_t> base;
-  std::vector<double> lnw, total;
-  float kernel_ms = 0;
-};
-int draw_samples(cml_ctx* ctx, uint32_t n, uint64_t seed, std::vector<uint64_t> const& key, Drawn& d) {
-  uint64_t n_ex = 0, n_states = 0, n_arcs = 0, n_levels = 0;
-  int rc = cml_trellis_totals(ctx, &n_ex, &n_states, &n_arcs, &n_levels);
-  if (rc != CML_OK) return rc;
-  d.len.assign(n_ex * n, 0);
-  d.arcs.assign(std::max<uint64_t>(1, n_levels * n), 0);
-  d.base.assign(n_ex * n + 1, 0);
-  d.lnw.assign(n_ex * n, 0.);
-  d.total.assign(n_ex, 0.);
-  if (!n_ex) return CML_OK;
-  rc = cml_sample(ctx, n, seed, key.data(), d.len.data(), d.base.data(), d.arcs.data(), d.arcs.size(), d.lnw.data(),
-                  d.total.data());
-  if (rc != CML_OK) return rc;
-  return cml_sample_stats(ctx, nullptr, nullptr, &d.kernel_ms);
-}
-
-// --sum=FILE: one line per example (lat_of[e] < 0: no lattice), ln of its total weight as %.17g, or -inf; the log line
-// gives the product of the totals of the examples with a derivation
-void write_sums(std::ostream& log, bool quiet, std::string const& path, std::vector<int64_t> const& lat_of,
-                std::vector<double> const& total, const char* what) {
-  std::ofstream o(path);
-  if (!o) throw std::runtime_error("cannot write " + path);
-  double prod = 0;
-  uint64_t none = 0;
-  char buf[64];
-  for (int64_t i : lat_of) {
-    const double t = i < 0 ? kNegInf : total[i];
-    std::snprintf(buf, sizeof buf, "%.17g", t);
-    o << buf << "\n";
-    if (t > kNegInf)
-      prod += t;
-    else
-      ++none;
-  }
-  if (!quiet)
-    log << "Sum: total weights of " << lat_of.size() << " " << what << ", " << none
-        << " without a derivation; product of the others=" << format_base2(prod) << "\n";
-}
-
-}  // namespace
-
-// Decode: the -k n best derivations per training pair (cml_viterbi for n = 1, cml_kbest otherwise), n lines per example
-// in corpus order, best first; ranks past the number of derivations read "-inf 0 |".  The weights are the model's as
-// read, after the same normalisation a training run starts from (train.cc:509); no training happens.
-void TrainJob::run_viterbi(std::ostream& log, std::string const& path) {
-  opt.precision = 64;
-  opt.space = CML_SPACE_LOG;  // layered-CSR lattices keep the reference's per-state arc order
-  opt.no_ell = true;
-  opt.dense = -1;
-  if (opt.shard_count > 1) throw std::runtime_error("--viterbi decodes on one GPU");
-  prepare();
-  std::vector<int64_t> lat_of(corpus_size, -1);
-  std::vector<uint64_t> key(kept_example.begin(), kept_example.end());  // the example's index in the corpus
-  for (size_t i = 0; i < kept_example.size(); ++i) lat_of[kept_example[i]] = (int64_t)i;
-  const std::vector<std::string> plabel = param_labels(members);
-  Drawn d;
-  if (opt.sample || !opt.sum_file.empty()) ok(draw_samples(ctx, opt.sample, opt.seed, key, d));
-  if (!opt.sum_file.empty()) write_sums(log, opt.quiet, opt.sum_file, lat_of, d.total, "examples");
-  if (opt.sample) {  // n lines per example in corpus order, "-inf 0 |" for an example without a derivation
-    const uint32_t n = opt.sample;
-    std::ofstream o(path);
-    if (!o) throw std::runtime_error("cannot write " + path);
-    o.precision(17);
-    for (int64_t i : lat_of)
-      for (uint32_t r = 0; r < n; ++r) {
-        const uint64_t j = i < 0 ? 0 : (uint64_t)i * n + r;
-        if (i < 0)
-          write_derivation(o, kNegInf, nullptr, 0, plabel, using_cascade, M);
-        else
-          write_derivation(o, d.lnw[j], d.arcs.data() + d.base[j], d.len[j], plabel, using_cascade, M);
-        o << "\n";
-      }
-    if (!opt.quiet)
-      log << "Sample: " << n << " derivations drawn per example (seed " << opt.seed << ") from " << kept_example.size()
-          << " of " << corpus_size << " examples (kernels " << d.kernel_ms << " ms)\n";
-    return;
-  }
-  const uint64_t K = opt.kbest;
-  uint64_t n_ex = 0, n_states = 0, n_arcs = 0, n_levels = 0;
-  ok(cml_trellis_totals(ctx, &n_ex, &n_states, &n_arcs, &n_levels));
-  std::vector<uint32_t> len(n_ex * K), arcs(std::max<uint64_t>(1, n_levels * K));
-  std::vector<uint64_t> base(n_ex * K + 1);
-  std::vector<double> lnw(n_ex * K);
-  if (n_ex && K == 1) ok(cml_viterbi(ctx, len.data(), base.data(), arcs.data(), arcs.size(), lnw.data()));
-  if (n_ex && K > 1) ok(cml_kbest(ctx, (uint32_t)K, len.data(), base.data(), arcs.data(), arcs.size(), lnw.data()));
-  std::ofstream o(path);
-  if (!o) throw std::runtime_error("cannot write " + path);
-  o.precision(17);
-  double total = 0;
-  uint64_t found = 0;
-  for (uint64_t i = 0; i < n_ex * K; ++i) {
-    write_derivation(o, lnw[i], arcs.data() + base[i], len[i], plabel, using_cascade, M);
-    o << "\n";
-    if (i % K == 0) total += lnw[i];
-    if (lnw[i] > kNegInf) ++found;
-  }
-  if (!opt.quiet) {
-    log << "Viterbi: best derivations of " << n_ex << " examples, product of their weights=" << format_base2(total) << "\n";
-    if (K > 1) log << "Viterbi: " << K << "-best lists, " << found << " derivations found\n";
-  }
-}
-
-// Decode new strings: the lattice of every string on the given tape x the composed machine, the other tape free, built on
-// the GPU (cml_build_free_trellises), then the same decoders and line format as run_viterbi.  The model is set up as for
-// --viterbi (prepare_model: the weights as read, normalised as a training run starts from them).
-void TrainJob::run_decode(std::ostream& log, std::string const& path) {
-  opt.precision = 64;
-  opt.space = CML_SPACE_LOG;
-  opt.no_ell = true;
-  opt.dense = -1;
-  if (opt.shard_count > 1) throw std::runtime_error("--decode decodes on one GPU");
-  prepare_model();
-  const int g = opt.given_tape;
-  std::vector<uint32_t> soff, ain, aout, adest;
-  x->arc_offsets(soff);
-  for (auto const& st : x->states)
-    for (Arc const& a : st) {
-      ain.push_back(a.in);
-      aout.push_back(a.out);
-      adest.push_back(a.dest);
-    }
-  const size_t n = corpus.examples.size();
-  std::vector<uint64_t> off(n + 1, 0);
-  std::vector<uint32_t> sym;
-  for (size_t e = 0; e < n; ++e) {
-    auto const& v = g ? corpus.examples[e].out : corpus.examples[e].in;
-    sym.insert(sym.end(), v.begin(), v.end());
-    off[e + 1] = sym.size();
-  }
-  cml_wfst_view xv{};
-  xv.n_states = x->num_states();
-  xv.final_state = x->final_state;
-  xv.n_arcs = ain.size();
-  xv.state_arc_off = soff.data();
-  xv.arc_in = ain.data();
-  xv.arc_out = aout.data();
-  xv.arc_dest = adest.data();
-  cml_string_batch sb{n, off.data(), sym.data()};
-  cml_built_trellises* b = nullptr;
-  ok(cml_build_free_trellises(ctx, &xv, &sb, g, &b));
-  std::unique_ptr<cml_built_trellises, void (*)(cml_built_trellises*)> hold(b, cml_free_built_trellises);
-  auto t0 = std::chrono::steady_clock::now();
-  if (b->batch.n_ex) ok(cml_add_trellises(ctx, &b->batch));
-  const double add_s = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
-  const uint64_t K = opt.sample ? opt.sample : opt.kbest;
-  uint64_t n_ex = 0, n_states = 0, n_arcs = 0, n_levels = 0;
-  ok(cml_trellis_totals(ctx, &n_ex, &n_states, &n_arcs, &n_levels));
-  std::vector<int64_t> lat_of(n, -1);
-  for (uint64_t i = 0; i < b->batch.n_ex; ++i) lat_of[b->kept_example[i]] = (int64_t)i;
-  // --sample / --sum: keyed by the string's line, so a string's draws do not depend on the other lines
-  const std::vector<uint64_t> key(b->kept_example, b->kept_example + b->batch.n_ex);
-  Drawn d;
-  if (!opt.sum_file.empty() && !opt.sample) ok(draw_samples(ctx, 0, opt.seed, key, d));
-  std::vector<uint32_t> len(n_ex * K), arcs(std::max<uint64_t>(1, n_levels * K));
-  std::vector<uint64_t> base(n_ex * K + 1);
-  std::vector<double> lnw(n_ex * K);
-  t0 = std::chrono::steady_clock::now();
-  if (opt.sample) {
-    ok(draw_samples(ctx, opt.sample, opt.seed, key, d));
-    len.swap(d.len);
-    arcs.swap(d.arcs);
-    base.swap(d.base);
-    lnw.swap(d.lnw);
-  }
-  if (n_ex && K == 1 && !opt.sample) ok(cml_viterbi(ctx, len.data(), base.data(), arcs.data(), arcs.size(), lnw.data()));
-  if (n_ex && K > 1 && !opt.sample)
-    ok(cml_kbest(ctx, (uint32_t)K, len.data(), base.data(), arcs.data(), arcs.size(), lnw.data()));
-  const double dec_s = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
-  float dec_ms = d.kernel_ms;
-  if (!opt.sample) ok(cml_kbest_stats(ctx, nullptr, nullptr, &dec_ms));
-  if (!opt.sum_file.empty()) write_sums(log, opt.quiet || flags[(unsigned)'q'], opt.sum_file, lat_of, d.total, "strings");
-  const std::vector<std::string> plabel = param_labels(members);
-  const std::vector<uint32_t>& free_label = g ? ain : aout;
-  const std::vector<std::string>& free_name = x->alph[1 - g]->names;
-  std::ofstream o(path);
-  if (!o) throw std::runtime_error("cannot write " + path);
-  o.precision(17);
-  double total = 0;
-  uint64_t found = 0;
-  for (size_t e = 0; e < n; ++e)
-    for (uint64_t r = 0; r < K; ++r) {
-      if (lat_of[e] < 0) {
-        o << "-inf 0 | ||\n";
-        continue;
-      }
-      const uint64_t i = (uint64_t)lat_of[e] * K + r;
-      const uint32_t* p = arcs.data() + base[i];
-      write_derivation(o, lnw[i], p, len[i], plabel, using_cascade, M);
-      o << " ||";
-      for (uint32_t k = 0; k < len[i]; ++k)
-        if (free_label[p[k]] != kEps) o << " " << free_name[free_label[p[k]]];
-      o << "\n";
-      if (r == 0) total += lnw[i];
-      if (lnw[i] > kNegInf) ++found;
-    }
-  if (!opt.quiet && !flags[(unsigned)'q']) {
-    log << "Decode: " << n << " strings on the " << (g ? "output" : "input") << " tape, " << b->n_dropped
-        << " without a derivation";
-    if (opt.sample)
-      log << "; " << K << " derivations drawn per string (seed " << opt.seed << ")\n";
-    else
-      log << "; product of the best weights of the others=" << format_base2(total) << "\n";
-    if (K > 1 && !opt.sample)
-      log << "Decode: " << K << "-best lists, " << found << " derivations found\n";
-    log << "Decode: lattices built on the GPU in " << b->seconds << " s (k_build_free " << b->kernel_ms << " ms, "
-        << b->chunks << " chunk(s); " << n_states << " states, " << n_arcs << " arcs), cml_add_trellises " << add_s
-        << " s, decode " << dec_s << " s (kernels " << dec_ms << " ms)\n";
-  }
 }
 
 }  // namespace cb

@@ -238,7 +238,8 @@ int cml_cyclic_stats(cml_ctx* ctx, uint64_t* n_examples, uint64_t* n_back_edges)
  * pass over the layered CSR (states in topological order, out-arcs in the reference's stored order, a destination takes
  * a new best only on a strict improvement), then the walk back from the goal.  Among derivations of exactly equal
  * weight (the same arcs in another order) the one found first in that order is reported.  Needs an fp64 CML_SPACE_LOG context
- * whose lattices are all in the layered-CSR layout (CML_OPT_NO_ELL), like the samplers.
+ * whose lattices are all in the layered-CSR layout (CML_OPT_NO_ELL), like the samplers.  cml_viterbi and cml_kbest are
+ * in cml_decode.cu, cml_sample in cml_sample.cu.
  *   path_len[n_ex]       arcs of example e's best derivation (0: none)
  *   path_base[n_ex + 1]  example e's arcs are path_arcs[path_base[e] .. path_base[e] + path_len[e])
  *   path_arcs[cap]       arc-table ids in path order; cap >= the total number of lattice levels (cml_trellis_totals)
