@@ -41,6 +41,13 @@ __host__ __device__ __forceinline__ uint64_t mix64(uint64_t x) {
   return x ^ (x >> 31);
 }
 
+// sample_uniform(seed, key, r, t) of include/carmel_b200.h (cml_sample, cml_forests_sample), with
+// h0 = mix64(seed ^ mix64(key)) computed once per lattice or forest
+__host__ __device__ __forceinline__ double sample_uniform(uint64_t h0, uint32_t r, uint32_t t) {
+  const uint64_t h = mix64(h0 + (((uint64_t)r << 32) | t));
+  return (double)(h >> 11) * (1.0 / 9007199254740992.0);
+}
+
 // Two CUDA events that bracket a call's kernels (its kernel time), destroyed on every return path
 struct EventPair {
   cudaEvent_t a = nullptr, b = nullptr;

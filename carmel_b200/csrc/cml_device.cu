@@ -2166,7 +2166,7 @@ extern "C" const char* const* cml_exported_symbols(size_t* n) {
       "cml_forests_estimate_launch", "cml_forests_estimate_finish", "cml_forests_last_time_ms", "cml_forests_get_inside",
       "cml_forests_get_counts", "cml_forests_reduce_buffer", "cml_forests_comm_init_rank", "cml_forests_allreduce_counts", "cml_forests_maximize", "cml_forests_normalize_params",
       "cml_forest_job_open", "cml_forest_job_close", "cml_forest_job_error", "cml_forest_job_set_comm", "cml_forest_job_set_quiet", "cml_forest_job_set_allreduce", "cml_forests_synchronize", "cml_forests_viterbi", "cml_forests_kbest", "cml_forests_set_kbest_scratch_mb",
-      "cml_forests_kbest_stats", "cml_forests_gibbs_init", "cml_forests_gibbs_sweep", "cml_forests_gibbs_sample_capacity",
+      "cml_forests_kbest_stats", "cml_forests_sample", "cml_forests_sample_stats", "cml_forests_gibbs_init", "cml_forests_gibbs_sweep", "cml_forests_gibbs_sample_capacity",
       "cml_forests_gibbs_get_samples", "cml_forests_gibbs_get_state",
       "cml_forest_job_prepare", "cml_forest_job_context", "cml_forest_job_train", "cml_forest_job_write",
       "cml_forest_job_stats"};

@@ -980,6 +980,9 @@ struct cml_forests {
   // cml_forests_kbest: scratch budget of one chunk, and the last call's scratch / chunks / kernel time
   uint64_t kbest_scratch_mb = 4096, kbest_scratch = 0, kbest_chunks = 0;
   float kbest_ms = 0;
+  // cml_forests_sample (chunks under the same budget): the last call's scratch / chunks / kernel time
+  uint64_t sample_scratch = 0, sample_chunks = 0;
+  float sample_ms = 0;
 };
 // cml_comm.cu
 int cml_nccl_init_rank(void** comm, int n_ranks, int rank, const unsigned char* id, std::string& err);
@@ -2612,6 +2615,113 @@ extern "C" int cml_forests_normalize_params(cml_forests* f) {
 }
 
 // ---------------------------------------------------------------------------------------------------
+// host scaffold of the per-forest decoders (cml_forests_kbest, cml_forests_sample) over a batch as given to
+// cml_forests_add: validation and levelisation, and the chunk plan
+// ---------------------------------------------------------------------------------------------------
+namespace {
+struct ForestLevels {
+  std::vector<uint32_t> order;     // per forest, at its node_off: its real nodes by height, then pre-order index
+  std::vector<uint32_t> lvl;       // per forest, at lvl_base: n_levels + 1 offsets into its order
+  std::vector<uint64_t> lvl_base;  // [n_forests + 1]
+  uint32_t max_fanout = 0;         // the largest OR fan-out of the batch
+  uint32_t max_levels = 0;         // levels of the tallest forest (a root-to-leaf path has at most this many real nodes)
+};
+
+// forest_pass1's heights, real nodes sorted by (height, pre-order index), on up to 32 host threads.  Errors name
+// the entry point `who`: CML_ERR_ARG for an empty, too large or malformed forest or a rule id beyond rulespace,
+// CML_ERR_CYCLE for a cyclic back reference (the first such forest is reported).
+int forest_levelise(cml_forests* f, const cml_forest_batch* b, const char* who, ForestLevels& out) {
+  const uint64_t nf = b->n_forests;
+  for (uint64_t i = 0; i < nf; ++i) {
+    F_REQUIRE(b->node_off[i] < b->node_off[i + 1], CML_ERR_ARG, std::string(who) + ": empty forest");
+    F_REQUIRE(b->node_off[i + 1] - b->node_off[i] < 0x7fffffffull, CML_ERR_ARG, std::string(who) + ": forest too large");
+  }
+  const uint64_t n_nodes = b->node_off[nf];
+  std::vector<FlatForest> ff(nf);
+  std::vector<uint32_t> maxdeg(nf, 0);
+  std::vector<std::vector<uint32_t>> lv(nf);
+  out.order.assign(n_nodes, 0);
+  std::vector<uint32_t>& order = out.order;
+  {
+    unsigned nt = std::max(1u, std::min(32u, std::thread::hardware_concurrency()));
+    if (nf < 64) nt = 1;
+    std::atomic<uint64_t> nextf(0);
+    auto work = [&]() {
+      ForestScratch S;
+      for (;;) {
+        const uint64_t i0 = nextf.fetch_add(64);
+        if (i0 >= nf) break;
+        for (uint64_t i = i0; i < std::min(nf, i0 + 64); ++i) {
+          const uint64_t o = b->node_off[i];
+          const uint32_t n = (uint32_t)(b->node_off[i + 1] - o);
+          const uint32_t *nx = b->next + o, *lb = b->label + o;
+          const uint8_t* br = b->backref + o;
+          forest_pass1(n, nx, lb, br, f->rulespace, S, ff[i]);
+          if (ff[i].error) continue;
+          std::vector<uint32_t>& L = lv[i];
+          L.assign(ff[i].n_levels + 1, 0);
+          for (uint32_t p = 0; p < n; ++p)
+            if (!br[p]) {
+              ++L[S.height[p] + 1];
+              if (!lb[p]) {
+                uint32_t m = 0;
+                for (uint32_t q = p + 1; q < nx[p]; q = nx[q]) ++m;
+                maxdeg[i] = std::max(maxdeg[i], m);
+              }
+            }
+          for (uint32_t h = 0; h < ff[i].n_levels; ++h) L[h + 1] += L[h];
+          S.cnt.assign(L.begin(), L.end() - 1);
+          for (uint32_t p = 0; p < n; ++p)
+            if (!br[p]) order[o + S.cnt[S.height[p]]++] = p;
+        }
+      }
+    };
+    std::vector<std::thread> th;
+    for (unsigned t = 1; t < nt; ++t) th.emplace_back(work);
+    work();
+    for (auto& t : th) t.join();
+  }
+  out.lvl_base.assign(nf + 1, 0);
+  out.max_fanout = out.max_levels = 0;
+  for (uint64_t i = 0; i < nf; ++i) {
+    if (ff[i].error) {
+      f->err = std::string(who) + ": forest " + std::to_string(i) +
+               (ff[i].error == 2 ? " has a cyclic back reference" : ff[i].error == 3 ? " uses a rule id beyond rulespace" : " is malformed");
+      return ff[i].error == 2 ? CML_ERR_CYCLE : CML_ERR_ARG;
+    }
+    out.lvl_base[i + 1] = out.lvl_base[i] + lv[i].size();
+    out.max_fanout = std::max(out.max_fanout, maxdeg[i]);
+    out.max_levels = std::max(out.max_levels, ff[i].n_levels);
+  }
+  out.lvl.assign(out.lvl_base[nf], 0);
+  for (uint64_t i = 0; i < nf; ++i) std::copy(lv[i].begin(), lv[i].end(), out.lvl.begin() + out.lvl_base[i]);
+  return CML_OK;
+}
+
+// chunks of consecutive forests whose scratch (per_node bytes per pre-order node, per_forest per forest) fits the
+// budget; a larger forest gets a chunk of its own
+struct ForestChunks {
+  std::vector<uint64_t> begin;  // chunk c is forests [begin[c], begin[c + 1])
+  uint64_t max_nodes = 0, max_forests = 0;
+};
+ForestChunks forest_chunks(const cml_forest_batch* b, uint64_t per_node, uint64_t per_forest, uint64_t budget) {
+  const uint64_t nf = b->n_forests;
+  ForestChunks P;
+  P.begin.assign(1, 0);
+  for (uint64_t i = 0; i < nf; ++i) {
+    const uint64_t c0 = P.begin.back();
+    if (i > c0 && (b->node_off[i + 1] - b->node_off[c0]) * per_node + (i + 1 - c0) * per_forest > budget) P.begin.push_back(i);
+  }
+  P.begin.push_back(nf);
+  for (size_t c = 0; c + 1 < P.begin.size(); ++c) {
+    P.max_nodes = std::max(P.max_nodes, b->node_off[P.begin[c + 1]] - b->node_off[P.begin[c]]);
+    P.max_forests = std::max(P.max_forests, P.begin[c + 1] - P.begin[c]);
+  }
+  return P;
+}
+}  // namespace
+
+// ---------------------------------------------------------------------------------------------------
 // k best derivations of every forest (forest-em -v --kbest=n): an eager k-best merge over the hypergraph, bottom-up by
 // height.  A derivation is a choice of one child at every OR node it reaches; a shared node (back reference) is
 // expanded independently at every use.  Lists are best first, with a fixed tie key:
@@ -2924,81 +3034,17 @@ extern "C" int cml_forests_kbest(cml_forests* f, const cml_forest_batch* b, uint
   f->kbest_chunks = 0;
   base[0] = 0;
   if (!nf) return CML_OK;
-  for (uint64_t i = 0; i < nf; ++i) {
-    F_REQUIRE(b->node_off[i] < b->node_off[i + 1], CML_ERR_ARG, "cml_forests_kbest: empty forest");
-    F_REQUIRE(b->node_off[i + 1] - b->node_off[i] < 0x7fffffffull, CML_ERR_ARG, "cml_forests_kbest: forest too large");
-  }
+  ForestLevels L;
+  if (const int rc = forest_levelise(f, b, "cml_forests_kbest", L)) return rc;
   const uint64_t n_nodes = b->node_off[nf];
-  // levelise on the host: forest_pass1's heights, real nodes sorted by (height, pre-order index)
-  std::vector<FlatForest> ff(nf);
-  std::vector<uint32_t> order(n_nodes), maxdeg(nf, 0);
-  std::vector<std::vector<uint32_t>> lv(nf);
-  {
-    unsigned nt = std::max(1u, std::min(32u, std::thread::hardware_concurrency()));
-    if (nf < 64) nt = 1;
-    std::atomic<uint64_t> nextf(0);
-    auto work = [&]() {
-      ForestScratch S;
-      for (;;) {
-        const uint64_t i0 = nextf.fetch_add(64);
-        if (i0 >= nf) break;
-        for (uint64_t i = i0; i < std::min(nf, i0 + 64); ++i) {
-          const uint64_t o = b->node_off[i];
-          const uint32_t n = (uint32_t)(b->node_off[i + 1] - o);
-          const uint32_t *nx = b->next + o, *lb = b->label + o;
-          const uint8_t* br = b->backref + o;
-          forest_pass1(n, nx, lb, br, f->rulespace, S, ff[i]);
-          if (ff[i].error) continue;
-          std::vector<uint32_t>& L = lv[i];
-          L.assign(ff[i].n_levels + 1, 0);
-          for (uint32_t p = 0; p < n; ++p)
-            if (!br[p]) {
-              ++L[S.height[p] + 1];
-              if (!lb[p]) {
-                uint32_t m = 0;
-                for (uint32_t q = p + 1; q < nx[p]; q = nx[q]) ++m;
-                maxdeg[i] = std::max(maxdeg[i], m);
-              }
-            }
-          for (uint32_t h = 0; h < ff[i].n_levels; ++h) L[h + 1] += L[h];
-          S.cnt.assign(L.begin(), L.end() - 1);
-          for (uint32_t p = 0; p < n; ++p)
-            if (!br[p]) order[o + S.cnt[S.height[p]]++] = p;
-        }
-      }
-    };
-    std::vector<std::thread> th;
-    for (unsigned t = 1; t < nt; ++t) th.emplace_back(work);
-    work();
-    for (auto& t : th) t.join();
-  }
-  std::vector<uint64_t> lvl_base(nf + 1, 0);
-  uint32_t cstride = k;
-  for (uint64_t i = 0; i < nf; ++i) {
-    if (ff[i].error) {
-      f->err = "cml_forests_kbest: forest " + std::to_string(i) +
-               (ff[i].error == 2 ? " has a cyclic back reference" : ff[i].error == 3 ? " uses a rule id beyond rulespace" : " is malformed");
-      return ff[i].error == 2 ? CML_ERR_CYCLE : CML_ERR_ARG;
-    }
-    lvl_base[i + 1] = lvl_base[i] + lv[i].size();
-    cstride = std::max(cstride, maxdeg[i]);
-  }
-  std::vector<uint32_t> lvl(lvl_base[nf]);
-  for (uint64_t i = 0; i < nf; ++i) std::copy(lv[i].begin(), lv[i].end(), lvl.begin() + lvl_base[i]);
-  lv.clear();
-  lv.shrink_to_fit();
-  // chunks of consecutive forests whose scratch fits the budget (a larger forest gets a chunk of its own)
-  const uint64_t per_node = 40ull * k + 16, budget = f->kbest_scratch_mb << 20;
-  std::vector<uint64_t> chunk(1, 0);
-  uint64_t max_nodes = 0, max_forests = 0;
-  for (uint64_t i = 0; i < nf; ++i)
-    if (i > chunk.back() && (b->node_off[i + 1] - b->node_off[chunk.back()]) * per_node > budget) chunk.push_back(i);
-  chunk.push_back(nf);
-  const uint64_t n_chunks = chunk.size() - 1;
-  for (uint64_t c = 0; c < n_chunks; ++c) {
-    max_nodes = std::max(max_nodes, b->node_off[chunk[c + 1]] - b->node_off[chunk[c]]);
-    max_forests = std::max(max_forests, chunk[c + 1] - chunk[c]);
-  }
+  std::vector<uint32_t>& order = L.order;
+  std::vector<uint32_t>& lvl = L.lvl;
+  std::vector<uint64_t>& lvl_base = L.lvl_base;
+  const uint32_t cstride = std::max(k, L.max_fanout);
+  const uint64_t per_node = 40ull * k + 16;
+  const ForestChunks P = forest_chunks(b, per_node, 0, f->kbest_scratch_mb << 20);
+  const std::vector<uint64_t>& chunk = P.begin;
+  const uint64_t n_chunks = chunk.size() - 1, max_nodes = P.max_nodes, max_forests = P.max_forests;
   cudaStream_t s = f->stream;
   const int G = k > 16 ? 32 : 8;
   const unsigned max_blocks = (unsigned)f->sm_count * 16u;
@@ -3087,5 +3133,289 @@ extern "C" int cml_forests_kbest(cml_forests* f, const cml_forest_batch* b, uint
   F_REQUIRE(!too_big, CML_ERR_ARG, "cml_forests_kbest: a derivation has more than 2^32 - 2 AND nodes");
   F_REQUIRE(!nodes || base[nf * k] <= cap, CML_ERR_ARG,
             "cml_forests_kbest: nodes buffer too small (need base[n_forests * k] = " + std::to_string(base[nf * k]) + ")");
+  return CML_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------
+// The total weight of every forest, and derivations drawn in proportion to their weight (forest-em -v FILE --sample=n):
+// the pre-order walk of FForest::choose_random (forest-em/forest.hpp:726-758) at fixed weights, on counter-based
+// uniforms, so a draw does not depend on the launch shape, the chunking or the other forests.
+//
+// k_forest_sample: one warp per forest.  First an inside pass over the real nodes by height (the levelisation of
+// cml_forests_kbest; the nodes of one height never feed each other, so they are spread over the lanes, and heights are
+// separated by __syncwarp): in(AND) = ln_w[rule] + in(s1) + ... + in(sm) in slot order, in(OR) = a max-shifted
+// log-sum-exp over the children in order, next to the saturating size of the node's largest derivation of non-zero
+// weight.  Then lane j draws samples j, j + 32, ...  A walk records every AND node it reaches and draws one uniform per
+// OR node; it keeps one (next slot, end of slots) entry for every AND node on the current path with slots still to
+// visit.  The real nodes of a path have strictly falling heights, so a walker's stack holds at most n_levels entries;
+// the stacks live in a chunk scratch of n_levels of the tallest forest per walker.
+// k_forest_sample_paths: one thread per sample walks it again with the same uniforms and writes its AND nodes.
+// ---------------------------------------------------------------------------------------------------
+namespace {
+const int kFsWarps = 4;  // warps per block of k_forest_sample; k_forest_sample_paths runs kFsWarps * 32 threads a block
+struct FsArgs {
+  const uint64_t* node_off;  // [n_forests + 1] the batch's pre-order arrays
+  const uint32_t* next;
+  const uint32_t* label;
+  const uint8_t* backref;
+  const uint32_t* order;     // per forest, at its node_off: its real nodes by height, then pre-order index
+  const uint32_t* lvl;       // per forest, at lvl_base: n_levels + 1 offsets into its order
+  const uint64_t* lvl_base;  // [n_forests + 1]
+  const double* ln_w;
+  const uint64_t* key;       // [n_forests] the key of forest i's uniforms, or null (key = i)
+  uint64_t seed;
+  uint64_t f0, s0;           // first forest of the chunk and its first node (chunk-local node = batch node - s0)
+  uint32_t n_f, n;
+  double* ins;               // [chunk-local pre-order node] inside value of a real node
+  uint32_t* big;             // [chunk-local pre-order node] AND nodes of its largest derivation of non-zero weight
+  uint2* stack;              // [walker * stride] (next slot, end of the slots) of an AND node on the walk's path
+  uint32_t stride;
+  double* ln_total;          // [n_f] this chunk's results
+  double* ln_weight;         // [n_f * n]
+  uint32_t* n_and;           // [n_f * n]
+};
+
+// sample r of chunk forest w: returns its number of AND nodes and sets wsum to the sum of their rules' ln weights, in
+// pre-order; with out != null also writes the nodes (in-forest pre-order indices)
+__device__ uint32_t fs_walk(const FsArgs& A, uint32_t w, uint32_t r, uint2* __restrict__ st, double& wsum,
+                            uint32_t* __restrict__ out) {
+  const uint64_t f = A.f0 + w, nb = A.node_off[f];
+  const uint32_t* __restrict__ nx = A.next + nb;
+  const uint32_t* __restrict__ lb = A.label + nb;
+  const uint8_t* __restrict__ br = A.backref + nb;
+  const double* __restrict__ I = A.ins + (nb - A.s0);
+  const uint64_t h0 = mix64(A.seed ^ mix64(A.key ? A.key[f] : f));
+  uint32_t c = 0, t = 0, m = 0, depth = 0;
+  double ws = 0.;
+  for (;;) {
+    while (!lb[c]) {  // OR node (in(c) > -inf): the first child after which u - p_1 - ... - p_j < 0
+      double u = sample_uniform(h0, r, t++);
+      const double ic = I[c];
+      uint32_t pick = kFkNone, last = kFkNone;
+      for (uint32_t b = c + 1; b < nx[c]; b = nx[b]) {
+        const uint32_t d = br[b] ? lb[b] : b;
+        const double p = exp(I[d] - ic);
+        if (p > 0.) {
+          last = d;
+          u -= p;
+          if (u < 0.) {
+            pick = d;
+            break;
+          }
+        }
+      }
+      c = pick != kFkNone ? pick : last;  // rounding left u >= 0: the last child that can be taken
+    }
+    if (out) out[m] = c;
+    ++m;
+    ws += A.ln_w[lb[c]];
+    const uint32_t e = nx[c];
+    uint32_t b;
+    if (e > c + 1) {  // its first slot next, the others pending
+      b = c + 1;
+      if (nx[b] < e) st[depth++] = make_uint2(nx[b], e);
+    } else {  // a leaf rule: the next slot of the innermost AND node with one left
+      if (!depth) break;
+      const uint2 top = st[depth - 1];
+      b = top.x;
+      if (nx[b] < top.y)
+        st[depth - 1].x = nx[b];
+      else
+        --depth;
+    }
+    c = br[b] ? lb[b] : b;
+  }
+  wsum = ws;
+  return m;
+}
+
+__global__ void __launch_bounds__(kFsWarps * 32) k_forest_sample(FsArgs A) {
+  const uint32_t lane = threadIdx.x & 31;
+  const uint32_t gw = blockIdx.x * kFsWarps + threadIdx.x / 32, nw = gridDim.x * kFsWarps;
+  uint2* __restrict__ st = A.stack + ((uint64_t)gw * 32 + lane) * A.stride;
+  for (uint32_t w = gw; w < A.n_f; w += nw) {
+    const uint64_t f = A.f0 + w, nb = A.node_off[f], sb = nb - A.s0;
+    const uint32_t* __restrict__ nx = A.next + nb;
+    const uint32_t* __restrict__ lb = A.label + nb;
+    const uint8_t* __restrict__ br = A.backref + nb;
+    const uint32_t* __restrict__ ord = A.order + nb;
+    const uint32_t* __restrict__ lv = A.lvl + A.lvl_base[f];
+    const uint32_t nl = (uint32_t)(A.lvl_base[f + 1] - A.lvl_base[f]) - 1;
+    double* __restrict__ I = A.ins + sb;
+    uint32_t* __restrict__ Z = A.big + sb;
+    for (uint32_t l = 0; l < nl; ++l) {
+      for (uint32_t j = lv[l] + lane; j < lv[l + 1]; j += 32) {
+        const uint32_t p = ord[j], e = nx[p], lab = lb[p];
+        double v;
+        uint32_t z = 0;
+        if (lab) {  // AND node: the rule, then the slots in order
+          v = A.ln_w[lab];
+          z = 1;
+          for (uint32_t b = p + 1; b < e; b = nx[b]) {
+            const uint32_t d = br[b] ? lb[b] : b;
+            v = v + I[d];
+            z = fk_sat(z, Z[d]);
+          }
+          if (!(v > -CUDART_INF)) z = 0;
+        } else {  // OR node
+          double mx = -CUDART_INF;
+          for (uint32_t b = p + 1; b < e; b = nx[b]) {
+            const uint32_t d = br[b] ? lb[b] : b;
+            mx = fmax(mx, I[d]);
+            if (I[d] > -CUDART_INF) z = max(z, Z[d]);
+          }
+          if (mx > -CUDART_INF) {
+            double sum = 0.;
+            for (uint32_t b = p + 1; b < e; b = nx[b]) sum += exp(I[br[b] ? lb[b] : b] - mx);
+            v = mx + log(sum);
+          } else {
+            v = -CUDART_INF;
+          }
+        }
+        I[p] = v;
+        Z[p] = z;
+      }
+      __syncwarp();
+    }
+    const double total = I[0];
+    const bool too_big = Z[0] == kFkNone;  // refused: no draw starts
+    if (lane == 0) A.ln_total[w] = total;
+    for (uint32_t r = lane; r < A.n; r += 32) {
+      const uint64_t o = (uint64_t)w * A.n + r;
+      if (!(total > -CUDART_INF) || too_big) {
+        A.ln_weight[o] = -CUDART_INF;
+        A.n_and[o] = too_big ? kFkNone : 0u;
+        continue;
+      }
+      double ws;
+      A.n_and[o] = fs_walk(A, w, r, st, ws, nullptr);
+      A.ln_weight[o] = ws;
+    }
+    __syncwarp();
+  }
+}
+
+// sample t = (chunk forest t / n, sample t % n): its AND nodes at out[obase[t] ..]
+__global__ void __launch_bounds__(kFsWarps * 32) k_forest_sample_paths(FsArgs A, const uint64_t* __restrict__ obase,
+                                                                       uint32_t* __restrict__ out) {
+  const uint64_t g = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x, ng = (uint64_t)gridDim.x * blockDim.x;
+  uint2* __restrict__ st = A.stack + g * A.stride;
+  for (uint64_t t = g; t < (uint64_t)A.n_f * A.n; t += ng) {
+    if (!A.n_and[t]) continue;
+    double ws;
+    fs_walk(A, (uint32_t)(t / A.n), (uint32_t)(t % A.n), st, ws, out + obase[t]);
+  }
+}
+}  // namespace
+
+extern "C" int cml_forests_sample_stats(cml_forests* f, uint64_t* scratch_bytes, uint64_t* chunks, float* kernel_ms) {
+  if (!f) return CML_ERR_ARG;
+  if (scratch_bytes) *scratch_bytes = f->sample_scratch;
+  if (chunks) *chunks = f->sample_chunks;
+  if (kernel_ms) *kernel_ms = f->sample_ms;
+  return CML_OK;
+}
+
+extern "C" int cml_forests_sample(cml_forests* f, const cml_forest_batch* b, uint32_t n, uint64_t seed, const uint64_t* key,
+                                  double* ln_weight, uint32_t* n_and, uint64_t* base, uint32_t* nodes, uint64_t cap,
+                                  double* ln_total) {
+  if (!f) return CML_ERR_ARG;
+  F_REQUIRE(b && ln_total && (!n || (ln_weight && n_and && base)), CML_ERR_ARG, "cml_forests_sample: null argument");
+  F_REQUIRE(f->have_params, CML_ERR_STATE, "cml_forests_sample before cml_forests_set_params");
+  const uint64_t nf = b->n_forests;
+  F_REQUIRE(nf == 0 || (b->node_off && b->next && b->label && b->backref), CML_ERR_ARG, "cml_forests_sample: null array");
+  CML_CUDA(cudaSetDevice(f->device));
+  f->sample_ms = 0;
+  f->sample_scratch = 0;
+  f->sample_chunks = 0;
+  if (n) base[0] = 0;
+  if (!nf) return CML_OK;
+  ForestLevels L;
+  if (const int rc = forest_levelise(f, b, "cml_forests_sample", L)) return rc;
+  const uint64_t n_nodes = b->node_off[nf];
+  // chunk scratch: per pre-order node its inside value and largest size; per forest its total and, per sample, its
+  // weight, size and output offset
+  const uint64_t per_node = sizeof(double) + sizeof(uint32_t), per_forest = sizeof(double) + 20ull * n;
+  const ForestChunks P = forest_chunks(b, per_node, per_forest, f->kbest_scratch_mb << 20);
+  const uint64_t n_chunks = P.begin.size() - 1;
+  cudaStream_t s = f->stream;
+  const unsigned max_blocks = (unsigned)f->sm_count * 16u;
+  const unsigned grid_cap = std::max(1u, std::min(f_cdiv(P.max_forests, kFsWarps), max_blocks));
+  const uint32_t stride = std::max(1u, L.max_levels);
+  const uint64_t walkers = n ? (uint64_t)grid_cap * kFsWarps * 32 : 0;
+  DevArray<uint64_t> d_off, d_lvlb, d_key, d_obase;
+  DevArray<uint32_t> d_next, d_label, d_order, d_lvl, d_big, d_nand, d_out;
+  DevArray<uint8_t> d_br;
+  DevArray<double> d_ins, d_tot, d_lnw;
+  DevArray<uint2> d_stack;
+  CML_CUDA(d_off.upload(b->node_off, nf + 1, s));
+  CML_CUDA(d_next.upload(b->next, n_nodes, s));
+  CML_CUDA(d_label.upload(b->label, n_nodes, s));
+  CML_CUDA(d_br.upload(b->backref, n_nodes, s));
+  CML_CUDA(d_order.upload(L.order.data(), n_nodes, s));
+  CML_CUDA(d_lvl.upload(L.lvl.data(), L.lvl.size(), s));
+  CML_CUDA(d_lvlb.upload(L.lvl_base.data(), nf + 1, s));
+  if (key && n) CML_CUDA(d_key.upload(key, nf, s));
+  CML_CUDA(d_ins.alloc(P.max_nodes));
+  CML_CUDA(d_big.alloc(P.max_nodes));
+  CML_CUDA(d_tot.alloc(P.max_forests));
+  CML_CUDA(d_lnw.alloc(std::max<uint64_t>(1, P.max_forests * n)));
+  CML_CUDA(d_nand.alloc(std::max<uint64_t>(1, P.max_forests * n)));
+  CML_CUDA(d_obase.alloc(std::max<uint64_t>(1, P.max_forests * n)));
+  CML_CUDA(d_stack.alloc(std::max<uint64_t>(1, walkers * stride)));
+  f->sample_chunks = n_chunks;
+  f->sample_scratch = P.max_nodes * per_node + P.max_forests * per_forest + walkers * stride * sizeof(uint2);
+  FsArgs A{d_off.p, d_next.p, d_label.p, d_br.p, d_order.p, d_lvl.p, d_lvlb.p, f->ln_w.p, key && n ? d_key.p : nullptr,
+           seed, 0, 0, 0, n, d_ins.p, d_big.p, d_stack.p, stride, d_tot.p, d_lnw.p, d_nand.p};
+  EventPair ev, ev_paths;  // k_forest_sample, k_forest_sample_paths
+  CML_CUDA(ev.create());
+  CML_CUDA(ev_paths.create());
+  bool fits = true;
+  std::vector<uint64_t> obase;
+  for (uint64_t c = 0; c < n_chunks; ++c) {
+    const uint64_t f0 = P.begin[c], nfc = P.begin[c + 1] - f0, e0 = f0 * n, ne = nfc * n;
+    A.f0 = f0;
+    A.s0 = b->node_off[f0];
+    A.n_f = (uint32_t)nfc;
+    const unsigned grid = std::max(1u, std::min(f_cdiv(nfc, kFsWarps), grid_cap));
+    CML_CUDA(cudaEventRecord(ev.a, s));
+    k_forest_sample<<<grid, kFsWarps * 32, 0, s>>>(A);
+    ++f->launches;
+    CML_CUDA(cudaGetLastError());
+    CML_CUDA(cudaEventRecord(ev.b, s));
+    CML_CUDA(cudaMemcpyAsync(ln_total + f0, d_tot.p, nfc * sizeof(double), cudaMemcpyDeviceToHost, s));
+    if (ne) {
+      CML_CUDA(cudaMemcpyAsync(ln_weight + e0, d_lnw.p, ne * sizeof(double), cudaMemcpyDeviceToHost, s));
+      CML_CUDA(cudaMemcpyAsync(n_and + e0, d_nand.p, ne * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+    }
+    CML_CUDA(cudaStreamSynchronize(s));
+    float ms = 0;
+    CML_CUDA(cudaEventElapsedTime(&ms, ev.a, ev.b));
+    f->sample_ms += ms;
+    if (!ne) continue;
+    obase.resize(ne);
+    for (uint64_t i = 0; i < ne; ++i) {
+      F_REQUIRE(n_and[e0 + i] != kFkNone, CML_ERR_ARG,
+                "cml_forests_sample: forest " + std::to_string(f0 + i / n) + " has a derivation of more than 2^32 - 2 AND nodes");
+      obase[i] = base[e0 + i] - base[e0];
+      base[e0 + i + 1] = base[e0 + i] + n_and[e0 + i];
+    }
+    const uint64_t total = base[e0 + ne] - base[e0];
+    fits = fits && (!nodes || base[e0 + ne] <= cap);
+    if (!nodes || !fits || !total) continue;
+    if (d_out.n < total) CML_CUDA(d_out.alloc(total));
+    CML_CUDA(cudaMemcpyAsync(d_obase.p, obase.data(), ne * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
+    CML_CUDA(cudaEventRecord(ev_paths.a, s));
+    k_forest_sample_paths<<<std::min(f_cdiv(ne, kFsWarps * 32), grid_cap), kFsWarps * 32, 0, s>>>(A, d_obase.p, d_out.p);
+    ++f->launches;
+    CML_CUDA(cudaGetLastError());
+    CML_CUDA(cudaEventRecord(ev_paths.b, s));
+    CML_CUDA(cudaMemcpyAsync(nodes + base[e0], d_out.p, total * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+    CML_CUDA(cudaStreamSynchronize(s));
+    CML_CUDA(cudaEventElapsedTime(&ms, ev_paths.a, ev_paths.b));
+    f->sample_ms += ms;
+  }
+  F_REQUIRE(!n || !nodes || base[nf * n] <= cap, CML_ERR_ARG,
+            "cml_forests_sample: nodes buffer too small (need base[n_forests * n] = " + std::to_string(base[nf * n]) + ")");
   return CML_OK;
 }

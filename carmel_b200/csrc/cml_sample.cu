@@ -38,12 +38,6 @@ struct SampleArgs {
   double* ln_weight;         // [n_ex * n]
 };
 
-// sample_uniform(seed, key, r, t) of include/carmel_b200.h, with h0 = mix64(seed ^ mix64(key)) computed once per lattice
-__device__ __forceinline__ double sample_uniform(uint64_t h0, uint32_t r, uint32_t t) {
-  const uint64_t h = mix64(h0 + (((uint64_t)r << 32) | t));
-  return (double)(h >> 11) * (1.0 / 9007199254740992.0);
-}
-
 __global__ void __launch_bounds__(kSampleWarps * 32) k_sample(SampleArgs A) {
   const uint32_t lane = threadIdx.x & 31;
   for (uint32_t w = blockIdx.x * kSampleWarps + threadIdx.x / 32; w < A.n_list; w += gridDim.x * kSampleWarps) {

@@ -699,8 +699,36 @@ void ForestJob::write_outputs(std::ostream& log) {
       }
       o << '\n';
     };
-    const uint32_t K = opt.kbest;
-    if (K == 1) {
+    const uint32_t K = opt.sample ? opt.sample : opt.kbest;
+    if (opt.sample) {  // n drawn derivations per forest, seed --seed, key = the forest's index in the file
+      std::vector<double> lnw(nf * K), total(nf);
+      std::vector<uint32_t> len(nf * K), nodes(std::max<uint64_t>(1, (nf ? off[nf] : 0) * K));
+      std::vector<uint64_t> base(nf * K + 1);
+      int rc = cml_forests_sample(ctx, &b, K, opt.crp_seed, nullptr, lnw.data(), len.data(), base.data(), nodes.data(),
+                                  nodes.size(), total.data());
+      if (rc == CML_ERR_ARG && base[nf * K] > nodes.size()) {
+        nodes.resize(base[nf * K]);
+        rc = cml_forests_sample(ctx, &b, K, opt.crp_seed, nullptr, lnw.data(), len.data(), base.data(), nodes.data(),
+                                nodes.size(), total.data());
+      }
+      ok(rc);
+      uint64_t found = 0;
+      for (uint64_t f = 0; f < nf; ++f) {
+        found += total[f] > kNegInfD;
+        for (uint32_t r = 0; r < K; ++r) {
+          const uint64_t i = f * K + r;
+          o << fmt_forest_weight(lnw[i], dbl, opt.human_probs) << '/' << fmt_forest_weight(sum[f], dbl, opt.human_probs);
+          if (!(lnw[i] > kNegInfD)) {
+            o << "=0% \n";
+            continue;
+          }
+          o << '=' << 100 * std::exp(lnw[i] - sum[f]) << "% ";
+          const uint32_t* next_and = nodes.data() + base[i];
+          write_tree(f, [&](uint32_t) { return *next_and++; });
+        }
+      }
+      log << "Viterbi: " << K << " samples per forest, " << found << " forests with a derivation\n";
+    } else if (K == 1) {
       std::vector<uint32_t> choice(nf ? off[nf] : 0);
       ok(cml_forests_viterbi(ctx, &b, best.data(), choice.data()));
       for (uint64_t f = 0; f < nf; ++f) {
@@ -800,6 +828,13 @@ int open_forest_job(int argc, const char* const* argv, ForestJob& job, std::ostr
           have_kbest = true;
           continue;
         }
+        if (key == "sample") {
+          char* end = nullptr;
+          const unsigned long long n = val.empty() || val[0] < '0' || val[0] > '9' ? 0 : std::strtoull(val.c_str(), &end, 10);
+          if (!n || *end || n > 0xFFFFFFFFull) throw std::runtime_error("--sample=n needs a whole number of samples >= 1 (got \"" + val + "\")");
+          a.sample = (uint32_t)n;
+          continue;
+        }
         if (key == "crp") { a.crp_iter = (unsigned)std::atol(val.c_str()); continue; }
         if (key == "burnin") { a.crp_burnin = (unsigned)std::atol(val.c_str()); continue; }
         if (key == "const-alpha") { a.crp_alpha = std::atof(val.c_str()); continue; }
@@ -870,6 +905,9 @@ int open_forest_job(int argc, const char* const* argv, ForestJob& job, std::ostr
     }
     if (have_kbest && a.outviterbi_file.empty()) throw std::runtime_error("--kbest=n needs -v (outviterbi-file)");
     if (have_kbest && a.shard_count > 1) throw std::runtime_error("--kbest decodes on one GPU (no --gpus / --shard)");
+    if (a.sample && a.outviterbi_file.empty()) throw std::runtime_error("--sample=n needs -v (outviterbi-file)");
+    if (a.sample && have_kbest) throw std::runtime_error("--sample=n draws derivations in place of --kbest: give one of them");
+    if (a.sample && a.shard_count > 1) throw std::runtime_error("--sample draws on one GPU (no --gpus / --shard)");
     if (a.max_iter && a.forests_file.empty()) throw std::runtime_error("Missing forests-file.");
     if (a.normgroups_file.empty() && (a.max_iter || a.normalize_initial)) throw std::runtime_error("Missing normgroups-file.\n");
     job.load();

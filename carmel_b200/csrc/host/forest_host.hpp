@@ -59,6 +59,7 @@ struct ForestOpts {
   int shard_rank = 0, shard_count = 1;  // --shard=r/N
   int layout = CML_FOREST_LAYOUT_AUTO;  // --layout=auto|group|thread|level (device layout family, see cml_forests_set_layout)
   uint32_t kbest = 1;                  // --kbest=n : -v writes the n best derivations per forest (cml_forests_kbest)
+  uint32_t sample = 0;                 // --sample=n : -v writes n drawn derivations per forest instead (cml_forests_sample)
   bool parse_only = false;            // --parse-only : read (and --print-forests) without touching the GPU
   // checkpoints (forest-em.hpp:166-201,621-641; forest-em-params.hpp:138-145): on every "watch" iteration (the first
   // watch_period iterations, then every watch_period-th) write <prefix>.params / <prefix>.counts
@@ -68,7 +69,7 @@ struct ForestOpts {
   double crp_alpha = .1;               // --const-alpha (gibbs_opts.hpp:229): prior = alpha * p0 * |group|
   bool crp_uniform_p0 = false, crp_final_counts = false, crp_exclude_prior = false, crp_sample_prob = false, crp_batched = false;
   double crp_high_temp = 1, crp_low_temp = 1, crp_n_sym = 0;
-  uint64_t crp_seed = 1;               // --seed : key of the counter-based uniforms
+  uint64_t crp_seed = 1;               // --seed : seed of the counter-based uniforms (--crp, --sample)
   std::string outsample_file;          // --outsample-file : the final sample, rule ids in record order, one forest per line
   unsigned watch_period = 10;          // -W
   std::string checkpoint_prefix;       // -x

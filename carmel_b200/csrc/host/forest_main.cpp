@@ -16,11 +16,16 @@
 #include "carmel_b200.h"
 
 static int run_multi_gpu(int argc, char** argv, int n_gpus) {
-  for (int i = 1; i < argc; ++i)
+  for (int i = 1; i < argc; ++i) {
     if (std::strncmp(argv[i], "--kbest", 7) == 0) {
       std::cerr << "ERROR: --kbest decodes on one GPU (no --gpus / --shard)\n\nTry 'forest-em -h' for documentation\n";
       return 1;
     }
+    if (std::strncmp(argv[i], "--sample=", 9) == 0 || std::strcmp(argv[i], "--sample") == 0) {
+      std::cerr << "ERROR: --sample draws on one GPU (no --gpus / --shard)\n\nTry 'forest-em -h' for documentation\n";
+      return 1;
+    }
+  }
   unsigned char id[CML_COMM_ID_BYTES];
   if (cml_comm_unique_id(id) != CML_OK) {
     std::cerr << "ERROR: --gpus needs NCCL (libnccl.so.2 could not be loaded)\n";

@@ -72,6 +72,9 @@ def _lib():
         lib.cml_forests_kbest.argtypes = [_vp, C.POINTER(CmlForestBatch), C.c_uint32, _f64p, _u32p, _u64p, _u32p, C.c_uint64]
         lib.cml_forests_set_kbest_scratch_mb.argtypes = [_vp, C.c_uint64]
         lib.cml_forests_kbest_stats.argtypes = [_vp, _u64p, _u64p, C.POINTER(C.c_float)]
+        lib.cml_forests_sample.argtypes = [_vp, C.POINTER(CmlForestBatch), C.c_uint32, C.c_uint64, _u64p, _f64p, _u32p,
+                                           _u64p, _u32p, C.c_uint64, _f64p]
+        lib.cml_forests_sample_stats.argtypes = [_vp, _u64p, _u64p, C.POINTER(C.c_float)]
         lib.cml_forest_job_open.argtypes = [C.POINTER(_vp), C.c_int, C.POINTER(C.c_char_p)]
         lib.cml_forest_job_close.argtypes = [_vp]
         lib.cml_forest_job_close.restype = None
@@ -207,11 +210,52 @@ class Forests:
     def set_kbest_scratch_mb(self, mb: int):
         self._ok(self.lib.cml_forests_set_kbest_scratch_mb(self.h, mb))
 
+    def _decode_stats(self, fn) -> dict:
+        b, c, ms = C.c_uint64(), C.c_uint64(), C.c_float()
+        self._ok(fn(self.h, C.byref(b), C.byref(c), C.byref(ms)))
+        return {"scratch_bytes": b.value, "chunks": c.value, "kernel_ms": ms.value}
+
     def kbest_stats(self) -> dict:
         """the last kbest() call: scratch bytes of its largest chunk, chunks, kernel time (CUDA events, ms)"""
-        b, c, ms = C.c_uint64(), C.c_uint64(), C.c_float()
-        self._ok(self.lib.cml_forests_kbest_stats(self.h, C.byref(b), C.byref(c), C.byref(ms)))
-        return {"scratch_bytes": b.value, "chunks": c.value, "kernel_ms": ms.value}
+        return self._decode_stats(self.lib.cml_forests_kbest_stats)
+
+    def sample(self, n: int, seed: int, node_off, nxt, label, backref, key=None, nodes: bool = True, cap: int | None = None):
+        """the total weight of every forest of the batch and n derivations of each drawn in proportion to their weight
+        (cml_forests_sample): (ln_weight [n_forests, n], n_and [n_forests, n], base [n_forests * n + 1], nodes,
+        ln_total [n_forests]); sample (i, r) is nodes[base[i*n+r]:][:n_and[i, r]], in-forest pre-order indices of its AND
+        nodes.  key: per forest key of its uniforms (default: the forest's index).  nodes=False asks for weights and sizes
+        only (nodes is None).  cap: size of the node buffer handed to the library (default: n * n_nodes, grown once if
+        that is too small)."""
+        b, keep = self._batch(node_off, nxt, label, backref)
+        nf, nn = b.n_forests, int(keep[0][-1])
+        lnw, lens = np.empty(max(nf * n, 1)), np.empty(max(nf * n, 1), np.uint32)
+        base, total = np.zeros(nf * n + 1, np.uint64), np.empty(max(nf, 1))
+        k = None if key is None else _arr(key, np.uint64)
+        assert k is None or len(k) == nf
+
+        def call(buf, c):
+            return self.lib.cml_forests_sample(self.h, C.byref(b), n, seed, k.ctypes.data_as(_u64p) if k is not None else None,
+                                               lnw.ctypes.data_as(_f64p), lens.ctypes.data_as(_u32p), base.ctypes.data_as(_u64p),
+                                               buf.ctypes.data_as(_u32p) if buf is not None else None, c,
+                                               total.ctypes.data_as(_f64p))
+        out = None
+        if nodes and n:
+            c = n * nn if cap is None else cap
+            out = np.empty(max(c, 1), np.uint32)
+            rc = call(out, c)
+            if rc == -1 and cap is None and int(base[-1]) > c:
+                c = int(base[-1])
+                out = np.empty(max(c, 1), np.uint32)
+                rc = call(out, c)
+            self._ok(rc)
+            out = out[:int(base[-1])]
+        else:
+            self._ok(call(None, 0))
+        return lnw[:nf * n].reshape(nf, n), lens[:nf * n].reshape(nf, n), base, out, total[:nf]
+
+    def sample_stats(self) -> dict:
+        """the last sample() call: scratch bytes of its largest chunk, chunks, kernel time (CUDA events, ms)"""
+        return self._decode_stats(self.lib.cml_forests_sample_stats)
 
     def totals(self):
         v = [C.c_uint64() for _ in range(4)]

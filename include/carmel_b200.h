@@ -648,6 +648,56 @@ int cml_forests_set_kbest_scratch_mb(cml_forests* f, uint64_t mb); /* scratch bu
 /* the last cml_forests_kbest call: device scratch bytes of its largest chunk, chunks, and the time of its derivation
  * kernels from CUDA events (ms) */
 int cml_forests_kbest_stats(cml_forests* f, uint64_t* scratch_bytes, uint64_t* chunks, float* kernel_ms);
+/* The total weight of every forest of `b` (the batch as given to cml_forests_add) at the current weights, and n
+ * derivations of each drawn in proportion to their weight, P(d | forest) = w(d) / sum of w over its derivations
+ * (forest-em -v FILE --sample=n).  Scores are fp64, from the handle's fp64 weights whatever its precision.
+ *   ln_total[n_forests]       the inside weight of forest i's root, in fp64:
+ *                               AND node, rule r, slots s1..sm   ln_w[r] + in(s1) + ... + in(sm), summed in slot order
+ *                               OR node                          a max-shifted log-sum-exp over its children, in order;
+ *                                                                -inf when every child is -inf
+ *                               back reference                   its shared node's value
+ *                             This is not the E-step's pairwise log-add with its cutoff (cml_forests_get_inside): the
+ *                             two agree to rounding, not bit for bit.
+ *   n = 0                     computes ln_total only; key and the other outputs may then be null
+ *   key[n_forests]            the key of forest i's uniforms, or null for key = i
+ *   ln_weight[n_forests * n]  ln weight of sample (i, r) at [i * n + r]: the sum of its rules' ln weights, added in
+ *                             the order of its nodes
+ *   n_and, base, nodes, cap   as in cml_forests_kbest with k = n: sample r of forest i is nodes[base[i * n + r] ..
+ *                             + n_and[i * n + r]), the in-forest pre-order indices of its AND nodes in derivation
+ *                             pre-order; nodes = NULL for weights and sizes only
+ * A forest with ln_total = -inf gives n entries with n_and 0 and ln_weight -inf.
+ * Sample r of forest i walks the derivation in pre-order from the root, as FForest::choose_random does
+ * (forest-em/forest.hpp:726-758): depth first, children in order.  A back reference stands for its shared node.  An AND
+ * node is recorded, then its slots are visited first to last, each slot's whole sub-derivation before the next.  At the
+ * t-th OR decision of the sample (t = 0, 1, ... in visiting order) it draws u = sample_uniform(seed, key_i, r, t) (as
+ * defined at cml_sample), sets c = u and goes through the OR node's children in pre-order: child j has
+ * p_j = exp(in(child_j) - in(or)); children with p_j = 0 are skipped, otherwise c -= p_j, and the first child after
+ * which c < 0 is taken.  When rounding leaves c >= 0 after the last child, the last child with p_j > 0 is taken.
+ *   determinism  the same inputs give the same bytes on every run; results do not depend on the chunking or the launch
+ *                shape, and a forest's samples depend only on that forest, the weights, seed and its key
+ *   nesting      no depth limit: a forest nested deeper than cml_forests_viterbi's 96 levels samples
+ *   size         with n > 0, a forest whose largest derivation of non-zero weight has more than 2^32 - 2 AND nodes is
+ *                refused with CML_ERR_ARG and none of its samples is drawn (a saturating max-size pass runs next to
+ *                the inside pass)
+ *   memory       device scratch of 12 B per pre-order node (inside value, largest derivation size) and 8 B + 20 B * n
+ *                per forest (total; per sample its weight, size and output offset); forests are processed in chunks of
+ *                consecutive forests whose scratch fits the budget of cml_forests_set_kbest_scratch_mb (a forest
+ *                larger than that gets a chunk of its own).  The walk adds 8 B * (levels of the tallest forest) per
+ *                walker, with 32 walkers per warp of up to min(chunk forests / 4, 16 * SMs) blocks of 4 warps, and the
+ *                drawn nodes of a chunk take 4 B each.
+ * Errors: CML_ERR_STATE before cml_forests_set_params; CML_ERR_CYCLE for a cyclic back reference; CML_ERR_ARG for a
+ * malformed forest, a rule id beyond rulespace, a null ln_total, n > 0 with a null ln_weight, n_and or base, a forest
+ * too large (above), or a non-NULL `nodes` with cap < base[n_forests * n] -- then ln_weight, n_and, base and ln_total
+ * are still filled, so the caller can size the buffer and call again.
+ * GPU work: k_forest_sample, one warp per forest: an inside pass by height, the nodes of one height across the lanes,
+ * then lane j draws samples j, j + 32, ...; k_forest_sample_paths, one thread per sample, walks it again with the
+ * same uniforms and writes its nodes. */
+int cml_forests_sample(cml_forests* f, const cml_forest_batch* b, uint32_t n, uint64_t seed, const uint64_t* key,
+                       double* ln_weight, uint32_t* n_and, uint64_t* base, uint32_t* nodes, uint64_t cap,
+                       double* ln_total);
+/* the last cml_forests_sample call: device scratch bytes of its largest chunk, chunks, and the time of its kernels
+ * from CUDA events (ms) */
+int cml_forests_sample_stats(cml_forests* f, uint64_t* scratch_bytes, uint64_t* chunks, float* kernel_ms);
 int cml_forests_synchronize(cml_forests* f);
 int cml_forests_comm_init_rank(cml_forests* f, int n_ranks, int rank, const unsigned char id[CML_COMM_ID_BYTES]);
 int cml_forests_allreduce_counts(cml_forests* f);
